@@ -20,6 +20,8 @@ the global top-100 with abo_topk_allgather.  `iteration_ms` breaks the step down
           bounded sample of the same workload (the Julia reference cannot run here: no Julia)
 
 `--impl reference` times that CPU restatement as the reference arm.
+`--dump-outputs DIR` writes the scores and the top-k of the last timed step as .npy files; the inputs are seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +41,7 @@ sys.path.insert(0, ROOT)
 N_OBS, DIM = 8192, 20
 M_PER_GPU = 2_097_152
 TOPK = 100
+DUMP_BYTES = 60_000_000          # --dump-outputs stays under 64 MB in all, whatever the candidate count and world size
 METRIC = "candidate posterior+EI evals/sec at n=8192,d=20"
 UNIT = "candidates/s"
 
@@ -161,6 +164,23 @@ def workload_config(n, d, m, world):
             "n": n, "d": d, "candidates_per_gpu": m, "l2": "inputs larger than L2"}
 
 
+def dump_outputs(out_dir, scores, top_idx, top_val, rank, world):
+    """What the last timed step handed its caller, as .npy files for comparing two builds output for output: the
+    global top-k (indices as float64, exact below 2^53) and this rank's candidate scores.  Scores that would exceed
+    the size budget are replaced by a fixed, seeded sample, and the sampled candidate indices are written beside them."""
+    os.makedirs(out_dir, exist_ok=True)
+    tag = "" if world == 1 else f"_rank{rank}"
+    if rank == 0:
+        np.save(os.path.join(out_dir, "topk_index.npy"), np.asarray(top_idx, dtype=np.float64))
+        np.save(os.path.join(out_dir, "topk_value.npy"), np.asarray(top_val, dtype=np.float64))
+    cap = DUMP_BYTES // world // 16                 # float64 score + float64 index per sampled candidate
+    if len(scores) > 2 * cap:
+        idx = np.sort(np.random.default_rng(0).choice(len(scores), cap, replace=False))
+        np.save(os.path.join(out_dir, f"scores_index{tag}.npy"), idx.astype(np.float64))
+        scores = scores[idx]
+    np.save(os.path.join(out_dir, f"scores{tag}.npy"), np.asarray(scores, dtype=np.float64))
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU implementation of the path.  The reference is Julia
     and cannot run in this image (no Julia toolchain, no network); the timed stand-in is the CPU
@@ -211,7 +231,13 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=8192)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cholesky", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the scores and the top-k of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -306,6 +332,8 @@ def main():
     barrier()
     wall = time.perf_counter() - w0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, scores_dev.cpu().numpy(), top_idx, top_val, rank, world)
     ms = max(e0.elapsed_time(e1), 0.0)
     launches = ctx.launch_count() - launches0
     # the posterior the sweeps ran on, kept for the e2e leg and the checks below
