@@ -558,6 +558,12 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
         if (jn < T) { CU(cudaEventRecord(c->ev_b, su)); rest_pending = true; }
     }
     if (rest_pending) CU(cudaStreamWaitEvent(sp, c->ev_b, 0));
+    if (notify_stream && notify_tile > 0) {
+        // no outer-block boundary fell in [notify_tile, T) (the loop breaks at je = T before notifying): the notified
+        // work waits for the whole factor instead; every side stream has joined the panel stream by now
+        CU(cudaEventRecord(c->ev_a, sp));
+        CU(cudaStreamWaitEvent(notify_stream, c->ev_a, 0));
+    }
     if (trace) {
         cudaStreamSynchronize(sp); cudaStreamSynchronize(su);
         fprintf(stderr, "potrf trace (ms since start), %zu events:", tev.size());
@@ -913,7 +919,20 @@ static KSpec gp_spec(const abo_gp* g) {
     return k;
 }
 
+static int gp_fit_run(abo_gp* g, const double* X, const double* y, int64_t n, int64_t* info_out);
 extern "C" int32_t abo_gp_fit(abo_gp* g, const double* X, const double* y, int64_t n, int64_t* info_out) {
+    const int rc = gp_fit_run(g, X, y, n, info_out);
+    if (rc && g && g->ctx) {
+        // an error return must not leave the factorisation's side streams or the overlapped inverse on stream4 running:
+        // they write L, L^-1 and workspace slots that the next call may reuse.  Drain every stream, keep the first error.
+        const std::string keep = g_err;
+        ctx_sync_all(g->ctx);
+        cudaGetLastError();
+        g_err = keep;
+    }
+    return rc;
+}
+static int gp_fit_run(abo_gp* g, const double* X, const double* y, int64_t n, int64_t* info_out) {
     if (!g || !X || !y) return abo_fail(ABO_ERR_INVALID, "null argument");
     if (n < 1) return abo_fail(ABO_ERR_DIM, "need at least one observation");
     if (!g->ctx) return abo_fail(ABO_ERR_INVALID, "the context of this handle has been destroyed");
@@ -984,10 +1003,8 @@ extern "C" int32_t abo_gp_fit(abo_gp* g, const double* X, const double* y, int64
     CU(cudaMemcpyAsync(&hinfo, dinfo, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (info_out) *info_out = hinfo;
-    if (hinfo != 0) {
-        if (overlap) CU(cudaStreamSynchronize(c->stream4));
+    if (hinfo != 0)                                                   // abo_gp_fit drains stream4 on the way out
         return abo_fail(ABO_ERR_NOT_POSDEF, "matrix is not positive definite; Cholesky factorization failed at pivot %d", hinfo);
-    }
     if (overlap) {
         const int64_t off = (int64_t)b_top * NB * (g->ld + 1);
         if ((rc = trtri_tma_on(c, g->dL + off, g->dLinv + off, U + off, W + off, Npad - (int64_t)b_top * NB, g->ld, 0,

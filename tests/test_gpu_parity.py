@@ -292,18 +292,28 @@ def test_gradient_gp_known_answer(abo, orc):
 
 
 def test_potrf_dev(abo):
+    """The look-ahead Cholesky at tile counts T = n / 128 on every branch of its schedule: T <= OB = 3 (one blocked
+    call), the outer-block ramp 1, 2, 3 (T = 4, 5, 7, 8, 17), around the overlapped inverse's b_top = 32 (31-33), the PDL
+    threshold of 40 trailing tiles (40, 41) and the 64-row panel GEMMs of panels with 4096 rows or more (33 on; 44, 64-66).
+    Against LAPACK, by the backward error |L L^T - A| <= N eps max|A| (gamma_{N+1}), and bit-identical when repeated."""
     import torch
     ctx = abo.default_context()
-    for n in (128, 640, 1024, 2176):
+    eps = np.finfo(np.float64).eps
+    for T in (1, 2, 3, 4, 5, 7, 8, 17, 31, 32, 33, 40, 41, 44, 64, 65, 66):
+        n = 128 * T
         g = torch.Generator(device="cpu").manual_seed(n)
-        A = torch.randn(n, n, dtype=torch.float64, generator=g)
-        A = A @ A.T / n + torch.eye(n, dtype=torch.float64)
-        dA = A.cuda()
+        B = torch.randn(n, n, dtype=torch.float64, generator=g).cuda()
+        A = B @ B.T / n + torch.eye(n, dtype=torch.float64, device="cuda")     # O(n^3) products on the device: n = 8448
+        dA = A.clone(); dB = A.clone()
         torch.cuda.synchronize()
         assert ctx.potrf_dev(dA.data_ptr(), n, n) == 0
-        L = torch.tril(dA).cpu().numpy()
-        ref = np.linalg.cholesky(A.numpy())
-        assert np.max(np.abs(L - ref)) < 1e-11
+        assert ctx.potrf_dev(dB.data_ptr(), n, n) == 0
+        L = torch.tril(dA)
+        assert torch.equal(L, torch.tril(dB)), T
+        resid = float((L @ L.T - A).abs().max())
+        assert resid <= n * eps * float(A.abs().max()), (T, resid)
+        ref = np.linalg.cholesky(A.cpu().numpy())
+        assert np.max(np.abs(L.cpu().numpy() - ref)) < 1e-11, T
 
 
 def test_standardgp_copy_semantics(abo):
