@@ -46,9 +46,7 @@ extern "C" int32_t abo_version(void) { return 100; }
 // context
 // ------------------------------------------------------------------------------------------
 static int configure_kernels() {
-    CU(configure_gemm<KC, KC, EPI_STORE>());
-    CU(configure_gemm<KC, MC, EPI_STORE>());
-    CU(configure_gemm<MC, MC, EPI_STORE>());
+    CU(cudaFuncSetAttribute(gemm_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU(cudaFuncSetAttribute(gemm_small_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmS<32, 8>::SMEM_BYTES));
     CU(cudaFuncSetAttribute(gemm_small_kernel<64, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmS<64, 8>::SMEM_BYTES));
     CU(cudaFuncSetAttribute(gemm_k128_kernel<16, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmK128<16, 128>::SMEM_BYTES));
@@ -56,8 +54,6 @@ static int configure_kernels() {
     CU(cudaFuncSetAttribute(fill_distance_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 256 * 96 * 8));
     CU(cudaFuncSetAttribute(potf2_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PW_SMEM_BYTES));
     CU(cudaFuncSetAttribute(sweep_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SW_SMEM_BYTES));
-    CU(cudaFuncSetAttribute(gemm_ws_kernel<KC, MC>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SMEM_BYTES));
-    CU(cudaFuncSetAttribute(gemm_ws_kernel<MC, MC>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SMEM_BYTES));
     CU(cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SY_SMEM_BYTES));
     CU(cudaFuncSetAttribute(gemm_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TG_SMEM_BYTES));
 #define ABO_FS_CFG(DT) CU(cudaFuncSetAttribute(sweep_fused_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, fused_smem_bytes<DT>()))
@@ -277,33 +273,27 @@ int pinned_get(abo_ctx* c, size_t bytes, void** out) {
 }
 
 // ------------------------------------------------------------------------------------------
-// blocked Cholesky (right-looking, NB = 128): potf2+inverse of the diagonal block (1 CTA),
-// panel TRSM as a DMMA GEMM with the block inverse, SYRK trailing update as a DMMA GEMM.
-// A: batch matrices, row-major, Npad x Npad (ld), lower triangle referenced.
+// blocked Cholesky (right-looking, NB = 128) of `batch` contiguously stacked matrices: potf2+inverse of the diagonal
+// block (1 CTA per matrix), then panel TRSM (as a GEMM with the block inverse) and SYRK trailing update on the persistent
+// TMA pipeline (both operands k-contiguous; K = 128 per step, so the missing pipeline fill / drain per tile is most of the
+// gain).  A single matrix takes the same schedule, so a restart evaluated alone gives the same bits as in a batch.
+// A: batch matrices, row-major, Npad x Npad (ld), matrix z at A + z Npad ld, lower triangle referenced.
 // Dinv: batch x T x 128 x 128 block inverses.  info: batch ints (0 = ok).
 // ------------------------------------------------------------------------------------------
 int make_tmap_k4(CUtensorMap* map, const double* base, int64_t K, int64_t rows, int64_t ld);
 static int launch_gemm_tma(abo_ctx* c, const CUtensorMap& tmA, const CUtensorMap& tmB, TmaGemmParams p, cudaStream_t st, int max_ctas = 0);
-int potrf_blocked(abo_ctx* c, double* A, int64_t Npad, int64_t ld, int64_t strideA, double* Dinv, int64_t strideD,
-                  int* info, int batch) {
+int potrf_blocked(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Dinv, int* info, int batch) {
     const int T = (int)(Npad / NB);
+    const int64_t strideA = Npad * ld, strideD = (int64_t)T * NB * NB;
     cudaStream_t st = c->stream;
-    // batched, contiguously stacked matrices (the NLML restarts): panel TRSM and trailing SYRK on the persistent TMA pipeline
-    // (both operands k-contiguous; K = 128 per step, so the missing pipeline fill / drain per tile is most of the gain)
-    static const bool tma_env = getenv("ABO_POTRF_TMA") ? atoi(getenv("ABO_POTRF_TMA")) != 0 : true;
-    // (a single matrix passed with the stacked-layout strides takes the same path: a restart evaluated alone gives the same bits)
-    const bool tma = tma_env && batch >= 1 && strideA == Npad * ld && strideD == (int64_t)T * NB * NB;
     CUtensorMap tmA, tmD;
-    if (tma) {
-        int rc;
-        if ((rc = make_tmap_k4(&tmA, A, Npad, (int64_t)batch * Npad, ld)) || (rc = make_tmap_k4(&tmD, Dinv, NB, (int64_t)batch * T * NB, NB)))
-            return rc;
-    }
-    // two-level blocking of the batched path: inside an outer block of OB tile columns the SYRK touches the block's own
-    // columns only (K = 128); everything to the right is updated ONCE per outer block with K = OB * 128, i.e. one
-    // read-modify-write of the trailing tiles per OB panels instead of one per panel
-    static const int ob_env = getenv("ABO_POTRF_BATCH_OB") ? atoi(getenv("ABO_POTRF_BATCH_OB")) : 2;
-    const int OB = tma ? std::max(1, ob_env) : 1;
+    int rc;
+    if ((rc = make_tmap_k4(&tmA, A, Npad, (int64_t)batch * Npad, ld)) || (rc = make_tmap_k4(&tmD, Dinv, NB, (int64_t)batch * T * NB, NB)))
+        return rc;
+    // two-level blocking: inside an outer block of OB tile columns the SYRK touches the block's own columns only (K = 128);
+    // everything to the right is updated ONCE per outer block with K = OB * 128, i.e. one read-modify-write of the trailing
+    // tiles per OB panels instead of one per panel.  OB = 3 and 4 measure the same as 2 (DESIGN.md).
+    constexpr int OB = 2;
     for (int jb = 0; jb < T; ++jb) {
         double* Ajj = A + (int64_t)jb * NB * (ld + 1);
         double* Dj = Dinv + (int64_t)jb * NB * NB;
@@ -311,49 +301,30 @@ int potrf_blocked(abo_ctx* c, double* A, int64_t Npad, int64_t ld, int64_t strid
         KL(c);
         const int rem = (int)(Npad - (int64_t)(jb + 1) * NB);
         if (rem <= 0) break;
-        double* P = Ajj + (int64_t)NB * ld;            // panel below the diagonal block
-        if (tma) {
-            int rc;
-            const int ob0 = jb / OB * OB, obend = std::min(ob0 + OB, T);      // this panel's outer block [ob0, obend)
-            TmaGemmParams g{};                         // L_ij = A_ij * inv(L_jj)^T, in place (a tile is read completely before it is written)
-            g.Mt = rem / NB; g.Nt = 1; g.batch = batch; g.K = NB; g.flags = 0; g.alpha = 1.0; g.beta = 0.0;
-            g.a_row0 = (jb + 1) * NB; g.a_rstep = (int)Npad; g.a_col0 = jb * NB; g.a_cstep = 0;
-            g.b_row0 = jb * NB; g.b_rstep = T * NB; g.b_col0 = 0; g.b_cstep = 0;
-            g.C = A; g.ldc = ld; g.c_off0 = (int64_t)(jb + 1) * NB * ld + (int64_t)jb * NB; g.c_zstep = strideA;
-            if ((rc = launch_gemm_tma(c, tmA, tmD, g, st))) return rc;
-            const int nin = obend - jb - 1;            // tile columns of the outer block still to the right of this panel
-            if (nin > 0) {
-                TmaGemmParams q{};                     // columns jb+1 .. obend-1: A -= L_panel L_panel^T (lower tiles), K = 128
-                q.Mt = rem / NB; q.Nt = nin; q.batch = batch; q.K = NB; q.flags = LOWER_ONLY; q.alpha = -1.0; q.beta = 1.0;
-                q.a_row0 = (jb + 1) * NB; q.a_rstep = (int)Npad; q.a_col0 = jb * NB; q.a_cstep = 0;
-                q.b_row0 = q.a_row0; q.b_rstep = q.a_rstep; q.b_col0 = q.a_col0; q.b_cstep = 0;
-                q.C = A; q.ldc = ld; q.c_off0 = (int64_t)(jb + 1) * NB * (ld + 1); q.c_zstep = strideA;
-                if ((rc = launch_gemm_tma(c, tmA, tmA, q, st))) return rc;
-            }
-            if (jb == obend - 1 && obend < T) {
-                TmaGemmParams q{};                     // columns >= obend: A -= L_block L_block^T, K = (obend - ob0) * 128
-                q.Mt = T - obend; q.Nt = T - obend; q.batch = batch; q.K = (obend - ob0) * NB; q.flags = LOWER_ONLY; q.alpha = -1.0; q.beta = 1.0;
-                q.a_row0 = obend * NB; q.a_rstep = (int)Npad; q.a_col0 = ob0 * NB; q.a_cstep = 0;
-                q.b_row0 = q.a_row0; q.b_rstep = q.a_rstep; q.b_col0 = q.a_col0; q.b_cstep = 0;
-                q.C = A; q.ldc = ld; q.c_off0 = (int64_t)obend * NB * (ld + 1); q.c_zstep = strideA;
-                if ((rc = launch_gemm_tma(c, tmA, tmA, q, st))) return rc;
-            }
-            continue;
+        const int ob0 = jb / OB * OB, obend = std::min(ob0 + OB, T);      // this panel's outer block [ob0, obend)
+        TmaGemmParams g{};                             // L_ij = A_ij * inv(L_jj)^T, in place (a tile is read completely before it is written)
+        g.Mt = rem / NB; g.Nt = 1; g.batch = batch; g.K = NB; g.flags = 0; g.alpha = 1.0; g.beta = 0.0;
+        g.a_row0 = (jb + 1) * NB; g.a_rstep = (int)Npad; g.a_col0 = jb * NB; g.a_cstep = 0;
+        g.b_row0 = jb * NB; g.b_rstep = T * NB; g.b_col0 = 0; g.b_cstep = 0;
+        g.C = A; g.ldc = ld; g.c_off0 = (int64_t)(jb + 1) * NB * ld + (int64_t)jb * NB; g.c_zstep = strideA;
+        if ((rc = launch_gemm_tma(c, tmA, tmD, g, st))) return rc;
+        const int nin = obend - jb - 1;                // tile columns of the outer block still to the right of this panel
+        if (nin > 0) {
+            TmaGemmParams q{};                         // columns jb+1 .. obend-1: A -= L_panel L_panel^T (lower tiles), K = 128
+            q.Mt = rem / NB; q.Nt = nin; q.batch = batch; q.K = NB; q.flags = LOWER_ONLY; q.alpha = -1.0; q.beta = 1.0;
+            q.a_row0 = (jb + 1) * NB; q.a_rstep = (int)Npad; q.a_col0 = jb * NB; q.a_cstep = 0;
+            q.b_row0 = q.a_row0; q.b_rstep = q.a_rstep; q.b_col0 = q.a_col0; q.b_cstep = 0;
+            q.C = A; q.ldc = ld; q.c_off0 = (int64_t)(jb + 1) * NB * (ld + 1); q.c_zstep = strideA;
+            if ((rc = launch_gemm_tma(c, tmA, tmA, q, st))) return rc;
         }
-        GemmParams g{};
-        g.A = P; g.lda = ld; g.strideA = strideA;
-        g.B = Dj; g.ldb = NB; g.strideB = strideD;
-        g.C = P; g.ldc = ld; g.strideC = strideA;
-        g.M = rem; g.N = NB; g.K = NB; g.alpha = 1.0; g.beta = 0.0; g.flags = 0;
-        CU((launch_gemm_small<64, 8>(g, batch, st)));        // L_ij = A_ij * inv(L_jj)^T
-        KL(c);
-        GemmParams s{};
-        s.A = P; s.lda = ld; s.strideA = strideA;
-        s.B = P; s.ldb = ld; s.strideB = strideA;
-        s.C = Ajj + (int64_t)NB * (ld + 1); s.ldc = ld; s.strideC = strideA;
-        s.M = rem; s.N = rem; s.K = NB; s.alpha = -1.0; s.beta = 1.0; s.flags = LOWER_ONLY;
-        CU((launch_gemm_small<64, 8>(s, batch, st)));        // A_22 -= L_21 L_21^T
-        KL(c);
+        if (jb == obend - 1 && obend < T) {
+            TmaGemmParams q{};                         // columns >= obend: A -= L_block L_block^T, K = (obend - ob0) * 128
+            q.Mt = T - obend; q.Nt = T - obend; q.batch = batch; q.K = (obend - ob0) * NB; q.flags = LOWER_ONLY; q.alpha = -1.0; q.beta = 1.0;
+            q.a_row0 = obend * NB; q.a_rstep = (int)Npad; q.a_col0 = ob0 * NB; q.a_cstep = 0;
+            q.b_row0 = q.a_row0; q.b_rstep = q.a_rstep; q.b_col0 = q.a_col0; q.b_cstep = 0;
+            q.C = A; q.ldc = ld; q.c_off0 = (int64_t)obend * NB * (ld + 1); q.c_zstep = strideA;
+            if ((rc = launch_gemm_tma(c, tmA, tmA, q, st))) return rc;
+        }
     }
     return ABO_OK;
 }
@@ -374,30 +345,23 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 
 // ------------------------------------------------------------------------------------------
 // Single-matrix Cholesky with two-level blocking and look-ahead (the "Cholesky TFLOP/s" path).
-//   outer block = OB tile columns (512): inside it the panels are factored right-looking
+//   outer block = LA_OB tile columns (384): inside it the panels are factored right-looking
 //   (potf2+inverse, TRSM-as-GEMM, SYRK restricted to the block's own columns, K = 128);
-//   the rest of the trailing matrix is updated ONCE per outer block with K = 512 by the
+//   the rest of the trailing matrix is updated ONCE per outer block with K = 384 by the
 //   TMA/mbarrier DMMA kernel (syrk_tma_kernel), split into
 //       U_next : the next outer block's columns  -> panel stream (high priority)
 //       U_rest : everything further right        -> second stream, overlaps the next panel
+// The four schedule constants were scanned on B200 at n = 4096 and 8192 (outer block 2-4, PDL from 24-80 tiles, 64-row
+// panel tiles from 2048 rows or never, 32-row slabs up to 30-120 tiles): every setting came within 3 %, the panel chain
+// and not the schedule is the limit.
 // ------------------------------------------------------------------------------------------
+constexpr int LA_OB = 3;             // outer block in tiles: the trailing matrix is read and written once per 384 columns
+constexpr int LA_PDL_TILES = 40;     // PDL once T - Jb <= 40: earlier, resident dependents take shared memory from the U_rest CTAs
+constexpr int LA_SMALL_NEXT = 60;    // largest U_next slab (tiles) on 32-row tiles: one 128-row tile per CTA would idle most SMs
+constexpr int LA_BIG_REM = 4096;     // panel GEMMs: 64-row tiles while >= 4096 rows remain (throughput), 32-row below (latency)
 int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Dinv, int* info, int notify_tile, cudaStream_t notify_stream) {
     const int T = (int)(Npad / NB);
-    static const int OB_env = getenv("ABO_POTRF_OB") ? atoi(getenv("ABO_POTRF_OB")) : 3;
-    static const bool one_stream = getenv("ABO_POTRF_1STREAM") != nullptr;
-    static const bool pdl_on = getenv("ABO_NO_PDL") == nullptr;
-    static const int pdl_tiles = getenv("ABO_POTRF_PDLTILES") ? atoi(getenv("ABO_POTRF_PDLTILES")) : 40;
-    static const bool ramp = getenv("ABO_POTRF_NORAMP") == nullptr;
-    static const int small_next = getenv("ABO_POTRF_SMALLNEXT") ? atoi(getenv("ABO_POTRF_SMALLNEXT")) : 60;
-    // panel GEMMs: 64-row tiles while the panel is tall (throughput), 32-row tiles once it is short (latency)
-    static const int big_rem = getenv("ABO_POTRF_BIGREM") ? atoi(getenv("ABO_POTRF_BIGREM")) : 4096;
-    const int OB = std::max(1, OB_env);
-    if (T <= OB) {
-        int rc0 = potrf_blocked(c, A, Npad, ld, 0, Dinv, 0, info, 1);
-        if (!rc0 && notify_stream) { CU(cudaEventRecord(c->ev_a, c->stream)); CU(cudaStreamWaitEvent(notify_stream, c->ev_a, 0)); }
-        return rc0;
-    }
-    cudaStream_t sp = c->stream, su = one_stream ? c->stream : c->stream2;
+    cudaStream_t sp = c->stream, su = c->stream2;
     CUtensorMap tmL;
     int rc = make_tmap_k4(&tmL, A, Npad, Npad, ld);
     if (rc) return rc;
@@ -407,22 +371,13 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
     bool s3_pending = false;
     bool boundary_split = false;
     cudaStream_t s3 = c->stream3;
-    static const bool split = getenv("ABO_POTRF_NOSPLIT") == nullptr;
-    static const bool k128 = getenv("ABO_POTRF_NOK128") == nullptr;
-    static const bool trace = getenv("ABO_POTRF_TRACE") != nullptr;
-    std::vector<cudaEvent_t> tev;           // per outer block: start, panel done, U_next done (sp), U_rest start, done (su)
-    auto mark = [&](cudaStream_t s_) { if (trace) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, s_); tev.push_back(e); } };
-    mark(sp);
-    // outer blocks ramp up (1, 2, OB, OB, ...): the first panels are not hidden behind any update, so
+    // outer blocks ramp up (1, 2, LA_OB, LA_OB, ...): the first panels are not hidden behind any update, so
     // the trailing-update stream is given work as early as possible
     int step = 0;
     for (int Jb = 0, je = 0; Jb < T; Jb = je, ++step) {
-        je = std::min(Jb + (ramp ? std::min(step + 1, OB) : OB), T);
-        // PDL only once the trailing matrix is small: early-resident dependents would otherwise take
-        // shared memory away from the big trailing-update CTAs of the second stream
-        const bool pdl = pdl_on && (T - Jb) <= pdl_tiles;
+        je = std::min(Jb + std::min(step + 1, LA_OB), T);
+        const bool pdl = (T - Jb) <= LA_PDL_TILES;
         // ---- panel block: tile columns [Jb, je)
-        mark(sp);
         for (int jp = Jb; jp < je; ++jp) {
             double* Ajj = A + (int64_t)jp * NB * (ld + 1);
             double* Dj = Dinv + (int64_t)jp * NB * NB;
@@ -435,7 +390,7 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
             const int ncol = (je - jp - 1) * NB;       // remaining columns of this outer block
             auto gemm_panel = [&](const GemmParams& q, cudaStream_t s_, bool pdl_) -> int {
                 if (q.M <= 0 || q.N <= 0) return ABO_OK;
-                if (q.M >= big_rem) CU(launch_pdl(gemm_small_kernel<64, 8>, dim3(q.N / BN, q.M / 64, 1), dim3(256), GemmS<64, 8>::SMEM_BYTES, s_, pdl_, q));
+                if (q.M >= LA_BIG_REM) CU(launch_pdl(gemm_small_kernel<64, 8>, dim3(q.N / BN, q.M / 64, 1), dim3(256), GemmS<64, 8>::SMEM_BYTES, s_, pdl_, q));
                 else CU(launch_pdl(gemm_small_kernel<32, 8>, dim3(q.N / BN, q.M / 32, 1), dim3(256), GemmS<32, 8>::SMEM_BYTES, s_, pdl_, q));
                 KL(c);
                 return ABO_OK;
@@ -448,7 +403,7 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
             s.C = Ajj + (int64_t)NB * (ld + 1); s.ldc = ld;
             s.M = rem; s.N = ncol; s.K = NB; s.alpha = -1.0; s.beta = 1.0; s.flags = LOWER_ONLY;
             int rc2;
-            if (split && k128 && ncol <= 0 && rem > NB) {
+            if (ncol <= 0 && rem > NB) {
                 // last panel of the outer block: the next potf2 waits for tile row je of this TRSM and for the
                 // update of tile (je, je) only (diag_next below); the other rows go to the bulk stream
                 GemmParams g1 = g; g1.M = NB;
@@ -460,7 +415,7 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
                 CU(cudaEventRecord(c->ev_p[2], s3));
                 s3_pending = true;
                 boundary_split = true;
-            } else if (!split || ncol <= 0 || rem <= NB) {
+            } else if (ncol <= 0 || rem <= NB) {
                 if ((rc2 = gemm_panel(g, sp, pdl))) return rc2;
                 if ((rc2 = gemm_panel(s, sp, pdl))) return rc2;
             } else {
@@ -470,13 +425,9 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
                 //  the bulk stream picks up after them — it has a full potf2 of slack)
                 GemmParams g1 = g; g1.M = NB;                              // tile row jp+1
                 GemmParams s1 = s; s1.M = NB; s1.N = NB; s1.flags = 0;     // diagonal tile (jp+1, jp+1)
-                if (k128) {                                                // latency kernels: 8 / 16 CTAs, one load group
-                    CU(launch_pdl(gemm_k128_kernel<16, 128>, dim3(1, 8, 1), dim3(128), GemmK128<16, 128>::SMEM_BYTES, sp, pdl, g1)); KL(c);   // in place: whole rows per CTA
-                    CU(launch_pdl(gemm_k128_kernel<32, 32>, dim3(4, 4, 1), dim3(128), GemmK128<32, 32>::SMEM_BYTES, sp, pdl, s1)); KL(c);
-                } else {
-                    if ((rc2 = gemm_panel(g1, sp, pdl))) return rc2;
-                    if ((rc2 = gemm_panel(s1, sp, pdl))) return rc2;
-                }
+                // latency kernels: 8 / 16 CTAs, one load group
+                CU(launch_pdl(gemm_k128_kernel<16, 128>, dim3(1, 8, 1), dim3(128), GemmK128<16, 128>::SMEM_BYTES, sp, pdl, g1)); KL(c);   // in place: whole rows per CTA
+                CU(launch_pdl(gemm_k128_kernel<32, 32>, dim3(4, 4, 1), dim3(128), GemmK128<32, 32>::SMEM_BYTES, sp, pdl, s1)); KL(c);
                 CU(cudaEventRecord(c->ev_p[1], sp));                       // potf2(jp), L[jp+1, jp] final
                 CU(cudaStreamWaitEvent(s3, c->ev_p[1], 0));
                 GemmParams g2 = g; g2.A = P + (int64_t)NB * ld; g2.C = P + (int64_t)NB * ld; g2.M = rem - NB;
@@ -487,18 +438,13 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
                 CU(cudaEventRecord(c->ev_p[2], s3));
                 s3_pending = true;
             }
-            if (s3_pending && jp + 1 < je) {
-                // the next panel's potf2 only needs the diagonal tile; its TRSM needs everything: make the
-                // panel stream wait for the bulk right after that potf2 has been enqueued (below)
-            }
         }
         if (s3_pending && !boundary_split) { CU(cudaStreamWaitEvent(sp, c->ev_p[2], 0)); s3_pending = false; }
-        mark(sp);
         if (je >= T) break;
         SyrkParams u;
         u.C = A; u.ld = ld; u.kcol0 = Jb * NB; u.nk = (je - Jb) * (NB / 16); u.skip_first = 0;
         // ---- U_rest(b) on the second stream: needs panel(b) (event) and, by stream order, U_rest(b-1)
-        const int jn = std::min(je + (ramp ? std::min(step + 2, OB) : OB), T);
+        const int jn = std::min(je + std::min(step + 2, LA_OB), T);
         CU(cudaEventRecord(c->ev_a, sp));
         if (notify_stream && notify_tile > 0 && je >= notify_tile) {
             // every column tile < je of L is final once the panel stream reaches this point (and the bulk rows of the last
@@ -511,10 +457,8 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
             CU(cudaStreamWaitEvent(su, c->ev_a, 0));
             if (boundary_split) CU(cudaStreamWaitEvent(su, c->ev_p[2], 0));   // the bulk rows of the last TRSM
             u.row_t0 = jn; u.col_t0 = jn;
-            mark(su);
             syrk_tma_kernel<<<dim3(T - jn, T - jn), SW_THREADS, SY_SMEM_BYTES, su>>>(tmL, u);
             KL(c);
-            mark(su);
         }
         // ---- U_next(b) on the panel stream: the next block's columns; they were last touched by
         //      U_rest(b-1), so wait for it
@@ -533,7 +477,7 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
             if (rest_pending) CU(cudaStreamWaitEvent(s3, c->ev_b, 0));
             sn = s3; pdl_next = false; u.skip_first = 1;
         }
-        if ((T - je) * (jn - je) <= small_next) {
+        if ((T - je) * (jn - je) <= LA_SMALL_NEXT) {
             // few tiles: one 128x128xK tile per CTA would leave most SMs idle for a full tile time
             // (~55 us); 32-row tiles finish the slab in ~1/3 of that
             GemmParams nx{};
@@ -554,7 +498,6 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
             s3_pending = true;
             boundary_split = false;
         }
-        mark(sp);
         if (jn < T) { CU(cudaEventRecord(c->ev_b, su)); rest_pending = true; }
     }
     if (rest_pending) CU(cudaStreamWaitEvent(sp, c->ev_b, 0));
@@ -564,81 +507,15 @@ int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Din
         CU(cudaEventRecord(c->ev_a, sp));
         CU(cudaStreamWaitEvent(notify_stream, c->ev_a, 0));
     }
-    if (trace) {
-        cudaStreamSynchronize(sp); cudaStreamSynchronize(su);
-        fprintf(stderr, "potrf trace (ms since start), %zu events:", tev.size());
-        for (size_t i = 1; i < tev.size(); ++i) { float ms = 0; cudaEventElapsedTime(&ms, tev[0], tev[i]); fprintf(stderr, " %.3f", ms); }
-        fprintf(stderr, "\n");
-        for (auto e : tev) cudaEventDestroy(e);
-    }
     return ABO_OK;
 }
 
 // ------------------------------------------------------------------------------------------
-// triangular inverse  Linv = L^-1  by recursive doubling on tiles: the diagonal tiles are the
-// block inverses from potf2; at level b (tiles) every pair computes
-//     X21 = - X22 * (L21 * X11)
-// as two batched DMMA GEMMs that skip the structurally-zero k-ranges.  W: scratch, same shape.
-// ------------------------------------------------------------------------------------------
-static int ws_min_n() {
-    static const int v = getenv("ABO_WS_MIN") ? atoi(getenv("ABO_WS_MIN")) : 4096;
-    return v;
-}
-int trtri_blocked(abo_ctx* c, const double* L, double* Linv, double* W, int64_t Npad, int64_t ld, int64_t strideM,
-                  const double* Dinv, int64_t strideD, int batch) {
-    const int T = (int)(Npad / NB);
-    cudaStream_t st = c->stream;
-    // the warp-specialised kernel pays off once the k-loops are long; small / batched problems keep the
-    // lighter barrier-synchronised kernel
-    const bool use_ws = Npad >= ws_min_n();
-    place_diag_kernel<<<dim3(T, batch), 256, 0, st>>>(Dinv, Linv, ld, strideD, strideM);
-    KL(c);
-    for (int b = 1; b < T; b <<= 1) {
-        // pairs start at tile o = 2*b*q; rows22 = [o+b, min(o+2b, T)).  For a single matrix all full
-        // pairs of a level go out as one launch batched over q; a ragged last pair goes separately.
-        const int npairs = (T - b + 2 * b - 1) / (2 * b);          // pairs with a non-empty block 22
-        const int nfull = T / (2 * b);                             // pairs with a full block 22
-        for (int pass = 0; pass < 2; ++pass) {
-            for (int grp = 0; grp < 2; ++grp) {
-                int q0, nq, r22;
-                if (batch == 1) {
-                    if (grp == 0) { q0 = 0; nq = nfull; r22 = b; }
-                    else { q0 = nfull; nq = npairs - nfull; r22 = (nq > 0) ? (T - 2 * b * nfull - b) : 0; }
-                    if (nq <= 0 || r22 <= 0) continue;
-                } else {
-                    if (grp == 1) continue;
-                    q0 = 0; nq = npairs; r22 = b;                  // handled pair by pair below
-                }
-                for (int q = q0; q < q0 + (batch == 1 ? 1 : nq); ++q) {
-                    const int o = 2 * b * q;
-                    const int rr = (batch == 1) ? r22 : (std::min(2 * b, T - o) - b);
-                    const int zb = (batch == 1) ? nq : batch;
-                    const int64_t zs = (batch == 1) ? (int64_t)2 * b * NB * (ld + 1) : strideM;
-                    const int64_t off11 = (int64_t)o * NB * (ld + 1);
-                    const int64_t off22 = (int64_t)(o + b) * NB * (ld + 1);
-                    const int64_t off21 = (int64_t)(o + b) * NB * ld + (int64_t)o * NB;
-                    GemmParams g{};
-                    if (pass == 0) {                              // W21 = L21 * X11   (X11 lower: k >= n)
-                        g.A = L + off21; g.B = Linv + off11; g.C = W + off21;
-                        g.M = rr * NB; g.N = b * NB; g.K = b * NB; g.alpha = 1.0; g.flags = KLO_N;
-                    } else {                                      // X21 = -X22 * W21  (X22 lower: k <= m)
-                        g.A = Linv + off22; g.B = W + off21; g.C = Linv + off21;
-                        g.M = rr * NB; g.N = b * NB; g.K = rr * NB; g.alpha = -1.0; g.flags = KHI_M;
-                    }
-                    g.lda = g.ldb = g.ldc = ld; g.strideA = g.strideB = g.strideC = zs; g.beta = 0.0;
-                    if (use_ws) CU((launch_gemm_ws<KC, MC>(g, zb, st, c->sms))); else CU((launch_gemm<KC, MC, EPI_STORE>(g, zb, st)));
-                    KL(c);
-                }
-            }
-        }
-    }
-    return ABO_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// The same recursion on the TMA pipeline (gemm_tma.cuh): every operand k-contiguous.  Besides X = L^-1 the
-// recursion carries U = X^T (written by the transposed-store epilogue) and keeps the intermediate W21 only as
-// its transpose:     Wt = (L21 U11^T ... ) i.e.  W21^T  <- A = L21, B = U11 (rows of X11^T)
+// triangular inverse  X = L^-1  by recursive doubling on tiles, on the TMA pipeline (gemm_tma.cuh): the diagonal tiles
+// are the block inverses from potf2; at level b (tiles) every pair computes  X21 = - X22 * (L21 * X11)  as two GEMMs that
+// skip the structurally-zero k-ranges.  To keep every operand k-contiguous the recursion also carries U = X^T (written by
+// the transposed-store epilogue) and keeps the intermediate W21 = L21 X11 only as its transpose:
+//                    Wt = W21^T                   <- A = L21, B = U11 (rows of X11^T)
 //                    X21 = -X22 W21               <- A = X22, B = W21^T ;  U12 = X21^T by the same launch
 // Single matrix: all pairs of a level are one launch batched over the pairs; batched matrices (NLML): one
 // launch per pair batched over the matrices.  Wt, U: scratch / output of the shape of L.
@@ -666,25 +543,46 @@ static int launch_gemm_tma(abo_ctx* c, const CUtensorMap& tmA, const CUtensorMap
     KL(c);
     return ABO_OK;
 }
-// which: 0 everything | 1 only levels b < b_stop plus nothing else | (see trtri_split below).  st / max_ctas: stream and CTA cap.
-static int trtri_tma_on(abo_ctx* c, const double* L, double* Linv, double* U, double* Wt, int64_t Npad, int64_t ld, int64_t strideM,
-                        const double* Dinv, int64_t strideD, int batch, cudaStream_t st, int max_ctas);
-int trtri_tma(abo_ctx* c, const double* L, double* Linv, double* U, double* Wt, int64_t Npad, int64_t ld, int64_t strideM,
-              const double* Dinv, int64_t strideD, int batch) {
-    return trtri_tma_on(c, L, Linv, U, Wt, Npad, ld, strideM, Dinv, strideD, batch, c->stream, 0);
+// One pair of the recursion: block 11 = tile rows / columns [o, o + b), block 22 = tile rows [o + b, o + b + rr).  The launch
+// covers zb such pairs, item z displaced by (z rstep, z cstep) elements in the tensor maps and by z zoff doubles in memory.
+struct TrtriPair { int o, b, rr, zb, rstep, cstep; int64_t zoff; };
+// Wt(o, o+b) = (L21 X11)^T : A = L21, B = U11 (k >= n)
+static int trtri_pair_w(abo_ctx* c, const CUtensorMap& tmL, const CUtensorMap& tmU, double* Wt, int64_t ld, const TrtriPair& q,
+                        cudaStream_t st, int max_ctas) {
+    TmaGemmParams g{};
+    g.batch = q.zb; g.alpha = 1.0; g.beta = 0.0;
+    g.Mt = q.rr; g.Nt = q.b; g.K = q.b * NB; g.flags = KLO_N;
+    g.a_row0 = (q.o + q.b) * NB; g.a_col0 = q.o * NB; g.a_rstep = q.rstep; g.a_cstep = q.cstep;
+    g.b_row0 = q.o * NB; g.b_col0 = q.o * NB; g.b_rstep = q.rstep; g.b_cstep = q.cstep;
+    g.C = nullptr; g.CT = Wt; g.ldct = ld; g.ct_off0 = (int64_t)q.o * NB * ld + (int64_t)(q.o + q.b) * NB; g.ct_zstep = q.zoff;
+    return launch_gemm_tma(c, tmL, tmU, g, st, max_ctas);
 }
+// X21 = -X22 W21 (k <= m): A = X22, B = W21^T ; U12 = X21^T
+static int trtri_pair_x(abo_ctx* c, const CUtensorMap& tmX, const CUtensorMap& tmW, double* Linv, double* U, int64_t ld,
+                        const TrtriPair& q, cudaStream_t st, int max_ctas) {
+    TmaGemmParams h{};
+    h.batch = q.zb; h.alpha = -1.0; h.beta = 0.0;
+    h.Mt = q.rr; h.Nt = q.b; h.K = q.rr * NB; h.flags = KHI_M;
+    h.a_row0 = (q.o + q.b) * NB; h.a_col0 = (q.o + q.b) * NB; h.a_rstep = q.rstep; h.a_cstep = q.cstep;
+    h.b_row0 = q.o * NB; h.b_col0 = (q.o + q.b) * NB; h.b_rstep = q.rstep; h.b_cstep = q.cstep;
+    h.C = Linv; h.ldc = ld; h.c_off0 = (int64_t)(q.o + q.b) * NB * ld + (int64_t)q.o * NB; h.c_zstep = q.zoff;
+    h.CT = U; h.ldct = ld; h.ct_off0 = (int64_t)q.o * NB * ld + (int64_t)(q.o + q.b) * NB; h.ct_zstep = q.zoff;
+    return launch_gemm_tma(c, tmX, tmW, h, st, max_ctas);
+}
+// st / max_ctas: stream and CTA cap of every launch
 static int trtri_tma_on(abo_ctx* c, const double* L, double* Linv, double* U, double* Wt, int64_t Npad, int64_t ld, int64_t strideM,
                         const double* Dinv, int64_t strideD, int batch, cudaStream_t st, int max_ctas) {
     const int T = (int)(Npad / NB);
     const int64_t rows = (batch == 1) ? Npad : (int64_t)batch * Npad;        // batched matrices are stacked (strideM = Npad * ld)
     if (batch > 1 && strideM != Npad * ld) return abo_fail(ABO_ERR_INVALID, "trtri_tma: batched matrices must be contiguous");
+    place_diag_both_kernel<<<dim3(T, batch), 256, 0, st>>>(Dinv, Linv, U, ld, strideD, strideM);
+    KL(c);
+    if (T == 1) return ABO_OK;                                              // a single tile: no level, no tensor maps
     CUtensorMap tmL, tmX, tmU, tmW;
     int rc;
     if ((rc = make_tmap_k4(&tmL, L, Npad, rows, ld)) || (rc = make_tmap_k4(&tmX, Linv, Npad, rows, ld)) ||
         (rc = make_tmap_k4(&tmU, U, Npad, rows, ld)) || (rc = make_tmap_k4(&tmW, Wt, Npad, rows, ld)))
         return rc;
-    place_diag_both_kernel<<<dim3(T, batch), 256, 0, st>>>(Dinv, Linv, U, ld, strideD, strideM);
-    KL(c);
     for (int b = 1; b < T; b <<= 1) {
         const int npairs = (T - b + 2 * b - 1) / (2 * b), nfull = T / (2 * b);
         // groups of pairs with equal shapes: (first pair, count, rows of block 22)
@@ -695,32 +593,21 @@ static int trtri_tma_on(abo_ctx* c, const double* L, double* Linv, double* U, do
         for (const Grp& gq : groups) {
             const int launches = (batch == 1) ? 1 : gq.nq;                  // batched matrices: one launch per pair
             for (int li = 0; li < launches; ++li) {
-                const int q = gq.q0 + li;
-                const int o = 2 * b * q;
-                const int zb = (batch == 1) ? gq.nq : batch;
-                const int rstep = (batch == 1) ? 2 * b * NB : (int)Npad, cstep = (batch == 1) ? 2 * b * NB : 0;
-                const int64_t zoff = (batch == 1) ? (int64_t)2 * b * NB * (ld + 1) : strideM;
-                TmaGemmParams g{};
-                g.batch = zb; g.alpha = 1.0; g.beta = 0.0;
-                // Wt(o, o+b) = (L21 X11)^T : A = L21, B = U11 (k >= n)
-                g.Mt = gq.rr; g.Nt = b; g.K = b * NB; g.flags = KLO_N;
-                g.a_row0 = (o + b) * NB; g.a_col0 = o * NB; g.a_rstep = rstep; g.a_cstep = cstep;
-                g.b_row0 = o * NB; g.b_col0 = o * NB; g.b_rstep = rstep; g.b_cstep = cstep;
-                g.C = nullptr; g.CT = Wt; g.ldct = ld; g.ct_off0 = (int64_t)o * NB * ld + (int64_t)(o + b) * NB; g.ct_zstep = zoff;
-                if ((rc = launch_gemm_tma(c, tmL, tmU, g, st, max_ctas))) return rc;
-                // X21 = -X22 W21 (k <= m): A = X22, B = W21^T ; U12 = X21^T
-                TmaGemmParams h{};
-                h.batch = zb; h.alpha = -1.0; h.beta = 0.0;
-                h.Mt = gq.rr; h.Nt = b; h.K = gq.rr * NB; h.flags = KHI_M;
-                h.a_row0 = (o + b) * NB; h.a_col0 = (o + b) * NB; h.a_rstep = rstep; h.a_cstep = cstep;
-                h.b_row0 = o * NB; h.b_col0 = (o + b) * NB; h.b_rstep = rstep; h.b_cstep = cstep;
-                h.C = Linv; h.ldc = ld; h.c_off0 = (int64_t)(o + b) * NB * ld + (int64_t)o * NB; h.c_zstep = zoff;
-                h.CT = U; h.ldct = ld; h.ct_off0 = (int64_t)o * NB * ld + (int64_t)(o + b) * NB; h.ct_zstep = zoff;
-                if ((rc = launch_gemm_tma(c, tmX, tmW, h, st, max_ctas))) return rc;
+                TrtriPair q;
+                q.o = 2 * b * (gq.q0 + li); q.b = b; q.rr = gq.rr;
+                q.zb = (batch == 1) ? gq.nq : batch;
+                q.rstep = (batch == 1) ? 2 * b * NB : (int)Npad; q.cstep = (batch == 1) ? 2 * b * NB : 0;
+                q.zoff = (batch == 1) ? (int64_t)2 * b * NB * (ld + 1) : strideM;
+                if ((rc = trtri_pair_w(c, tmL, tmU, Wt, ld, q, st, max_ctas)) || (rc = trtri_pair_x(c, tmX, tmW, Linv, U, ld, q, st, max_ctas)))
+                    return rc;
             }
         }
     }
     return ABO_OK;
+}
+int trtri_tma(abo_ctx* c, const double* L, double* Linv, double* U, double* Wt, int64_t Npad, int64_t ld, int64_t strideM,
+              const double* Dinv, int64_t strideD, int batch) {
+    return trtri_tma_on(c, L, Linv, U, Wt, Npad, ld, strideM, Dinv, strideD, batch, c->stream, 0);
 }
 
 // beta = Linv * delta ; alpha = Linv^T * beta      (alpha = (K + noise I)^-1 (y - m))
@@ -920,6 +807,8 @@ static KSpec gp_spec(const abo_gp* g) {
 }
 
 static int gp_fit_run(abo_gp* g, const double* X, const double* y, int64_t n, int64_t* info_out);
+constexpr int FIT_OVERLAP_MIN_TILES = 32;   // smallest system (tiles) whose leading inverse runs alongside the factorisation
+constexpr int FIT_OVERLAP_CTAS = 112;       // CTA cap of the overlapped launches: 36 of the 148 SMs stay with the factorisation
 extern "C" int32_t abo_gp_fit(abo_gp* g, const double* X, const double* y, int64_t n, int64_t* info_out) {
     const int rc = gp_fit_run(g, X, y, n, info_out);
     if (rc && g && g->ctx) {
@@ -977,26 +866,20 @@ static int gp_fit_run(abo_gp* g, const double* X, const double* y, int64_t n, in
     // (W21 = L21 X11) only need the leading columns of L, which are final half-way through the factorisation — they run on a
     // low-priority stream with a capped grid while the factorisation's chain-bound tail leaves most SMs idle; the trailing
     // block's inverse and the second product (X21 = -X22 W21) follow once the factorisation is complete.
-    static const bool tma_inv = getenv("ABO_TRTRI_TMA") ? atoi(getenv("ABO_TRTRI_TMA")) != 0 : true;
-    static const int ovl_min = getenv("ABO_FIT_OVERLAP_MIN") ? atoi(getenv("ABO_FIT_OVERLAP_MIN")) : 32;      // tiles; 0 disables
-    static const int ovl_ctas = getenv("ABO_FIT_OVERLAP_CTAS") ? atoi(getenv("ABO_FIT_OVERLAP_CTAS")) : 112;
-    double* U = nullptr;
-    if (tma_inv && T > 1 && (rc = ws_get(c, WS_TRTRI_U, sizeof(double) * (size_t)Npad * Npad, (void**)&U))) return rc;
+    double* U;
+    if ((rc = ws_get(c, WS_TRTRI_U, sizeof(double) * (size_t)Npad * Npad, (void**)&U))) return rc;
     int b_top = 1;
     while (2 * b_top < T) b_top *= 2;                                  // largest power of two below T: the top-level pair is (0, b_top)
-    const bool overlap = U && ovl_min > 0 && T >= ovl_min;
+    const TrtriPair top{0, b_top, T - b_top, 1, 0, 0, 0};
+    const bool overlap = T >= FIT_OVERLAP_MIN_TILES;
     if ((rc = potrf_lookahead(c, g->dL, Npad, g->ld, Dinv, dinfo, overlap ? b_top : 0, overlap ? c->stream4 : nullptr))) return rc;
-    CUtensorMap tmL, tmU;
     if (overlap) {
         cudaStream_t s4 = c->stream4;
         const int64_t nl = (int64_t)b_top * NB;
-        if ((rc = trtri_tma_on(c, g->dL, g->dLinv, U, W, nl, g->ld, 0, Dinv, 0, 1, s4, ovl_ctas))) return rc;
+        if ((rc = trtri_tma_on(c, g->dL, g->dLinv, U, W, nl, g->ld, 0, Dinv, 0, 1, s4, FIT_OVERLAP_CTAS))) return rc;
+        CUtensorMap tmL, tmU;
         if ((rc = make_tmap_k4(&tmL, g->dL, Npad, Npad, g->ld)) || (rc = make_tmap_k4(&tmU, U, Npad, Npad, g->ld))) return rc;
-        TmaGemmParams q{};                                            // Wt(0, b_top) = (L21 X11)^T
-        q.batch = 1; q.alpha = 1.0; q.beta = 0.0; q.Mt = T - b_top; q.Nt = b_top; q.K = b_top * NB; q.flags = KLO_N;
-        q.a_row0 = b_top * NB; q.a_col0 = 0; q.b_row0 = 0; q.b_col0 = 0;
-        q.C = nullptr; q.CT = W; q.ldct = g->ld; q.ct_off0 = (int64_t)b_top * NB;
-        if ((rc = launch_gemm_tma(c, tmL, tmU, q, s4, ovl_ctas))) return rc;
+        if ((rc = trtri_pair_w(c, tmL, tmU, W, g->ld, top, s4, FIT_OVERLAP_CTAS))) return rc;
         CU(cudaEventRecord(c->ev_inv, s4));
     }
     int hinfo = 0;
@@ -1012,15 +895,8 @@ static int gp_fit_run(abo_gp* g, const double* X, const double* y, int64_t n, in
         CU(cudaStreamWaitEvent(st, c->ev_inv, 0));
         CUtensorMap tmX, tmW;
         if ((rc = make_tmap_k4(&tmX, g->dLinv, Npad, Npad, g->ld)) || (rc = make_tmap_k4(&tmW, W, Npad, Npad, g->ld))) return rc;
-        TmaGemmParams h{};                                            // X21 = -X22 W21 ;  U12 = X21^T
-        h.batch = 1; h.alpha = -1.0; h.beta = 0.0; h.Mt = T - b_top; h.Nt = b_top; h.K = (T - b_top) * NB; h.flags = KHI_M;
-        h.a_row0 = b_top * NB; h.a_col0 = b_top * NB; h.b_row0 = 0; h.b_col0 = b_top * NB;
-        h.C = g->dLinv; h.ldc = g->ld; h.c_off0 = (int64_t)b_top * NB * g->ld;
-        h.CT = U; h.ldct = g->ld; h.ct_off0 = (int64_t)b_top * NB;
-        if ((rc = launch_gemm_tma(c, tmX, tmW, h, st))) return rc;
-    } else if (U) {
-        if ((rc = trtri_tma(c, g->dL, g->dLinv, U, W, Npad, g->ld, 0, Dinv, 0, 1))) return rc;
-    } else if ((rc = trtri_blocked(c, g->dL, g->dLinv, W, Npad, g->ld, 0, Dinv, 0, 1))) return rc;
+        if ((rc = trtri_pair_x(c, tmX, tmW, g->dLinv, U, g->ld, top, st, 0))) return rc;
+    } else if ((rc = trtri_tma(c, g->dL, g->dLinv, U, W, Npad, g->ld, 0, Dinv, 0, 1))) return rc;
     if ((rc = solve_alpha(c, g->dLinv, g->ld, Npad, g->dDelta, g->dBeta, g->dAlpha, 0, 0, 1))) return rc;
     CU(cudaStreamSynchronize(st));
     g->fitted = true;
@@ -1311,7 +1187,7 @@ extern "C" int32_t abo_acq_eval_grad(abo_gp* g, int32_t acq_id, const double* pa
         GemmParams z{};                                        // Z = L^-T W      (k >= row)
         z.A = g->dLinv; z.lda = g->ld; z.B = W; z.ldb = mpad; z.C = Z; z.ldc = mpad;
         z.M = (int)Npad; z.N = (int)mpad; z.K = (int)Npad; z.alpha = 1.0; z.beta = 0.0; z.flags = KLO_M;
-        CU((launch_gemm<MC, MC, EPI_STORE>(z, 1, st)));
+        CU((launch_gemm(z, 1, st)));
         KL(c);
         acq_grad_partial_kernel<<<dim3(npbg, (unsigned)mpad), 128, 0, st>>>(gp_spec(g), g->dXsT, g->ldx, g->n, g->dAlpha, Z,
                                                                            mpad, dXc + c0 * d, mvalid, part);
@@ -1362,7 +1238,7 @@ extern "C" int32_t abo_gp_posterior_cov(abo_gp* g, const double* Xc, int64_t m, 
     GemmParams q{};                                                // G = W^T W
     q.A = W; q.lda = Mpad; q.B = W; q.ldb = Mpad; q.C = G; q.ldc = Mpad;
     q.M = (int)Mpad; q.N = (int)Mpad; q.K = (int)Npad; q.alpha = 1.0; q.beta = 0.0; q.flags = 0;
-    CU((launch_gemm<MC, MC, EPI_STORE>(q, 1, st)));
+    CU((launch_gemm(q, 1, st)));
     KL(c);
     const int64_t Mo = m * outputs;
     cov_finish_kernel<<<(unsigned)((Mo * Mo + 255) / 256), 256, 0, st>>>(gp_spec(g), dXc, m, outputs, mp, G, Mpad, dcov);

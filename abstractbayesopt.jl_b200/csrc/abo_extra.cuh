@@ -276,14 +276,13 @@ static int nlml_batch_impl(abo_gp* g, const double* X, const double* y, int64_t 
     size_t budget = std::min<size_t>((size_t)24 << 30, free_b / 2);
     int64_t Rc = std::max<int64_t>(1, std::min<int64_t>(R, (int64_t)(budget / (4 * mat))));
     int rc;
-    double *Kb, *Linv, *W, *Xb, *vec, *par, *Dinv, *dXraw, *dYraw;
+    double *Kb, *Linv, *W, *Ub, *Xb, *vec, *par, *Dinv, *dXraw, *dYraw;
     int* dinfo;
     if ((rc = ws_get(c, WS_NLML_K, mat * Rc, (void**)&Kb))) return rc;
     if ((rc = ws_get(c, WS_NLML_LINV, mat * Rc, (void**)&Linv))) return rc;
     if ((rc = ws_get(c, WS_NLML_W, mat * Rc, (void**)&W))) return rc;
-    static const bool tma_inv = getenv("ABO_TRTRI_TMA") ? atoi(getenv("ABO_TRTRI_TMA")) != 0 : true;
-    double* Ub = nullptr;                                 // U = (L^-1)^T of every matrix: keeps all GEMM operands k-contiguous (gemm_tma.cuh)
-    if (tma_inv && T > 1 && (rc = ws_get(c, WS_NLML_U, mat * Rc, (void**)&Ub))) return rc;
+    // U = (L^-1)^T of every matrix: keeps all GEMM operands k-contiguous (gemm_tma.cuh)
+    if ((rc = ws_get(c, WS_NLML_U, mat * Rc, (void**)&Ub))) return rc;
     if ((rc = ws_get(c, WS_NLML_X, sizeof(double) * (size_t)Rc * ldx * d, (void**)&Xb))) return rc;
     // vec: delta[Rc][Npad] | beta | alpha | out[Rc][1 + np]
     if ((rc = ws_get(c, WS_NLML_VEC, sizeof(double) * (size_t)Rc * (3 * Npad + 2 + np_), (void**)&vec))) return rc;
@@ -321,30 +320,20 @@ static int nlml_batch_impl(abo_gp* g, const double* X, const double* y, int64_t 
         KmatBatch bt{sb, scb, ldx * d, Npad * Npad, ard ? 1 : 0};
         launch_kmat(spec, Xb, ldx, N, Kb, Npad, bt, T, nb, st);
         KL(c);
-        if ((rc = potrf_blocked(c, Kb, Npad, Npad, Npad * Npad, Dinv, (int64_t)T * NB * NB, dinfo, nb))) return rc;
-        if (Ub) { if ((rc = trtri_tma(c, Kb, Linv, Ub, W, Npad, Npad, Npad * Npad, Dinv, (int64_t)T * NB * NB, nb))) return rc; }
-        else if ((rc = trtri_blocked(c, Kb, Linv, W, Npad, Npad, Npad * Npad, Dinv, (int64_t)T * NB * NB, nb))) return rc;
+        if ((rc = potrf_blocked(c, Kb, Npad, Npad, Dinv, dinfo, nb))) return rc;
+        if ((rc = trtri_tma(c, Kb, Linv, Ub, W, Npad, Npad, Npad * Npad, Dinv, (int64_t)T * NB * NB, nb))) return rc;
         if ((rc = solve_alpha(c, Linv, Npad, Npad, delta, beta, alpha, Npad * Npad, Npad, nb))) return rc;
         if (grad) {
-            GemmParams q{};                                        // Cinv = Linv^T Linv, lower tiles, k >= m
-            q.A = Linv; q.B = Linv; q.C = W;
-            q.lda = q.ldb = q.ldc = Npad; q.strideA = q.strideB = q.strideC = Npad * Npad;
-            q.M = q.N = q.K = (int)Npad; q.alpha = 1.0; q.beta = 0.0; q.flags = KLO_M | LOWER_ONLY;
-            if (Ub) {
-                // Cinv[m][n] = sum_k X[k][m] X[k][n] = sum_{k >= m} U[m][k] U[n][k]: both operands rows of U, k-contiguous
-                CUtensorMap tmU;
-                if ((rc = make_tmap_k4(&tmU, Ub, Npad, (int64_t)nb * Npad, Npad))) return rc;
-                TmaGemmParams t{};
-                t.Mt = T; t.Nt = T; t.batch = nb; t.K = (int)Npad; t.flags = KLO_M | LOWER_ONLY; t.alpha = 1.0; t.beta = 0.0;
-                t.a_row0 = 0; t.a_rstep = (int)Npad; t.a_col0 = 0; t.a_cstep = 0;
-                t.b_row0 = 0; t.b_rstep = (int)Npad; t.b_col0 = 0; t.b_cstep = 0;
-                t.C = W; t.ldc = Npad; t.c_off0 = 0; t.c_zstep = Npad * Npad;
-                if ((rc = launch_gemm_tma(c, tmU, tmU, t, st))) return rc;
-            } else {
-                if (Npad >= ws_min_n()) CU((launch_gemm_ws<MC, MC>(q, nb, st, c->sms)));
-                else CU((launch_gemm<MC, MC, EPI_STORE>(q, nb, st)));
-                KL(c);
-            }
+            // Cinv = Linv^T Linv, lower tiles:  Cinv[m][n] = sum_k X[k][m] X[k][n] = sum_{k >= m} U[m][k] U[n][k]: both operands
+            // rows of U, k-contiguous
+            CUtensorMap tmU;
+            if ((rc = make_tmap_k4(&tmU, Ub, Npad, (int64_t)nb * Npad, Npad))) return rc;
+            TmaGemmParams t{};
+            t.Mt = T; t.Nt = T; t.batch = nb; t.K = (int)Npad; t.flags = KLO_M | LOWER_ONLY; t.alpha = 1.0; t.beta = 0.0;
+            t.a_row0 = 0; t.a_rstep = (int)Npad; t.a_col0 = 0; t.a_cstep = 0;
+            t.b_row0 = 0; t.b_rstep = (int)Npad; t.b_col0 = 0; t.b_cstep = 0;
+            t.C = W; t.ldc = Npad; t.c_off0 = 0; t.c_zstep = Npad * Npad;
+            if ((rc = launch_gemm_tma(c, tmU, tmU, t, st))) return rc;
             if (ard) {
                 const dim3 grid(T, T, nb);
                 if (d <= 8) nlml_grad_ard_kernel<8><<<grid, 256, 0, st>>>(spec, bt, Xb, ldx, N, W, Npad, Npad * Npad, alpha, Npad, tpart);
@@ -369,7 +358,7 @@ static int nlml_batch_impl(abo_gp* g, const double* X, const double* y, int64_t 
             if (info) info[r0 + b] = hinfo[b];
         }
     }
-    if (3 * mat * Rc > ((size_t)16 << 30)) {       // an optimiser calls this in a loop: keep up to 16 GB of scratch resident
+    if (4 * mat * Rc > ((size_t)16 << 30)) {       // an optimiser calls this in a loop: keep up to 16 GB of scratch resident
         ws_release(c, WS_NLML_K); ws_release(c, WS_NLML_LINV); ws_release(c, WS_NLML_W); ws_release(c, WS_NLML_U);
     }
     return ABO_OK;

@@ -97,10 +97,7 @@ void ws_release(abo_ctx* c, int slot);
 int ws_get(abo_ctx* c, int slot, size_t bytes, void** out);
 int pinned_get(abo_ctx* c, size_t bytes, void** out);
 int potrf_lookahead(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Dinv, int* info, int notify_tile = 0, cudaStream_t notify_stream = nullptr);
-int potrf_blocked(abo_ctx* c, double* A, int64_t Npad, int64_t ld, int64_t strideA, double* Dinv, int64_t strideD,
-                  int* info, int batch);
-int trtri_blocked(abo_ctx* c, const double* L, double* Linv, double* W, int64_t Npad, int64_t ld, int64_t strideM,
-                  const double* Dinv, int64_t strideD, int batch);
+int potrf_blocked(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Dinv, int* info, int batch);
 int trtri_tma(abo_ctx* c, const double* L, double* Linv, double* U, double* Wt, int64_t Npad, int64_t ld, int64_t strideM,
               const double* Dinv, int64_t strideD, int batch);
 int solve_alpha(abo_ctx* c, const double* Linv, int64_t ld, int64_t N, const double* delta, double* beta,

@@ -1,15 +1,17 @@
-// gemm_dmma.cuh — FP64 tensor-core (DMMA.8x8x4) tile engine shared by every O(n^3) step of the
-// path: SYRK trailing update and panel TRSM of the blocked Cholesky, the triangular inverse,
-// K^-1 = L^-T L^-1 for the NLML gradient and the W = L^-1 K*, Z = L^-T W products of the
-// acquisition-gradient path.  (The candidate sweep itself runs on the TMA/mbarrier kernel of
-// sweep_tma.cuh, which shares the shared-memory tile layout and the DMMA inner loop.)
+// gemm_dmma.cuh — FP64 tensor-core (DMMA.8x8x4) GEMMs staged by cp.async:
+//   gemm_dmma_kernel                       MN-contiguous operands: Z = L^-T W of the acquisition gradient
+//                                          (abo_acq_eval_grad), G = W^T W of the posterior covariance;
+//   gemm_small_kernel, gemm_k128_kernel    K-contiguous operands: the panel TRSM / SYRK of the look-ahead Cholesky.
+// (The candidate sweep, the trailing updates, the batched Cholesky, the triangular inverse and K^-1 = L^-T L^-1 run
+// on the TMA/mbarrier kernels of sweep_tma.cuh / gemm_tma.cuh, which share the shared-memory tile layout and the
+// DMMA inner loop.)
 //
 // tcgen05 has no f64 kind, so on sm_100a FP64 tensor work is the warp-level
 // mma.sync.m8n8k4.f64 (SASS DMMA.8x8x4; the m16n8k{4,8,16} PTX shapes lower to the same SASS
 // instruction).  Measured issue peak on this pool: 36.9 TFLOP/s (profiles/fp64_peaks_r01.json).
 //
-// CTA tile 128 x 128, K step 16, 256 threads = 8 warps (4 along M x 2 along N), warp tile
-// 32 x 64 = 4 x 8 DMMA tiles (64 accumulator doubles / thread), 4-stage cp.async pipeline.
+// gemm_dmma_kernel: CTA tile 128 x 128, K step 16, 256 threads = 8 warps (4 along M x 2 along N), warp
+// tile 32 x 64 = 4 x 8 DMMA tiles (64 accumulator doubles / thread), 4-stage cp.async pipeline.
 // Shared-memory tiles are laid out so that every fragment load is conflict-free:
 //   K-contiguous operand (element (r,k) at r*ld + k in HBM)  -> smem [k/4][r][k%4]
 //        a fragment (8 rows x 4 k) is one 256-byte contiguous run
@@ -22,11 +24,9 @@
 namespace abo {
 
 constexpr int BM = 128, BN = 128, BK = 16, STAGES = 4, GEMM_THREADS = 256;
-constexpr int TILE_DOUBLES = 16 * 132;   // per operand per stage (covers both layouts)
+constexpr int TILE_DOUBLES = 16 * 132;   // per operand per stage: [k][132]
 constexpr int GEMM_SMEM_BYTES = STAGES * 2 * TILE_DOUBLES * (int)sizeof(double);
 
-enum Layout { KC = 0, MC = 1 };
-enum Epilogue { EPI_STORE = 0 };
 enum GemmFlags {
     KLO_M = 1,        // k starts at the tile's first row      (A^T-type lower operands)
     KLO_N = 2,        // k starts at the tile's first column   (B lower triangular, k >= n)
@@ -64,34 +64,24 @@ __device__ __forceinline__ void dmma8x8x4(double& c0, double& c1, double a, doub
                  : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
-// one 128 x 16 operand tile -> smem, 4 x 16-byte cp.async per thread
-template <int LAYOUT>
+// one 128 x 16 tile of an MN-contiguous operand -> smem, 4 x 16-byte cp.async per thread
 __device__ __forceinline__ void load_tile(double* s, const double* g, int64_t ld, int r0, int k0, int tid) {
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
         int c = tid + GEMM_THREADS * q;
-        if (LAYOUT == KC) {
-            int row = c >> 3, ch = c & 7;                    // 8 chunks of 2 doubles per row
-            const double* src = g + (int64_t)(r0 + row) * ld + k0 + 2 * ch;
-            double* dst = s + (((ch >> 1) * 128 + row) << 2) + ((ch & 1) << 1);
-            cp_async16(dst, src);
-        } else {
-            int krow = c >> 6, ch = c & 63;                  // 64 chunks per k-row
-            const double* src = g + (int64_t)(k0 + krow) * ld + r0 + 2 * ch;
-            double* dst = s + krow * 132 + 2 * ch;
-            cp_async16(dst, src);
-        }
+        int krow = c >> 6, ch = c & 63;                      // 64 chunks per k-row
+        const double* src = g + (int64_t)(k0 + krow) * ld + r0 + 2 * ch;
+        double* dst = s + krow * 132 + 2 * ch;
+        cp_async16(dst, src);
     }
 }
 
-template <int LAYOUT>
 __device__ __forceinline__ double frag(const double* s, int kk, int r, int lane) {
     // element (row = r + lane/4, k = 4*kk + lane%4)
-    if (LAYOUT == KC) return s[((kk * 128 + r + (lane >> 2)) << 2) + (lane & 3)];
     return s[(kk * 4 + (lane & 3)) * 132 + r + (lane >> 2)];
 }
 
-template <int LA, int LB, int EPI>
+// C = alpha * A^T B + beta * C  with A[k][m] at A + k lda + m and B[k][n] at B + k ldb + n
 __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_dmma_kernel(GemmParams p) {
     extern __shared__ __align__(16) double smem[];
     double* sA = smem;
@@ -119,8 +109,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_dmma_kernel(GemmParams p
 #pragma unroll
     for (int s = 0; s < STAGES - 1; ++s) {
         if (s < nk) {
-            load_tile<LA>(sA + s * TILE_DOUBLES, A, p.lda, m0, klo + s * BK, tid);
-            load_tile<LB>(sB + s * TILE_DOUBLES, B, p.ldb, n0, klo + s * BK, tid);
+            load_tile(sA + s * TILE_DOUBLES, A, p.lda, m0, klo + s * BK, tid);
+            load_tile(sB + s * TILE_DOUBLES, B, p.ldb, n0, klo + s * BK, tid);
         }
         cp_async_commit();
     }
@@ -132,8 +122,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_dmma_kernel(GemmParams p
             int nxt = kt + STAGES - 1;
             if (nxt < nk) {
                 int s = nxt % STAGES;
-                load_tile<LA>(sA + s * TILE_DOUBLES, A, p.lda, m0, klo + nxt * BK, tid);
-                load_tile<LB>(sB + s * TILE_DOUBLES, B, p.ldb, n0, klo + nxt * BK, tid);
+                load_tile(sA + s * TILE_DOUBLES, A, p.lda, m0, klo + nxt * BK, tid);
+                load_tile(sB + s * TILE_DOUBLES, B, p.ldb, n0, klo + nxt * BK, tid);
             }
             cp_async_commit();
         }
@@ -143,9 +133,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_dmma_kernel(GemmParams p
         for (int kk = 0; kk < 4; ++kk) {
             double a[4], b[8];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) a[i] = frag<LA>(a_s, kk, wm + i * 8, lane);
+            for (int i = 0; i < 4; ++i) a[i] = frag(a_s, kk, wm + i * 8, lane);
 #pragma unroll
-            for (int j = 0; j < 8; ++j) b[j] = frag<LB>(b_s, kk, wn + j * 8, lane);
+            for (int j = 0; j < 8; ++j) b[j] = frag(b_s, kk, wn + j * 8, lane);
 #pragma unroll
             for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -154,25 +144,23 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_dmma_kernel(GemmParams p
     }
     cp_async_wait<0>();
 
-    if (EPI == EPI_STORE) {
-        double* C = p.C + (int64_t)blockIdx.z * p.strideC;
+    double* C = p.C + (int64_t)blockIdx.z * p.strideC;
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            int row = m0 + wm + i * 8 + (lane >> 2);
+    for (int i = 0; i < 4; ++i) {
+        int row = m0 + wm + i * 8 + (lane >> 2);
 #pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                int col = n0 + wn + j * 8 + 2 * (lane & 3);
-                double2* dst = reinterpret_cast<double2*>(C + (int64_t)row * p.ldc + col);
-                double2 v;
-                v.x = p.alpha * acc[i][j][0];
-                v.y = p.alpha * acc[i][j][1];
-                if (p.beta != 0.0) {
-                    double2 o = *dst;
-                    v.x += p.beta * o.x;
-                    v.y += p.beta * o.y;
-                }
-                *dst = v;
+        for (int j = 0; j < 8; ++j) {
+            int col = n0 + wn + j * 8 + 2 * (lane & 3);
+            double2* dst = reinterpret_cast<double2*>(C + (int64_t)row * p.ldc + col);
+            double2 v;
+            v.x = p.alpha * acc[i][j][0];
+            v.y = p.alpha * acc[i][j][1];
+            if (p.beta != 0.0) {
+                double2 o = *dst;
+                v.x += p.beta * o.x;
+                v.y += p.beta * o.y;
             }
+            *dst = v;
         }
     }
 }
@@ -281,14 +269,6 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? 4 : 2) gemm_small_kernel(Ge
     }
 }
 
-template <int BMT, int NW>
-inline cudaError_t launch_gemm_small(const GemmParams& p, int batch, cudaStream_t st) {
-    if (p.M <= 0 || p.N <= 0 || batch <= 0) return cudaSuccess;
-    dim3 grid(p.N / BN, p.M / BMT, batch);
-    gemm_small_kernel<BMT, NW><<<grid, NW * 32, GemmS<BMT, NW>::SMEM_BYTES, st>>>(p);
-    return cudaGetLastError();
-}
-
 // ------------------------------------------------------------------------------------------
 // Latency kernels for the two GEMMs on the critical chain of the Cholesky (next diagonal tile: TRSM-as-GEMM and
 // its SYRK, M = N = K = 128): small TM x TN output tiles -> 8 / 16 CTAs of 4 warps, the whole k-range staged by
@@ -357,17 +337,10 @@ __global__ void __launch_bounds__(128) gemm_k128_kernel(GemmParams p) {
         }
 }
 
-template <int LA, int LB, int EPI>
-inline cudaError_t configure_gemm() {   // per device: opt in to > 48 KB dynamic shared memory
-    return cudaFuncSetAttribute(gemm_dmma_kernel<LA, LB, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                GEMM_SMEM_BYTES);
-}
-
-template <int LA, int LB, int EPI>
 inline cudaError_t launch_gemm(const GemmParams& p, int batch, cudaStream_t st) {
     if (p.M <= 0 || p.N <= 0 || batch <= 0) return cudaSuccess;
     dim3 grid(p.N / BN, p.M / BM, batch);
-    gemm_dmma_kernel<LA, LB, EPI><<<grid, GEMM_THREADS, GEMM_SMEM_BYTES, st>>>(p);
+    gemm_dmma_kernel<<<grid, GEMM_THREADS, GEMM_SMEM_BYTES, st>>>(p);
     return cudaGetLastError();
 }
 

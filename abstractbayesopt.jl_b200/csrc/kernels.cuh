@@ -547,15 +547,6 @@ __global__ void __launch_bounds__(512) potf2_ws_kernel(double* __restrict__ Ablk
     if (stamp) g_potf2_clk[6] = clock64();
 }
 
-// copy the T diagonal-block inverses into the diagonal tiles of Linv
-__global__ void place_diag_kernel(const double* __restrict__ Dinv, double* __restrict__ Linv, int64_t ld,
-                                  int64_t strideD, int64_t strideL) {
-    const int t = blockIdx.x;
-    const double* src = Dinv + (int64_t)blockIdx.y * strideD + (int64_t)t * NB * NB;
-    double* dst = Linv + (int64_t)blockIdx.y * strideL + (int64_t)t * NB * (ld + 1);
-    for (int e = threadIdx.x; e < NB * NB; e += blockDim.x) dst[(int64_t)(e >> 7) * ld + (e & 127)] = src[e];
-}
-
 // ------------------------------------------------------------------------------------------
 // O(n^2) vector kernels on row-major lower-triangular matrices
 // ------------------------------------------------------------------------------------------

@@ -299,173 +299,3 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmL, SyrkParams p) {
 
 
 }  // namespace abo
-
-// ------------------------------------------------------------------------------------------
-// gemm_ws_kernel<LA, LB> — warp-specialised general tile GEMM  C = alpha * A op(B) + beta * C  for the
-// operand layouts TMA boxes cannot stage conflict-free (MN-contiguous operands of the triangular
-// inverse and of L^-T L^-1): two PRODUCER warps issue 16-byte cp.async copies into the same
-// shared-memory layouts as gemm_dmma_kernel and signal an mbarrier ring with
-// cp.async.mbarrier.arrive; eight CONSUMER warps run the DMMA inner loop of the sweep kernel with no
-// block-wide barrier.  One 128 x 128 tile per CTA; k-range flags as in gemm_dmma.cuh.
-// ------------------------------------------------------------------------------------------
-namespace abo {
-
-constexpr int WS_STAGES = 5;
-constexpr int WS_THREADS = 256 + 64;
-constexpr int WS_SMEM_BYTES = WS_STAGES * 2 * TILE_DOUBLES * (int)sizeof(double) + 2 * WS_STAGES * 8 + 64;
-
-template <int LAYOUT>
-__device__ __forceinline__ void ws_load_tile(double* s, const double* g, int64_t ld, int r0, int k0, int lane) {
-    // one warp copies a 128 x 16 operand tile: 1024 chunks of 16 bytes, 32 per lane
-#pragma unroll 8
-    for (int q = 0; q < 32; ++q) {
-        const int c = lane + 32 * q;
-        if (LAYOUT == KC) {
-            const int row = c >> 3, ch = c & 7;
-            cp_async16(s + (((ch >> 1) * 128 + row) << 2) + ((ch & 1) << 1), g + (int64_t)(r0 + row) * ld + k0 + 2 * ch);
-        } else {
-            const int krow = c >> 6, ch = c & 63;
-            cp_async16(s + krow * 132 + 2 * ch, g + (int64_t)(k0 + krow) * ld + r0 + 2 * ch);
-        }
-    }
-}
-
-// persistent tile schedule: the launch covers `total` = batch x tiles-per-matrix work items, CTA c
-// runs items c, 2 grid - 1 - c, 2 grid + c, ... (serpentine).  Items are ordered heaviest first (longest k-range) with the batch
-// index fastest, so a static round-robin hands every CTA one item of each weight class:
-//   LOWER_ONLY (square, k >= m with KLO_M): triangular enumeration, rows ascending
-//   KLO_N: column-major ascending n      KHI_M: row-major descending m      else: row-major
-struct WsTile { int m0, n0, z, klo, nk; };
-__device__ __forceinline__ WsTile ws_decode(const GemmParams& p, int t, int Mt, int Nt, int batch) {
-    WsTile w;
-    w.z = t % batch;
-    const int tl = t / batch;
-    int mt, nt;
-    if (p.flags & LOWER_ONLY) {
-        mt = (int)((sqrt(8.0 * tl + 1.0) - 1.0) * 0.5);
-        while ((mt + 1) * (mt + 2) / 2 <= tl) ++mt;
-        while (mt * (mt + 1) / 2 > tl) --mt;
-        nt = tl - mt * (mt + 1) / 2;
-    } else if (p.flags & KLO_N) { nt = tl / Mt; mt = tl % Mt; }
-    else if (p.flags & KHI_M) { mt = Mt - 1 - tl / Nt; nt = tl % Nt; }
-    else { mt = tl / Nt; nt = tl % Nt; }
-    w.m0 = mt * BM; w.n0 = nt * BN;
-    int klo = 0, khi = p.K;
-    if (p.flags & KLO_M) klo = w.m0;
-    if ((p.flags & KLO_N) && w.n0 > klo) klo = w.n0;
-    if ((p.flags & KHI_M) && w.m0 + BM < khi) khi = w.m0 + BM;
-    w.klo = klo;
-    w.nk = (khi > klo) ? (khi - klo) / BK : 0;
-    return w;
-}
-
-template <int LA, int LB>
-__global__ void __launch_bounds__(WS_THREADS, 1) gemm_ws_kernel(GemmParams p, int Mt, int Nt, int batch, int total) {
-    extern __shared__ __align__(128) unsigned char ws_smem[];
-    double* sA = reinterpret_cast<double*>(ws_smem);
-    double* sB = sA + WS_STAGES * TILE_DOUBLES;
-    uint64_t* full = reinterpret_cast<uint64_t*>(ws_smem + WS_STAGES * 2 * TILE_DOUBLES * sizeof(double));
-    uint64_t* empty = full + WS_STAGES;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-    if (tid == 0) {
-        for (int s = 0; s < WS_STAGES; ++s) { mbar_init(&full[s], 64); mbar_init(&empty[s], 8); }
-        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    }
-    __syncthreads();
-
-    int stage = 0;
-    uint32_t phase = 0;
-    if (warp >= 8) {
-        // ------------------------------ cp.async producers (warp 8: A, warp 9: B) ------------------------------
-        for (int rnd = 0;; ++rnd) {
-            const int t = rnd * (int)gridDim.x + ((rnd & 1) ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x);
-            if (t >= total) { if (rnd * (int)gridDim.x >= total) break; continue; }
-            const WsTile w = ws_decode(p, t, Mt, Nt, batch);
-            const double* A = p.A + (int64_t)w.z * p.strideA;
-            const double* B = p.B + (int64_t)w.z * p.strideB;
-            for (int kt = 0; kt < w.nk; ++kt) {
-                mbar_wait(&empty[stage], phase ^ 1);
-                if (warp == 8) ws_load_tile<LA>(sA + stage * TILE_DOUBLES, A, p.lda, w.m0, w.klo + kt * BK, lane);
-                else ws_load_tile<LB>(sB + stage * TILE_DOUBLES, B, p.ldb, w.n0, w.klo + kt * BK, lane);
-                asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];\n" ::"r"(smem_u32(&full[stage])) : "memory");
-                if (++stage == WS_STAGES) { stage = 0; phase ^= 1; }
-            }
-        }
-        asm volatile("cp.async.wait_all;\n" ::: "memory");      // do not retire with copies (and their arrives) in flight
-        return;
-    }
-
-    const int wm = (warp & 3) * 32, wn = (warp >> 2) * 64;
-    for (int rnd = 0;; ++rnd) {                     // serpentine: odd rounds run the CTAs in reverse order
-        const int t = rnd * (int)gridDim.x + ((rnd & 1) ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x);
-        if (t >= total) { if (rnd * (int)gridDim.x >= total) break; continue; }
-        const WsTile w = ws_decode(p, t, Mt, Nt, batch);
-        double acc[4][8][2];
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 8; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
-        for (int kt = 0; kt < w.nk; ++kt) {
-            mbar_wait(&full[stage], phase);
-            const double* a_s = sA + stage * TILE_DOUBLES;
-            const double* b_s = sB + stage * TILE_DOUBLES;
-            double a[2][4], bb[2][8];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) a[0][i] = frag<LA>(a_s, 0, wm + i * 8, lane);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) bb[0][j] = frag<LB>(b_s, 0, wn + j * 8, lane);
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk) {
-                const int cur = kk & 1, nxt = cur ^ 1;
-                if (kk < 3) {
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) a[nxt][i] = frag<LA>(a_s, kk + 1, wm + i * 8, lane);
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) bb[nxt][j] = frag<LB>(b_s, kk + 1, wn + j * 8, lane);
-                }
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) dmma8x8x4(acc[i][j][0], acc[i][j][1], a[cur][i], bb[cur][j]);
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty[stage]);
-            if (++stage == WS_STAGES) { stage = 0; phase ^= 1; }
-        }
-        double* C = p.C + (int64_t)w.z * p.strideC;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int row = w.m0 + wm + i * 8 + (lane >> 2);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const int col = w.n0 + wn + j * 8 + 2 * (lane & 3);
-                double2* dst = reinterpret_cast<double2*>(C + (int64_t)row * p.ldc + col);
-                double2 v;
-                v.x = p.alpha * acc[i][j][0];
-                v.y = p.alpha * acc[i][j][1];
-                if (p.beta != 0.0) {
-                    double2 o = *dst;
-                    v.x += p.beta * o.x;
-                    v.y += p.beta * o.y;
-                }
-                *dst = v;
-            }
-        }
-    }
-}
-
-// sms: CTAs to launch at most (one persistent CTA per SM).  LOWER_ONLY needs a square tile grid.
-template <int LA, int LB>
-inline cudaError_t launch_gemm_ws(const GemmParams& p, int batch, cudaStream_t st, int sms) {
-    if (p.M <= 0 || p.N <= 0 || batch <= 0) return cudaSuccess;
-    const int Mt = p.M / BM, Nt = p.N / BN;
-    const int64_t per = (p.flags & LOWER_ONLY) ? (int64_t)Mt * (Mt + 1) / 2 : (int64_t)Mt * Nt;
-    const int64_t total = per * batch;
-    if (total > 0x7fffffff) return cudaErrorInvalidValue;
-    const int grid = (int)std::min<int64_t>(total, sms);
-    gemm_ws_kernel<LA, LB><<<grid, WS_THREADS, WS_SMEM_BYTES, st>>>(p, Mt, Nt, batch, (int)total);
-    return cudaGetLastError();
-}
-
-}  // namespace abo

@@ -1,5 +1,5 @@
 """abo_gp_fit at the tile counts T = ceil(N / 128), N = n p, where its conditioning schedule changes.  From T = 32 on
-(ABO_FIT_OVERLAP_MIN) the triangular inverse of the leading b_top tile columns (b_top: the largest power of two below T)
+(FIT_OVERLAP_MIN_TILES) the triangular inverse of the leading b_top tile columns (b_top: the largest power of two below T)
 runs on a second stream while the Cholesky factorisation finishes.  That stream is ordered after the factorisation at
 the first outer-block boundary in [b_top, T) or, where the ramped boundaries 1, 3, 6, 9, ... leave none there
 (T = 33, 65, 66, 129, ...), after the whole factor.  Each fit is checked against the CPU oracle on the same data: the

@@ -292,8 +292,8 @@ def test_gradient_gp_known_answer(abo, orc):
 
 
 def test_potrf_dev(abo):
-    """The look-ahead Cholesky at tile counts T = n / 128 on every branch of its schedule: T <= OB = 3 (one blocked
-    call), the outer-block ramp 1, 2, 3 (T = 4, 5, 7, 8, 17), around the overlapped inverse's b_top = 32 (31-33), the PDL
+    """The look-ahead Cholesky at tile counts T = n / 128 on every branch of its schedule: T <= 3 (inside the first
+    outer blocks of the ramp), the outer-block ramp 1, 2, 3 (T = 4, 5, 7, 8, 17), around the overlapped inverse's b_top = 32 (31-33), the PDL
     threshold of 40 trailing tiles (40, 41) and the 64-row panel GEMMs of panels with 4096 rows or more (33 on; 44, 64-66).
     Against LAPACK, by the backward error |L L^T - A| <= N eps max|A| (gamma_{N+1}), and bit-identical when repeated."""
     import torch
