@@ -9,11 +9,11 @@ from .kernels import (ADMatern52Kernel, ADMatern72Kernel, ApproxMatern52Kernel, 
                       extract_scale_and_lengthscale)
 from .surrogates import (AbstractSurrogate, GradientGP, StandardGP, get_kernel_constructor, get_lengthscale,
                          get_mean_std, get_scale, is_ard, nlml, nlml_batch, nlml_ls, posterior_grad_mean,
-                         posterior_grad_var, posterior_grad_cov, posterior_cov, posterior_mean, posterior_var, prep_input, prep_output, rescale_model,
-                         std_y, unstandardized_mean_and_var, update_surrogate, empty_posterior_like, _get_minimum,
+                         posterior_grad_var, posterior_grad_cov, posterior_cov, posterior_mean, posterior_sample, posterior_var, prep_input, prep_output, rescale_model,
+                         std_y, thompson_batch, unstandardized_mean_and_var, update_surrogate, empty_posterior_like, _get_minimum,
                          _update_model_parameters)
 from .acquisition import (AbstractAcquisition, EnsembleAcquisition, ExpectedImprovement, GradientNormUCB,
-                          ProbabilityImprovement, UpperConfidenceBound)
+                          ProbabilityImprovement, ThompsonSampling, UpperConfidenceBound)
 from .domains import AbstractDomain, ContinuousDomain
 from .parallel import (init_nccl_context, merge_topk, shard_range, sharded_nlml_batch, sharded_restarts, sharded_topk,
                        sync_posterior)

@@ -20,6 +20,7 @@ SYMBOLS = [
     "abo_gp_clone", "abo_gp_n", "abo_gp_alpha", "abo_gp_factor", "abo_gp_posterior", "abo_gp_posterior_cov", "abo_acq_eval", "abo_acq_eval_dev", "abo_acq_eval_grad",
     "abo_nlml_batch", "abo_potrf_dev", "abo_fill_distance", "abo_nccl_unique_id", "abo_ctx_init_rank", "abo_gp_sync",
     "abo_topk_allgather", "abo_allgather_f64", "abo_ctx_ranks", "abo_ctx_trim", "abo_acq_eval_multi", "abo_standardize", "abo_gp_set_params_ard", "abo_nlml_batch_ard",
+    "abo_gp_posterior_sample",
 ]
 
 
@@ -51,7 +52,7 @@ def lib():
                 f"{LIB_PATH} is missing: build it with `python -c 'import __graft_entry__ as g; g.build()'`. "
                 "There is no CPU fallback.")
         L = C.CDLL(LIB_PATH, mode=C.RTLD_GLOBAL)
-        vp, i32, i64, dbl = C.c_void_p, C.c_int32, C.c_int64, C.c_double
+        vp, i32, i64, u64, dbl = C.c_void_p, C.c_int32, C.c_int64, C.c_uint64, C.c_double
         pd = C.POINTER(C.c_double)
         L.abo_version.restype = i32
         L.abo_last_error.restype = C.c_char_p
@@ -77,6 +78,7 @@ def lib():
             "abo_gp_factor": [vp, i32, vp],
             "abo_gp_posterior": [vp, vp, i64, i32, vp, vp],
             "abo_gp_posterior_cov": [vp, vp, i64, i32, vp],
+            "abo_gp_posterior_sample": [vp, vp, i64, i64, u64, dbl, vp, vp, vp, C.POINTER(C.c_double)],
             "abo_acq_eval": [vp, i32, vp, vp, i64, vp, i64, vp, vp],
             "abo_acq_eval_dev": [vp, i32, vp, vp, i64, vp, i64, vp, vp],
             "abo_acq_eval_multi": [vp, i32, vp, vp, vp, vp, i64, vp, i64, vp, vp],
@@ -323,6 +325,21 @@ class GpHandle:
         cov = np.empty((M, M))
         check(lib().abo_gp_posterior_cov(self._h, ptr(Xc), Xc.shape[0], outputs, ptr(cov)))
         return cov
+
+    def posterior_sample(self, Xc, num_samples, seed, jitter=1e-10, want_samples=True):
+        """Joint draws of the value output over Xc: (samples (S, m) or None, argmin indices (S,), argmin values (S,),
+        the jitter tau actually added to the covariance)."""
+        Xc = f64(Xc)
+        if Xc.ndim != 2 or Xc.shape[1] != self.d:
+            raise DimensionMismatch(f"query points must be m x {self.d}")
+        m, S, seed = Xc.shape[0], int(num_samples), int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2^64)")
+        samples = np.empty((max(S, 0), m)) if want_samples else None
+        ai = np.empty(max(S, 1), dtype=np.int64); av = np.empty(max(S, 1)); tau = C.c_double(0.0)
+        check(lib().abo_gp_posterior_sample(self._h, ptr(Xc), m, S, seed, float(jitter),
+                                            ptr(samples), ptr(ai), ptr(av), C.byref(tau)))
+        return samples, ai[:max(S, 0)], av[:max(S, 0)], tau.value
 
     def acq_eval(self, acq_id, params, Xc, k=0, want_scores=True):
         Xc = f64(Xc)

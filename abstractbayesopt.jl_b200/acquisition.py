@@ -8,7 +8,7 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from .surrogates import _as_points, _get_minimum, _need_posterior
+from .surrogates import _as_points, _get_minimum, _need_posterior, posterior_sample
 from .parallel import merge_topk
 
 ACQ_EI, ACQ_PI, ACQ_UCB = 0, 1, 2
@@ -16,6 +16,7 @@ ACQ_EI, ACQ_PI, ACQ_UCB = 0, 1, 2
 
 class AbstractAcquisition:
     acq_id = -1
+    has_gradient = True          # False: optimize_acquisition returns the best grid point without refinement
 
     def params(self):
         raise NotImplementedError
@@ -71,6 +72,30 @@ class UpperConfidenceBound(AbstractAcquisition):
     def params(self): return [self.beta]
     def copy(self): return UpperConfidenceBound(self.beta)
     def update(self, ys, surrogate): return self
+
+
+@dataclass(frozen=True)
+class ThompsonSampling(AbstractAcquisition):
+    """Thompson sampling: the acquisition is minus ONE joint posterior draw of f over the evaluated point set
+    (abo_gp_posterior_sample), so its maximiser is the minimiser of that draw.  The draw is a function of (seed, point
+    set); `update` advances the seed, so every BO iteration draws afresh.  A draw has no gradient: optimize_acquisition
+    returns the best grid point."""
+    seed: int
+    has_gradient = False
+
+    def __call__(self, surrogate, x):
+        return -posterior_sample(surrogate, x, 1, seed=self.seed)[0]
+
+    def topk(self, surrogate, x, k, want_scores=True):
+        s = self(surrogate, x)
+        ti, tv = merge_topk([np.arange(len(s))], [s], k)
+        return (s if want_scores else None), ti, tv
+
+    def value_and_grad(self, surrogate, x):
+        raise TypeError("ThompsonSampling has no gradient: a posterior draw is not differentiable in x")
+
+    def copy(self): return ThompsonSampling(self.seed)
+    def update(self, ys, surrogate): return ThompsonSampling(self.seed + 1)
 
 
 ACQ_GRADNORM_UCB = 3

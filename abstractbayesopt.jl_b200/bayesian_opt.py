@@ -59,12 +59,13 @@ def optimize_acquisition(acqf, surrogate, domain, n_grid=10_000, n_local=100, rn
     lock-step and every step is ONE batched call returning the acquisition and its gradient for all of
     them (refine=True): analytic for EI / PI / UCB (abo_acq_eval_grad), batched central differences —
     all starts x (2 d + 1) points in one device call — for GradientNormUCB and ensembles.  refine="scipy" keeps the reference's sequential,
-    finite-difference scheme (SciPy L-BFGS-B); refine=False returns the best grid point."""
+    finite-difference scheme (SciPy L-BFGS-B); refine=False returns the best grid point, and so does an acquisition
+    without a gradient (ThompsonSampling), whatever `refine` says."""
     rng = np.random.default_rng() if rng is None else rng
     grid = latin_hypercube(n_grid, domain.lower, domain.upper, rng)
     _, top_idx, top_val = acqf.topk(surrogate, grid, n_local, want_scores=False)
     starts = grid[top_idx]
-    if refine is False or len(starts) == 0:
+    if refine is False or len(starts) == 0 or not getattr(acqf, "has_gradient", True):
         return np.array(starts[0])
     if refine == "scipy":
         best_acq, best_x = -math.inf, None

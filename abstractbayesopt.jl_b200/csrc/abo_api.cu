@@ -1,5 +1,5 @@
 // abo_api.cu — C ABI of libabo_cuda.so (include/abo.h): handles, host drivers of the blocked
-// Cholesky / triangular inverse / candidate sweep, top-k selection.  No CPU fallback anywhere:
+// Cholesky / triangular inverse / candidate sweep, top-k selection, joint posterior sampling.  No CPU fallback anywhere:
 // every entry point needs a live CUDA device.
 #include <algorithm>
 #include <cmath>
@@ -20,6 +20,7 @@
 #include "sweep_tma.cuh"
 #include "sweep_fused.cuh"
 #include "gemm_tma.cuh"
+#include "sample.cuh"
 #include "abo_internal.h"
 
 using namespace abo;
@@ -1128,14 +1129,16 @@ extern "C" int32_t abo_gp_posterior(abo_gp* g, const double* Xc, int64_t m, int3
     return ABO_OK;
 }
 
-// W = L^-1 K*^T  [Npad][ncol]  (k <= row): both operands k-contiguous -> the persistent TMA GEMM
-static int linv_times_ks(abo_ctx* c, const abo_gp* g, const double* Ks, int64_t ncol, double* W, cudaStream_t st) {
+// W = L^-1 K*^T  [Npad][ncol]  (k <= row): both operands k-contiguous -> the persistent TMA GEMM.
+// W and / or its transpose Wt [ncol][Npad] (nullable each).
+static int linv_times_ks(abo_ctx* c, const abo_gp* g, const double* Ks, int64_t ncol, double* W, cudaStream_t st, double* Wt = nullptr) {
     CUtensorMap tmX, tmK;
     int rc;
     if ((rc = make_tmap_k4(&tmX, g->dLinv, g->Npad, g->Npad, g->ld)) || (rc = make_tmap_k4(&tmK, Ks, g->Npad, ncol, g->Npad))) return rc;
     TmaGemmParams w{};
     w.batch = 1; w.alpha = 1.0; w.beta = 0.0; w.Mt = (int)(g->Npad / NB); w.Nt = (int)(ncol / NB); w.K = (int)g->Npad; w.flags = KHI_M;
     w.C = W; w.ldc = ncol;
+    w.CT = Wt; w.ldct = g->Npad;
     return launch_gemm_tma(c, tmX, tmK, w, st);
 }
 
@@ -1241,10 +1244,124 @@ extern "C" int32_t abo_gp_posterior_cov(abo_gp* g, const double* Xc, int64_t m, 
     CU((launch_gemm(q, 1, st)));
     KL(c);
     const int64_t Mo = m * outputs;
-    cov_finish_kernel<<<(unsigned)((Mo * Mo + 255) / 256), 256, 0, st>>>(gp_spec(g), dXc, m, outputs, mp, G, Mpad, dcov);
+    cov_finish_kernel<<<(unsigned)((Mo * Mo + 255) / 256), 256, 0, st>>>(gp_spec(g), dXc, m, outputs, mp, G, Mpad, dcov, Mo, 0, 0.0);
     KL(c);
     CU(cudaMemcpyAsync(cov, dcov, sizeof(double) * Mo * Mo, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
+    return ABO_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// joint posterior samples of the value output over a candidate set (sample.cuh):
+//   K* (value rows) -> W^T = (L^-1 K*^T)^T -> G = W^T W (lower tiles) -> Sigma + tau I (lower tiles, identity padding)
+//   -> look-ahead Cholesky (strict upper part of its diagonal tiles zeroed) -> L_Sigma Z^T, stored transposed: draws F [S][m] sample-major -> + mu, per-draw argmin.
+// Every product is a full-k GEMM tile per (candidate tile, draw tile): no reduction order depends on S, so the first S'
+// draws of a call are those of a call with S' draws, bit for bit.
+// ------------------------------------------------------------------------------------------
+constexpr int64_t SAMPLE_MAX_M = 16384, SAMPLE_MAX_S = 4096;
+constexpr int SAMPLE_JITTER_STEPS = 7;       // tau_k = jitter * sigma^2 * 10^k, k = 0 .. 6
+static int gp_posterior_sample_run(abo_gp* g, const double* Xc, int64_t m, int64_t S, uint64_t seed, double jitter,
+                                   double* samples, int64_t* argmin_idx, double* argmin_val, double* jitter_used);
+extern "C" int32_t abo_gp_posterior_sample(abo_gp* g, const double* Xc, int64_t m, int64_t S, uint64_t seed, double jitter,
+                                           double* samples, int64_t* argmin_idx, double* argmin_val, double* jitter_used) {
+    const int rc = gp_posterior_sample_run(g, Xc, m, S, seed, jitter, samples, argmin_idx, argmin_val, jitter_used);
+    if (rc && g && g->ctx) {
+        // as abo_gp_fit: no factorisation side stream may still be writing workspace slots the next call reuses
+        const std::string keep = g_err;
+        ctx_sync_all(g->ctx);
+        cudaGetLastError();
+        g_err = keep;
+    }
+    return rc;
+}
+static int gp_posterior_sample_run(abo_gp* g, const double* Xc, int64_t m, int64_t S, uint64_t seed, double jitter,
+                                   double* samples, int64_t* argmin_idx, double* argmin_val, double* jitter_used) {
+    if (!g || !Xc) return abo_fail(ABO_ERR_INVALID, "null argument");
+    if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
+    if (!(jitter > 0) || !std::isfinite(jitter)) return abo_fail(ABO_ERR_INVALID, "jitter must be positive and finite");
+    if (m > SAMPLE_MAX_M || S > SAMPLE_MAX_S)
+        return abo_fail(ABO_ERR_INVALID, "joint samples are limited to m <= %lld candidates and S <= %lld draws",
+                        (long long)SAMPLE_MAX_M, (long long)SAMPLE_MAX_S);
+    if (m <= 0 || S <= 0) return ABO_OK;
+    abo_ctx* c = g->ctx;
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const int64_t Npad = g->Npad, Mpad = (m + NB - 1) / NB * NB, Spad = (S + NB - 1) / NB * NB;
+    const int T = (int)(Mpad / NB);
+    const int npb = (int)(((Npad + g->p - 1) / g->p + 127) / 128);
+    double *dXc, *Ks, *pmean, *Wt, *G, *Sig, *Z, *F, *mu, *amin, *Dinv;
+    int* dinfo;
+    int rc;
+    if ((rc = ws_get(c, WS_CAND, sizeof(double) * (size_t)m * g->d, (void**)&dXc)) ||
+        (rc = ws_get(c, WS_KS, sizeof(double) * (size_t)Mpad * Npad, (void**)&Ks)) ||
+        (rc = ws_get(c, WS_PMEAN, sizeof(double) * (size_t)npb * Mpad, (void**)&pmean)) ||
+        (rc = ws_get(c, WS_GRAD_W, sizeof(double) * (size_t)Mpad * Npad, (void**)&Wt)) ||
+        (rc = ws_get(c, WS_SAMPLE_G, sizeof(double) * (size_t)Mpad * Mpad, (void**)&G)) ||
+        (rc = ws_get(c, WS_SAMPLE_SIGMA, sizeof(double) * (size_t)Mpad * Mpad, (void**)&Sig)) ||
+        (rc = ws_get(c, WS_SAMPLE_Z, sizeof(double) * (size_t)Spad * Mpad, (void**)&Z)) ||
+        (rc = ws_get(c, WS_SAMPLE_F, sizeof(double) * (size_t)Spad * Mpad, (void**)&F)) ||
+        (rc = ws_get(c, WS_OUT_B, sizeof(double) * (size_t)Mpad, (void**)&mu)) ||
+        (rc = ws_get(c, WS_OUT_A, sizeof(double) * (size_t)2 * S, (void**)&amin)) ||
+        (rc = ws_get(c, WS_DINV, sizeof(double) * (size_t)T * NB * NB, (void**)&Dinv)) ||
+        (rc = ws_get(c, WS_INFO, sizeof(int) * 16, (void**)&dinfo)))
+        return rc;
+    CU(cudaMemcpyAsync(dXc, Xc, sizeof(double) * m * g->d, cudaMemcpyHostToDevice, st));
+    // K* value rows for all Mpad candidate rows (rows >= m are built at the origin; the padding of Sigma overwrites them)
+    if ((rc = launch_ks_d(c, g, dXc, 0, m, 0, Ks, pmean, Mpad, Mpad, npb, st))) return rc;
+    if ((rc = linv_times_ks(c, g, Ks, Mpad, nullptr, st, Wt))) return rc;             // W^T [Mpad][Npad]
+    {
+        CUtensorMap tmW;
+        if ((rc = make_tmap_k4(&tmW, Wt, Npad, Mpad, Npad))) return rc;
+        TmaGemmParams q{};                                                               // G = W^T W, lower tiles
+        q.Mt = T; q.Nt = T; q.batch = 1; q.K = (int)Npad; q.flags = LOWER_ONLY; q.alpha = 1.0; q.beta = 0.0;
+        q.C = G; q.ldc = Mpad;
+        if ((rc = launch_gemm_tma(c, tmW, tmW, q, st))) return rc;
+    }
+    {
+        AcqSpec a{};                                                                     // mu = m + sum of the partial means
+        a.acq = -1; a.mean_c = g->mean_c[0]; a.kss = g->scale;
+        acq_epilogue_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(a, pmean, npb, nullptr, 0, Mpad, m, mu, nullptr, nullptr);
+        KL(c);
+    }
+    philox_normal_kernel<<<(unsigned)((Spad * Mpad / 4 + 255) / 256), 256, 0, st>>>(seed, S, m, Spad, Mpad, Z);
+    KL(c);
+    double tau = 0.0;
+    for (int k = 0;; ++k) {
+        double p10 = 1.0;
+        for (int e = 0; e < k; ++e) p10 *= 10.0;
+        tau = jitter * g->scale * p10;
+        cov_finish_kernel<<<(unsigned)((Mpad * Mpad + 255) / 256), 256, 0, st>>>(gp_spec(g), dXc, m, 1, Mpad, G, Mpad, Sig, Mpad,
+                                                                                 Mpad, tau);
+        KL(c);
+        CU(cudaMemsetAsync(dinfo, 0, sizeof(int) * 16, st));
+        if ((rc = potrf_lookahead(c, Sig, Mpad, Mpad, Dinv, dinfo))) return rc;
+        int hinfo = 0;
+        CU(cudaMemcpyAsync(&hinfo, dinfo, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (hinfo == 0) break;
+        ctx_sync_all(c);
+        if (k + 1 == SAMPLE_JITTER_STEPS)
+            return abo_fail(ABO_ERR_NOT_POSDEF, "posterior covariance + %g I is not positive definite (pivot %d)", tau, hinfo);
+    }
+    zero_diag_upper_kernel<<<T, 256, 0, st>>>(Sig, Mpad);
+    KL(c);
+    {
+        CUtensorMap tmL, tmZ;
+        if ((rc = make_tmap_k4(&tmL, Sig, Mpad, Mpad, Mpad)) || (rc = make_tmap_k4(&tmZ, Z, Mpad, Spad, Mpad))) return rc;
+        TmaGemmParams f{};                                                               // F = (L_Sigma Z^T)^T  [Spad][Mpad]
+        f.Mt = T; f.Nt = (int)(Spad / NB); f.batch = 1; f.K = (int)Mpad; f.flags = KHI_M; f.alpha = 1.0; f.beta = 0.0;
+        f.C = nullptr; f.CT = F; f.ldct = Mpad;
+        if ((rc = launch_gemm_tma(c, tmL, tmZ, f, st))) return rc;
+    }
+    long long* aidx = reinterpret_cast<long long*>(amin);
+    sample_finish_kernel<<<(unsigned)S, SF_THREADS, 0, st>>>(F, Mpad, mu, m, aidx, amin + S);
+    KL(c);
+    if (samples)
+        CU(cudaMemcpy2DAsync(samples, sizeof(double) * m, F, sizeof(double) * Mpad, sizeof(double) * m, S, cudaMemcpyDeviceToHost, st));
+    if (argmin_idx) CU(cudaMemcpyAsync(argmin_idx, aidx, sizeof(int64_t) * S, cudaMemcpyDeviceToHost, st));
+    if (argmin_val) CU(cudaMemcpyAsync(argmin_val, amin + S, sizeof(double) * S, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (jitter_used) *jitter_used = tau;
     return ABO_OK;
 }
 

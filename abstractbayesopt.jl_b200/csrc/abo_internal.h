@@ -31,7 +31,9 @@ int abo_fail(int code, const char* fmt, ...);
 enum WsSlot {
     WS_STAGE_X = 0, WS_STAGE_Y, WS_DINV, WS_INFO, WS_TRTRI, WS_VEC_PART, WS_KS, WS_PMEAN, WS_SUMSQ, WS_CAND,
     WS_OUT_A, WS_OUT_B, WS_NLML_K, WS_NLML_LINV, WS_NLML_W, WS_NLML_X, WS_NLML_VEC, WS_NLML_PAR, WS_APPEND,
-    WS_TOPK, WS_SELECT, WS_GRAD_W, WS_GRAD_Z, WS_GRAD_PART, WS_GRAD_OUT, WS_TRTRI_U, WS_NLML_U, WS_COUNT
+    WS_TOPK, WS_SELECT, WS_GRAD_W, WS_GRAD_Z, WS_GRAD_PART, WS_GRAD_OUT, WS_TRTRI_U, WS_NLML_U,
+    WS_SAMPLE_G, WS_SAMPLE_SIGMA, WS_SAMPLE_Z, WS_SAMPLE_F,       // joint posterior sampler: W^T W, Sigma + tau I -> its factor, Z^T, draws
+    WS_COUNT
 };
 
 struct WsBuf { void* ptr = nullptr; size_t bytes = 0; };

@@ -1584,13 +1584,22 @@ __global__ void acq_grad_finish_kernel(AcqSpec a, int d, const double* __restric
 // (posterior_grad_cov, src/surrogates/GradientGP.jl:968-971):
 //   cov[(b,c),(b',c')] = gk((x_c,b),(x_c',b')) - G[b*mp + c][b'*mp + c'] + 1e-18 * delta
 // with G = W^T W, W = L^-1 K*; one thread per output entry.
+//   Dense form (pad = 0): the M x M matrix, M = m nout, leading dimension ldc.
+//   Factor form (pad = the padded size, a multiple of 128): the pad x pad input of potrf_lookahead — lower 128-tiles only
+//   (tiles above the diagonal are not written), the strict upper part of the diagonal tiles zero, identity in the padding,
+//   and tau added to the diagonal on top of the 1e-18 (G is only read in its lower tiles).
 namespace abo {
 __global__ void cov_finish_kernel(KSpec spec, const double* __restrict__ Xc, int64_t m, int nout, int64_t mp,
-                                  const double* __restrict__ G, int64_t ldg, double* __restrict__ cov) {
-    const int64_t M = m * nout;
+                                  const double* __restrict__ G, int64_t ldg, double* __restrict__ cov, int64_t ldc,
+                                  int64_t pad, double tau) {
+    const int64_t M = m * nout, R = pad > 0 ? pad : M;
     const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (t >= M * M) return;
-    const int64_t r = t / M, q = t % M;
+    if (t >= R * R) return;
+    const int64_t r = t / R, q = t % R;
+    if (pad > 0) {
+        if (q / 128 > r / 128) return;
+        if (r >= M || q >= M || q > r) { cov[r * ldc + q] = (r == q) ? 1.0 : 0.0; return; }
+    }
     const int b = (int)(r / m), b2 = (int)(q / m);
     const int64_t c = r % m, c2 = q % m;
     double u = 0.0, Da = 0.0, Db = 0.0;
@@ -1603,7 +1612,8 @@ __global__ void cov_finish_kernel(KSpec spec, const double* __restrict__ Xc, int
     double p, dp, ddp;
     phi_eval(spec.kind, u, p, dp, ddp);
     const double prior = gk_entry(spec, p, dp, ddp, b, b2, Da, Db);
-    cov[t] = (prior - G[((int64_t)b * mp + c) * ldg + (int64_t)b2 * mp + c2]) + (r == q ? JITTER : 0.0);
+    const double v = (prior - G[((int64_t)b * mp + c) * ldg + (int64_t)b2 * mp + c2]) + (r == q ? JITTER : 0.0);
+    cov[r * ldc + q] = (r == q) ? v + tau : v;
 }
 }  // namespace abo
 

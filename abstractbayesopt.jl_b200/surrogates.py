@@ -219,6 +219,22 @@ def posterior_cov(model, x):
     return h.posterior_cov(_as_points(x, h.d), 1)
 
 
+def posterior_sample(model, x, num_samples, *, seed, jitter=1e-10):
+    """Joint draws of the latent value f over the points x: an (S, m) array, row s = draw s (AbstractGPs
+    rand(rng, posterior(fx)(x), S), transposed).  Draw s depends only on (seed, s): the first S' rows of S > S' draws are
+    the S' draws.  jitter is relative to the kernel scale and raised tenfold, up to six times, until the covariance
+    factors."""
+    h = _need_posterior(model)
+    return h.posterior_sample(_as_points(x, h.d), num_samples, seed, jitter)[0]
+
+
+def thompson_batch(model, x, q, *, seed, jitter=1e-10):
+    """q candidate indices (0-based) into x: the minimiser of each of q joint posterior draws, a Thompson-sampling batch
+    drawn with replacement.  Only the q indices leave the device."""
+    h = _need_posterior(model)
+    return h.posterior_sample(_as_points(x, h.d), q, seed, jitter, want_samples=False)[1]
+
+
 def unstandardized_mean_and_var(model, xs, params):
     """StandardGP.jl:395-404 / GradientGP.jl:1019-1030."""
     h = _need_posterior(model)

@@ -127,6 +127,26 @@ int32_t abo_gp_posterior(abo_gp* gp, const double* Xc, int64_t m, int32_t output
  * outputs == 1 or p; m*outputs <= 8192. */
 int32_t abo_gp_posterior_cov(abo_gp* gp, const double* Xc, int64_t m, int32_t outputs, double* cov);
 
+/* Joint samples of the latent value f over a candidate set: f_s = mu + chol(Sigma + tau I) z_s, where
+ * Sigma = K(Xc,Xc) - K(Xc,X) (K + noise I)^-1 K(X,Xc) (+ 1e-18 I, as abo_gp_posterior_cov). This is AbstractGPs
+ * rand(rng, posterior(fx)(Xc), S). Value output only, also for a GradientGP. Units are the model's own, the same as
+ * abo_gp_posterior's mean.
+ * samples: S x m, sample-major (row s = draw s). In Julia this is the m x S matrix rand returns. Nullable.
+ * argmin_idx / argmin_val: per draw, the minimising candidate. Ties go to the first index. A NaN in a draw yields that
+ * draw's first NaN, as Julia's findmin does. Both are nullable. The S argmins are a q = S Thompson batch, drawn with
+ * replacement.
+ * z_s[i] is a standard normal that depends only on (seed, s, i): Philox4x64-10 with key (seed, s), counter (i/4 + 1, 0, 0, 0)
+ * -- NumPy's np.random.Philox(key=[seed, s]).random_raw() words 4j..4j+3 -- turned into four normals by two Box-Muller
+ * pairs. So a call with S draws repeats, bit for bit, the S' < S draws of a call with S', and the argmins do not depend on
+ * whether samples is NULL.
+ * jitter > 0 is relative to the kernel scale: tau_k = jitter * sigma^2 * 10^k for k = 0..6, and the first tau whose
+ * Cholesky succeeds is used and returned in *jitter_used (nullable). ABO_ERR_NOT_POSDEF after k = 6.
+ * 1 <= m <= 16384, 1 <= S <= 4096; m <= 0 or S <= 0 is a no-op. The posterior held by gp is only read.
+ * Device workspace: about 8 (2 m^2 + 2 m n p + 2 m S) bytes, 8 GB at m = 16384, n p = 8192, S = 4096 (abo_ctx_trim
+ * releases it). */
+int32_t abo_gp_posterior_sample(abo_gp* gp, const double* Xc, int64_t m, int64_t S, uint64_t seed, double jitter,
+                                double* samples, int64_t* argmin_idx, double* argmin_val, double* jitter_used);
+
 /* fused acquisition sweep: scores = acq(surrogate, Xc) (ExpectedImprovement.jl:40-45 etc.) and
  * sortperm(scores; rev=true)[1:k] (acq_utils.jl:50-52): stable, descending, NaN first.
  * scores (m) may be NULL — then only the k selected (index, value) pairs leave the device (the

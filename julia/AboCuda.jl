@@ -391,6 +391,21 @@ function nlml_ard_value_grad(m::CuStandardGP, θ::Vector{Float64}, xs, ys)
     val[], g
 end
 
+# Joint draws of the latent value over xs, AbstractGPs rand(rng, posterior(fx)(xs), S): an m x S matrix, column s = draw s
+# (the library's sample-major S x m buffer is exactly this matrix in column-major order).  Draw s depends only on
+# (seed, s); jitter is relative to the kernel scale and raised tenfold, up to six times, until the covariance factors.
+# Thompson sampling proposes argmin of each column (argmin(posterior_sample(m, xs, q; seed=seed), dims=1)).
+function posterior_sample(m::Union{CuStandardGP,CuGradientGP}, xs, S::Integer; seed::Integer, jitter::Real=1e-10)
+    m.gpx === nothing && error("surrogate has no posterior: call update(model, xs, ys) first")
+    Xc = Matrix{Float64}(points(collect(xs))); mcount = size(Xc, 2)
+    out = Matrix{Float64}(undef, mcount, S)
+    τ = Ref{Float64}(0.0)
+    check(GC.@preserve Xc out ccall((:abo_gp_posterior_sample, LIB), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, UInt64, Float64, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ref{Float64}),
+        m.gpx.h, Xc, mcount, S, UInt64(seed), Float64(jitter), out, C_NULL, C_NULL, τ))
+    out
+end
+
 # monte_carlo_fill_distance (src/BO_utils.jl:140-159) on the device; the caller draws the uniform samples
 function fill_distance(X::Matrix{Float64}, S::Matrix{Float64})         # both d x count, column-major = point-major
     out = Ref{Float64}(0.0)

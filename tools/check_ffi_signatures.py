@@ -23,7 +23,7 @@ def c_prototypes(path=os.path.join(ROOT, "include", "abo.h")):
 
 
 def classify_c(a):
-    """C parameter -> canonical class: int32 | int64 | double | ptr:<pointee> | pptr"""
+    """C parameter -> canonical class: int32 | int64 | uint64 | double | ptr:<pointee> | pptr"""
     a = re.sub(r"\bconst\b", "", a).strip()
     arr = re.search(r"\[\s*\d*\s*\]\s*$", a)
     if arr:                                                           # `double ms[3]` decays to a pointer
@@ -32,14 +32,14 @@ def classify_c(a):
     base = a.replace("*", " ").split()
     typ = base[0] if base else ""
     if stars == 0:
-        return {"int32_t": "int32", "int64_t": "int64", "double": "double"}.get(typ, "?" + typ)
+        return {"int32_t": "int32", "int64_t": "int64", "uint64_t": "uint64", "double": "double"}.get(typ, "?" + typ)
     if stars >= 2:
         return "pptr"
     return "ptr:" + {"double": "double", "int64_t": "int64", "int32_t": "int32", "uint8_t": "uint8", "void": "void",
                      "abo_ctx": "void", "abo_gp": "void", "char": "char"}.get(typ, "?" + typ)
 
 
-JL = {"Int32": "int32", "Int64": "int64", "Float64": "double", "Cstring": "cstring", "Ptr{Cvoid}": "ptr:void",
+JL = {"Int32": "int32", "Int64": "int64", "UInt64": "uint64", "Float64": "double", "Cstring": "cstring", "Ptr{Cvoid}": "ptr:void",
       "Ref{Ptr{Cvoid}}": "pptr", "Ptr{Float64}": "ptr:double", "Ref{Float64}": "ptr:double", "Ptr{Int64}": "ptr:int64",
       "Ref{Int64}": "ptr:int64", "Ptr{Int32}": "ptr:int32", "Ref{Int32}": "ptr:int32", "Ptr{UInt8}": "ptr:uint8"}
 
@@ -120,7 +120,7 @@ def check_ctypes(protos):
         if len(args) != len(cargs):
             errs.append(f"_lib.py {name}: {len(args)} argtypes, the header has {len(cargs)}"); continue
         for q, (a, ct) in enumerate(zip(args, cargs)):
-            cls = {"i32": "int32", "i64": "int64", "dbl": "double"}.get(a, "ptr")
+            cls = {"i32": "int32", "i64": "int64", "u64": "uint64", "dbl": "double"}.get(a, "ptr")
             if (cls == "ptr") != (ct.startswith("ptr") or ct == "pptr") or (cls != "ptr" and cls != ct):
                 errs.append(f"_lib.py {name}: argument {q + 1} is {a}, the header says {ct}")
     declared = set(re.findall(r'"(abo_\w+)"', re.search(r"SYMBOLS = \[(.*?)\]", src, flags=re.S).group(1)))
