@@ -17,7 +17,6 @@
 #include "../../include/abo.h"
 #include "gemm_dmma.cuh"
 #include "kernels.cuh"
-#include "sweep_tma.cuh"
 #include "sweep_fused.cuh"
 #include "gemm_tma.cuh"
 #include "sample.cuh"
@@ -54,9 +53,9 @@ static int configure_kernels() {
     CU(cudaFuncSetAttribute(gemm_k128_kernel<32, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmK128<32, 32>::SMEM_BYTES));
     CU(cudaFuncSetAttribute(fill_distance_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 256 * 96 * 8));
     CU(cudaFuncSetAttribute(potf2_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PW_SMEM_BYTES));
-    CU(cudaFuncSetAttribute(sweep_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SW_SMEM_BYTES));
     CU(cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SY_SMEM_BYTES));
-    CU(cudaFuncSetAttribute(gemm_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TG_SMEM_BYTES));
+    CU(cudaFuncSetAttribute(gemm_tma_kernel<EPI_STORE>, cudaFuncAttributeMaxDynamicSharedMemorySize, tg_smem_bytes<EPI_STORE>()));
+    CU(cudaFuncSetAttribute(gemm_tma_kernel<EPI_COLSUMSQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, tg_smem_bytes<EPI_COLSUMSQ>()));
 #define ABO_FS_CFG(DT) CU(cudaFuncSetAttribute(sweep_fused_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, fused_smem_bytes<DT>()))
     ABO_FS_CFG(4); ABO_FS_CFG(8); ABO_FS_CFG(12); ABO_FS_CFG(16); ABO_FS_CFG(20); ABO_FS_CFG(24); ABO_FS_CFG(32);
 #undef ABO_FS_CFG
@@ -282,6 +281,7 @@ int pinned_get(abo_ctx* c, size_t bytes, void** out) {
 // Dinv: batch x T x 128 x 128 block inverses.  info: batch ints (0 = ok).
 // ------------------------------------------------------------------------------------------
 int make_tmap_k4(CUtensorMap* map, const double* base, int64_t K, int64_t rows, int64_t ld);
+template <int EPI = EPI_STORE>
 static int launch_gemm_tma(abo_ctx* c, const CUtensorMap& tmA, const CUtensorMap& tmB, TmaGemmParams p, cudaStream_t st, int max_ctas = 0);
 int potrf_blocked(abo_ctx* c, double* A, int64_t Npad, int64_t ld, double* Dinv, int* info, int batch) {
     const int T = (int)(Npad / NB);
@@ -533,6 +533,7 @@ __global__ void place_diag_both_kernel(const double* __restrict__ Dinv, double* 
         dsu[(int64_t)r * ld + cc] = src[cc * NB + r];
     }
 }
+template <int EPI>
 static int launch_gemm_tma(abo_ctx* c, const CUtensorMap& tmA, const CUtensorMap& tmB, TmaGemmParams p, cudaStream_t st, int max_ctas) {
     if (p.Mt <= 0 || p.Nt <= 0 || p.batch <= 0) return ABO_OK;
     if ((p.flags & LOWER_ONLY) && p.Nt > p.Mt) return abo_fail(ABO_ERR_INVALID, "gemm_tma: LOWER_ONLY needs Nt <= Mt");
@@ -540,7 +541,7 @@ static int launch_gemm_tma(abo_ctx* c, const CUtensorMap& tmA, const CUtensorMap
     const int64_t total = per * p.batch;
     if (total > 0x7fffffff) return abo_fail(ABO_ERR_INVALID, "too many tiles in one launch");
     p.total = (int)total;
-    gemm_tma_kernel<<<(int)std::min<int64_t>(total, max_ctas > 0 ? max_ctas : c->sms), SW_THREADS, TG_SMEM_BYTES, st>>>(tmA, tmB, p);
+    gemm_tma_kernel<EPI><<<(int)std::min<int64_t>(total, max_ctas > 0 ? max_ctas : c->sms), SW_THREADS, tg_smem_bytes<EPI>(), st>>>(tmA, tmB, p);
     KL(c);
     return ABO_OK;
 }
@@ -985,14 +986,10 @@ static double phi_prime0(int kind) {
     return -7.0 / 10.0;
 }
 
-// ---- fused single-kernel sweep (sweep_fused.cuh): scalar GPs up to ABO_FUSED_MAX observations (measured faster than the
+// ---- fused single-kernel sweep (sweep_fused.cuh): scalar GPs up to FS_MAX_NPAD observations (measured faster than the
 //      three-kernel path at every size: n = 8192 97.9 % vs 95.6 % of the Dgemm peak for the whole step) ------------
-static int fused_max_n() {
-    static const int v = getenv("ABO_FUSED_MAX") ? atoi(getenv("ABO_FUSED_MAX")) : 16384;
-    return v;
-}
 static bool fused_applies(const abo_gp* g, int bo) {
-    return g->p == 1 && bo == 0 && g->d <= 32 && g->Npad <= fused_max_n();
+    return g->p == 1 && bo == 0 && g->d <= 32 && g->Npad <= FS_MAX_NPAD;
 }
 static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const AcqSpec& a, double* d_mean, double* d_var,
                               double* d_score) {
@@ -1006,8 +1003,6 @@ static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const Acq
     fp.Xc = dXc; fp.m = m; fp.beta = g->dBeta;
     fp.mean_out = d_mean; fp.var_out = d_var; fp.score_out = d_score;
     fp.ntiles = (int)((m + NB - 1) / NB);
-    static const int dbg = getenv("ABO_FUSED_DBG") ? atoi(getenv("ABO_FUSED_DBG")) : 0;
-    fp.dbg = dbg;
     const int grid = std::min(c->sms, fp.ntiles);
     int rc;
     // private K* scratch: [CTA][2][128][Kld]; sized for the full grid so that the tensor map is stable between calls
@@ -1081,10 +1076,10 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
         if ((rc = launch_ks_d(c, g, dXc, c0, m, bo, Ks, pmean, mc_eff, mc, npb, st))) return rc;
         if ((rc = prof_mark(c))) return rc;
         if ((rc = prof_mark(c))) return rc;
-        SweepParams sp;
-        sp.T = T; sp.ncb = (int)(mc_eff / NB); sp.sumsq = sumsq; sp.sumsq_ld = mc;
-        sweep_tma_kernel<<<std::min(c->sms, sp.T * sp.ncb), SW_THREADS, SW_SMEM_BYTES, st>>>(tmA, tmB, sp);
-        KL(c);
+        TmaGemmParams sp{};                                 // sumsq[ib][c] = sum over row tile ib of (L^-1 K*^T)^2
+        sp.batch = 1; sp.Mt = T; sp.Nt = (int)(mc_eff / NB); sp.K = (int)Npad; sp.flags = KHI_M;
+        sp.C = sumsq; sp.ldc = mc;
+        if ((rc = launch_gemm_tma<EPI_COLSUMSQ>(c, tmA, tmB, sp, st))) return rc;
         if ((rc = prof_mark(c))) return rc;
         if ((rc = prof_mark(c))) return rc;
         acq_epilogue_kernel<<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
@@ -1101,7 +1096,8 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
     return ABO_OK;
 }
 
-static int64_t host_piece();
+// host candidates per piece of sweep_host_pieces
+constexpr int64_t HOST_PIECE = 262144;
 static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
                              double* h_var, double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
 
@@ -1112,7 +1108,7 @@ extern "C" int32_t abo_gp_posterior(abo_gp* g, const double* Xc, int64_t m, int3
     if (m <= 0) return ABO_OK;
     abo_ctx* c = g->ctx;
     CU(cudaSetDevice(c->device));
-    if (outputs == 1 && m > host_piece() && !c->profile)
+    if (outputs == 1 && m > HOST_PIECE && !c->profile)
         return sweep_host_pieces(g, Xc, m, -1, nullptr, mean, var, nullptr, 0, nullptr, nullptr);
     cudaStream_t st = c->stream;
     double *dXc, *dm, *dv;
@@ -1495,10 +1491,6 @@ static int acq_check(abo_gp* g, int acq_id, const double* params, const void* Xc
 // piece i-1 (scores if asked for, and the K best of the piece, selected on the device).  Per-candidate results
 // do not depend on the piece size.
 // acq_id < 0: posterior mean / variance of output 0 (h_mean / h_var, each may be NULL).
-static int64_t host_piece() {
-    static const int64_t piece = getenv("ABO_ACQ_PIECE") ? atoll(getenv("ABO_ACQ_PIECE")) : 262144;
-    return piece;
-}
 static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
                                  double* h_var, double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
 static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
@@ -1519,7 +1511,7 @@ static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, int acq
     abo_ctx* c = g->ctx;
     cudaStream_t st = c->stream, sc = c->stream3;
     const int d = g->d;
-    const int64_t piece = host_piece();
+    const int64_t piece = HOST_PIECE;
     const int64_t np = (m + piece - 1) / piece;
     int rc;
     double *dXc, *dA, *dB = nullptr;
@@ -1573,7 +1565,7 @@ extern "C" int32_t abo_acq_eval(abo_gp* g, int32_t acq_id, const double* params,
     if (m == 0) return ABO_OK;
     abo_ctx* c = g->ctx;
     CU(cudaSetDevice(c->device));
-    if (m > host_piece() && !c->profile) return sweep_host_pieces(g, Xc, m, acq_id, params, nullptr, nullptr, scores, k, top_idx, top_val);
+    if (m > HOST_PIECE && !c->profile) return sweep_host_pieces(g, Xc, m, acq_id, params, nullptr, nullptr, scores, k, top_idx, top_val);
     double* dXc;
     if ((rc = ws_get(c, WS_CAND, sizeof(double) * (size_t)m * g->d, (void**)&dXc))) return rc;
     CU(cudaMemcpyAsync(dXc, Xc, sizeof(double) * m * g->d, cudaMemcpyHostToDevice, c->stream));

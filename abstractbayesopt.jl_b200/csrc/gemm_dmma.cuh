@@ -3,8 +3,8 @@
 //                                          (abo_acq_eval_grad), G = W^T W of the posterior covariance;
 //   gemm_small_kernel, gemm_k128_kernel    K-contiguous operands: the panel TRSM / SYRK of the look-ahead Cholesky.
 // (The candidate sweep, the trailing updates, the batched Cholesky, the triangular inverse and K^-1 = L^-T L^-1 run
-// on the TMA/mbarrier kernels of sweep_tma.cuh / gemm_tma.cuh, which share the shared-memory tile layout and the
-// DMMA inner loop.)
+// on the TMA/mbarrier pipeline of tma_pipe.cuh (gemm_tma.cuh, sweep_fused.cuh), which shares the shared-memory tile
+// layout and the DMMA inner loop.)
 //
 // tcgen05 has no f64 kind, so on sm_100a FP64 tensor work is the warp-level
 // mma.sync.m8n8k4.f64 (SASS DMMA.8x8x4; the m16n8k{4,8,16} PTX shapes lower to the same SASS

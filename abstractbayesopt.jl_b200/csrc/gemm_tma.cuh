@@ -2,19 +2,25 @@
 //     C[m][n] (+)= alpha * sum_{k in [klo, khi)} A[m][k] * B[n][k]          (both operands row-major with k contiguous)
 // with an optional TRANSPOSED second store CT[n][m] = alpha * (...) — which is what lets every O(n^3) step of the conditioning
 // and of the batched marginal likelihood keep its operands k-contiguous (the triangular inverse carries X and X^T, the product
-// of the inverse factors reads X^T twice), so that all of them run on the TMA + mbarrier + DMMA pipeline of the sweep kernel
+// of the inverse factors reads X^T twice), so that all of them run on the TMA + mbarrier + DMMA pipeline of tma_pipe.cuh
 // instead of the cp.async kernels whose MN-contiguous shared-memory layout costs bank conflicts (ncu, round 1: 84.7 % DMMA).
+// The EPI_COLSUMSQ instance is the contraction of the candidate sweep when it is not fused (GradientGP outputs, n > FS_MAX_NPAD):
+//     C[mt][n] = sum over the 128 rows m of row tile mt of ( sum_k A[m][k] B[n][k] )^2
+// with A = L^-1 and B = K*, i.e. the posterior-variance term ||L^-1 k*||^2 (StandardGP.jl:377-379 via AbstractGPs
+// diag_Xt_invA_X) per row tile, summed over the row tiles by acq_epilogue_kernel.
 //
 // One CTA per SM, static serpentine schedule over (batch item, tile) work items ordered heaviest first; the producer warp runs
 // ahead across item boundaries (no pipeline fill / drain per tile — the short k-loops of the batched n ~ 1000 matrices are
 // exactly where that matters); k-ranges that are structurally zero are skipped (flags as in gemm_dmma.cuh).
+//
+// Also here: syrk_tma_kernel, the trailing update of the blocked Cholesky on the same pipeline.
 #pragma once
 #include <cstdint>
 #include <cuda.h>
 #include <cuda_runtime.h>
 
 #include "gemm_dmma.cuh"
-#include "sweep_tma.cuh"
+#include "tma_pipe.cuh"
 
 namespace abo {
 
@@ -27,8 +33,11 @@ struct TmaGemmParams {
     int b_row0, b_rstep, b_col0, b_cstep;
     double* C;  int64_t ldc,  c_off0,  c_zstep;     // C  element (m, n): C [c_off0  + z c_zstep  + m ldc  + n]   (nullable)
     double* CT; int64_t ldct, ct_off0, ct_zstep;    // CT element (n, m): CT[ct_off0 + z ct_zstep + n ldct + m]   (nullable, beta = 0)
-    double alpha, beta;
+    double alpha, beta;                             // EPI_COLSUMSQ: C[mt ldc + n] = column sums of squares of tile (mt, nt);
+                                                    // batch 1, c_off0 / CT / alpha / beta unused
 };
+
+enum { EPI_STORE = 0, EPI_COLSUMSQ = 1 };
 
 struct TgTile { int z, m0, n0, klo, nk; };
 __device__ __forceinline__ TgTile tg_decode(const TmaGemmParams& p, int t) {
@@ -58,13 +67,17 @@ __device__ __forceinline__ TgTile tg_decode(const TmaGemmParams& p, int t) {
     return w;
 }
 
-constexpr int TG_SMEM_BYTES = SW_STAGES * SW_STAGE_BYTES + 2 * SW_STAGES * 8 + 128;
+// shared memory: the stage ring, the [4][128] column-sum buffer of EPI_COLSUMSQ, the barriers
+template <int EPI> __host__ __device__ constexpr int tg_red_bytes() { return EPI == EPI_COLSUMSQ ? 4 * 128 * 8 : 0; }
+template <int EPI> constexpr int tg_smem_bytes() { return SW_STAGES * SW_STAGE_BYTES + tg_red_bytes<EPI>() + 2 * SW_STAGES * 8 + 128; }
 
+template <int EPI>
 __global__ void __launch_bounds__(SW_THREADS, 1)
 gemm_tma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const TmaGemmParams p) {
     extern __shared__ __align__(128) unsigned char tg_smem[];
     double* stage_base = reinterpret_cast<double*>(tg_smem);
-    uint64_t* full = reinterpret_cast<uint64_t*>(tg_smem + SW_STAGES * SW_STAGE_BYTES);
+    double* red = reinterpret_cast<double*>(tg_smem + SW_STAGES * SW_STAGE_BYTES);
+    uint64_t* full = reinterpret_cast<uint64_t*>(tg_smem + SW_STAGES * SW_STAGE_BYTES + tg_red_bytes<EPI>());
     uint64_t* empty = full + SW_STAGES;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int G = gridDim.x, b = blockIdx.x;
@@ -88,14 +101,8 @@ gemm_tma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 const int brow = p.b_row0 + w.z * p.b_rstep + w.n0, bcol = p.b_col0 + w.z * p.b_cstep + w.klo;
                 for (int kt = 0; kt < w.nk; ++kt) {
                     mbar_wait(&empty[stage], phase ^ 1);
-                    mbar_expect_tx(&full[stage], SW_STAGE_BYTES);
-                    double* sa = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES);
-                    double* sb = sa + SW_OPER_DOUBLES;
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        tma_load_2d(sa + q * 512, &tmA, acol + kt * 16 + 4 * q, arow, &full[stage]);
-                        tma_load_2d(sb + q * 512, &tmB, bcol + kt * 16 + 4 * q, brow, &full[stage]);
-                    }
+                    tma_stage_load(stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES), &full[stage], &tmA, acol + kt * 16, arow,
+                                   &tmB, bcol + kt * 16, brow);
                     if (++stage == SW_STAGES) { stage = 0; phase ^= 1; }
                 }
             }
@@ -118,32 +125,37 @@ gemm_tma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             for (int j = 0; j < 8; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
         for (int kt = 0; kt < w.nk; ++kt) {
             mbar_wait(&full[stage], phase);
-            const double* a_s = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES) + ((wm + fr) << 2) + fk;
-            const double* b_s = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES) + SW_OPER_DOUBLES + ((wn + fr) << 2) + fk;
-            double a[2][4], bb[2][8];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) a[0][i] = a_s[i * 32];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) bb[0][j] = b_s[j * 32];
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk) {
-                const int cur = kk & 1, nxt = cur ^ 1;
-                if (kk < 3) {
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) a[nxt][i] = a_s[(kk + 1) * 512 + i * 32];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) bb[nxt][j] = b_s[(kk + 1) * 512 + j * 32];
-                }
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) dmma8x8x4(acc[i][j][0], acc[i][j][1], a[cur][i], bb[cur][j]);
-            }
+            const double* st = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES);
+            dmma_stage<0, 4, 32>(st + ((wm + fr) << 2) + fk, st + SW_OPER_DOUBLES + ((wn + fr) << 2) + fk, acc);
             __syncwarp();
             if (lane == 0) mbar_arrive(&empty[stage]);
             if (++stage == SW_STAGES) { stage = 0; phase ^= 1; }
         }
         // ---- epilogue
+        if (EPI == EPI_COLSUMSQ) {
+            // column sums of squares over the tile's 128 rows: the warp's 32 rows in registers and shuffles, then the four row
+            // warps in a fixed order
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) s = fma(acc[i][j][e], acc[i][j][e], s);
+                    s += __shfl_xor_sync(0xffffffffu, s, 4);
+                    s += __shfl_xor_sync(0xffffffffu, s, 8);
+                    s += __shfl_xor_sync(0xffffffffu, s, 16);
+                    if (fr == 0) red[(warp & 3) * 128 + wn + j * 8 + 2 * fk + e] = s;
+                }
+            }
+            asm volatile("bar.sync 1, 256;\n" ::: "memory");       // consumer warps only
+            if (tid < 128) {
+                const double s = ((red[tid] + red[128 + tid]) + red[256 + tid]) + red[384 + tid];
+                p.C[(int64_t)(w.m0 / 128) * p.ldc + w.n0 + tid] = s;
+            }
+            asm volatile("bar.sync 1, 256;\n" ::: "memory");
+            continue;
+        }
         if (p.C) {
             double* C = p.C + p.c_off0 + (int64_t)w.z * p.c_zstep;
             if (p.beta != 0.0) {
@@ -187,6 +199,94 @@ gemm_tma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                     CT[(int64_t)(col + 1) * p.ldct + row] = p.alpha * acc[i][j][1];
                 }
             }
+        }
+    }
+}
+
+
+// ------------------------------------------------------------------------------------------
+// Trailing update of the blocked Cholesky with the same TMA / mbarrier / DMMA pipeline:
+//     C[i-tile, j-tile] -= L[i rows, kcol0 : kcol0 + 16*nk] * L[j rows, same columns]^T
+// for the lower tiles (j <= i) of a rectangular range of tiles.  One tile per CTA (not
+// persistent) so that the higher-priority panel stream of the look-ahead schedule can slip its
+// small kernels in between tiles.  A and B are both K-contiguous row panels of the SAME
+// row-major matrix, hence one tensor map.
+// ------------------------------------------------------------------------------------------
+// same ring depth as gemm_tma_kernel
+constexpr int SY_STAGES = 5;
+constexpr int SY_SMEM_BYTES = SY_STAGES * SW_STAGE_BYTES + 4 * 128 * 8 + 2 * SY_STAGES * 8 + 128;
+
+struct SyrkParams {
+    double* C;          // base of the matrix (row-major, ld)
+    int64_t ld;
+    int row_t0, col_t0; // first row tile / column tile of this launch's grid
+    int kcol0;          // first column of the panel block
+    int nk;             // k16 steps (panel width / 16)
+    int skip_first;     // leave out tile (row_t0, col_t0): it was updated by the latency kernel on the critical chain
+};
+
+__global__ void __launch_bounds__(SW_THREADS, 1)
+syrk_tma_kernel(const __grid_constant__ CUtensorMap tmL, SyrkParams p) {
+    extern __shared__ __align__(128) unsigned char sw_smem[];
+    double* stage_base = reinterpret_cast<double*>(sw_smem);
+    uint64_t* full = reinterpret_cast<uint64_t*>(sw_smem + SY_STAGES * SW_STAGE_BYTES + 4 * 128 * 8);
+    uint64_t* empty = full + SY_STAGES;
+    const int it = p.row_t0 + blockIdx.y, jt = p.col_t0 + blockIdx.x;
+    pdl_launch_dependents();
+    if (jt > it || (p.skip_first && blockIdx.x == 0 && blockIdx.y == 0)) return;
+    pdl_wait();
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int m0 = it * 128, n0 = jt * 128;
+
+    if (tid == 0) {
+        for (int s = 0; s < SY_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 8); }
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    __syncthreads();
+
+    if (warp == 8) {
+        if (lane == 0) {
+            int stage = 0;
+            uint32_t phase = 0;
+            for (int kt = 0; kt < p.nk; ++kt) {
+                mbar_wait(&empty[stage], phase ^ 1);
+                const int k0 = p.kcol0 + kt * 16;
+                tma_stage_load(stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES), &full[stage], &tmL, k0, m0, &tmL, k0, n0);
+                if (++stage == SY_STAGES) { stage = 0; phase ^= 1; }
+            }
+        }
+        return;
+    }
+
+    const int wm = (warp & 3) * 32, wn = (warp >> 2) * 64;
+    const int fr = lane >> 2, fk = lane & 3;
+    int stage = 0;
+    uint32_t phase = 0;
+    double acc[4][8][2];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 8; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
+
+    for (int kt = 0; kt < p.nk; ++kt) {
+        mbar_wait(&full[stage], phase);
+        const double* st = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES);
+        dmma_stage<0, 4, 32>(st + ((wm + fr) << 2) + fk, st + SW_OPER_DOUBLES + ((wn + fr) << 2) + fk, acc);
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[stage]);
+        if (++stage == SY_STAGES) { stage = 0; phase ^= 1; }
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int row = m0 + wm + i * 8 + fr;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int col = n0 + wn + j * 8 + 2 * fk;
+            double2* dst = reinterpret_cast<double2*>(p.C + (int64_t)row * p.ld + col);
+            double2 o = *dst;
+            o.x -= acc[i][j][0];
+            o.y -= acc[i][j][1];
+            *dst = o;
         }
     }
 }

@@ -1,7 +1,7 @@
 // sweep_fused.cuh — ONE kernel for the whole candidate sweep of a scalar GP (p = 1):
 //     K(X*, X) tile  ->  W = L^-1 K*^T on the FP64 tensor pipe  ->  sum_i W_ic^2 (variance) and sum_i W_ic beta_i
 //     (mean: k*^T alpha = (L^-1 k*)^T (L^-1 delta))  ->  EI / PI / UCB  ->  scores
-// replacing the three launches per chunk of the large-n path (ks_build_kernel, sweep_tma_kernel,
+// replacing the three launches per chunk of the large-n path (ks_build_kernel, gemm_tma_kernel<EPI_COLSUMSQ>,
 // acq_epilogue_kernel) and the HBM round trip of the K* chunk between them.
 // Reference call sites: acq(surrogate, grid) in optimize_acquisition (acq_utils.jl:44-52) ->
 // ExpectedImprovement.jl:40-66 / ProbabilityImprovement.jl:38-63 / UpperConfidenceBound.jl:38-45 ->
@@ -10,8 +10,9 @@
 // Persistent, one CTA per SM; a CTA OWNS whole candidate tiles (128 candidates) and walks all row tiles
 // of L^-1 for them, so
 //   * the K* tile (128 x n) of a candidate tile is private to its CTA: the eight DMMA warps BUILD the tile
-//     of the CTA's next candidate tile into a double-buffered private scratch (n <= 2048: <= 4 MB per CTA,
-//     written once and re-read through L2 by TMA) before contracting the current one — the kernel
+//     of the CTA's next candidate tile into a double-buffered private scratch (2 x 128 x ceil16(n) doubles per
+//     CTA, written once and read back by TMA; it stays in L2 only for small n: 4 MiB per CTA at n = 2048, 32 MiB
+//     at n = 16384) before contracting the current one — the kernel
 //     evaluations and the DMMA work share the FP64 pipe anyway, so running them back to back in the same
 //     warps loses nothing and needs no cross-CTA synchronisation;
 //   * every candidate tile costs the same, so the static schedule tile = b, b + G, ... is balanced;
@@ -29,12 +30,16 @@
 #include <type_traits>
 
 #include "kernels.cuh"
-#include "sweep_tma.cuh"
+#include "tma_pipe.cuh"
 
 namespace abo {
 
 constexpr int FS_STAGES = 5;
 constexpr int FS_THREADS = 256 + 32;
+// Largest padded system (Npad) of a scalar GP that takes the fused sweep; larger systems take the three-kernel path.  The
+// bound is the private K* scratch, 2 x 128 x Kld x 8 B per CTA, allocated for every SM: 32 MiB per CTA and 4.97 GB on 148 SMs
+// at n = 16384.
+constexpr int64_t FS_MAX_NPAD = 16384;
 
 struct FusedParams {
     KSpec spec;
@@ -52,7 +57,6 @@ struct FusedParams {
     double* var_out;
     double* score_out;
     int ntiles;             // candidate tiles = ceil(m / 128)
-    int dbg;                // timing experiments only (ABO_FUSED_DBG): 1 = skip the K* evaluation, 2 = skip the contraction
 };
 
 template <int DT>
@@ -63,45 +67,22 @@ constexpr int fused_smem_bytes() {
 __device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;\n" ::: "memory"); }
 __device__ __forceinline__ void bar_consumers() { asm volatile("bar.sync 1, 256;\n" ::: "memory"); }
 
-// one k16 stage of the 128 x 128 product; fragment rows interleaved: warp q owns rows 8 (4 i + q) + fr
-// Only the row fragments ILO <= i < IHI of this warp are live (compile-time: straight-line code for every range; a
-// run-time predicate inside the unrolled loops cost as much as the DMMAs it skipped).  Partial ranges occur in the
-// last row tile of a system that is not a multiple of 128, and inside the diagonal block (rows above the diagonal).
-template <int ILO, int IHI>
-__device__ __forceinline__ void fused_stage(const double* __restrict__ a_s, const double* __restrict__ b_s, double (&acc)[4][8][2]) {
-    double a[2][4], bb[2][8];
-#pragma unroll
-    for (int i = ILO; i < IHI; ++i) a[0][i] = a_s[i * 128];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) bb[0][j] = b_s[j * 32];
-#pragma unroll
-    for (int kk = 0; kk < 4; ++kk) {
-        const int cur = kk & 1, nxt = cur ^ 1;
-        if (kk < 3) {
-#pragma unroll
-            for (int i = ILO; i < IHI; ++i) a[nxt][i] = a_s[(kk + 1) * 512 + i * 128];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) bb[nxt][j] = b_s[(kk + 1) * 512 + j * 32];
-        }
-#pragma unroll
-        for (int i = ILO; i < IHI; ++i)
-#pragma unroll
-            for (int j = 0; j < 8; ++j) dmma8x8x4(acc[i][j][0], acc[i][j][1], a[cur][i], bb[cur][j]);
-    }
-}
+// one k16 stage of the 128 x 128 product; fragment rows interleaved: warp q owns rows 8 (4 i + q) + fr.  Only the row
+// fragments ilo <= i < ihi of this warp are live; partial ranges occur in the last row tile of a system that is not a
+// multiple of 128, and inside the diagonal block (rows above the diagonal).
 __device__ __forceinline__ void fused_stage_range(const double* __restrict__ a_s, const double* __restrict__ b_s, double (&acc)[4][8][2],
                                                   int ilo, int ihi) {
     switch (ilo * 5 + ihi) {
-        case 0 * 5 + 4: fused_stage<0, 4>(a_s, b_s, acc); break;
-        case 0 * 5 + 3: fused_stage<0, 3>(a_s, b_s, acc); break;
-        case 0 * 5 + 2: fused_stage<0, 2>(a_s, b_s, acc); break;
-        case 0 * 5 + 1: fused_stage<0, 1>(a_s, b_s, acc); break;
-        case 1 * 5 + 4: fused_stage<1, 4>(a_s, b_s, acc); break;
-        case 1 * 5 + 3: fused_stage<1, 3>(a_s, b_s, acc); break;
-        case 1 * 5 + 2: fused_stage<1, 2>(a_s, b_s, acc); break;
-        case 2 * 5 + 4: fused_stage<2, 4>(a_s, b_s, acc); break;
-        case 2 * 5 + 3: fused_stage<2, 3>(a_s, b_s, acc); break;
-        case 3 * 5 + 4: fused_stage<3, 4>(a_s, b_s, acc); break;
+        case 0 * 5 + 4: dmma_stage<0, 4, 128>(a_s, b_s, acc); break;
+        case 0 * 5 + 3: dmma_stage<0, 3, 128>(a_s, b_s, acc); break;
+        case 0 * 5 + 2: dmma_stage<0, 2, 128>(a_s, b_s, acc); break;
+        case 0 * 5 + 1: dmma_stage<0, 1, 128>(a_s, b_s, acc); break;
+        case 1 * 5 + 4: dmma_stage<1, 4, 128>(a_s, b_s, acc); break;
+        case 1 * 5 + 3: dmma_stage<1, 3, 128>(a_s, b_s, acc); break;
+        case 1 * 5 + 2: dmma_stage<1, 2, 128>(a_s, b_s, acc); break;
+        case 2 * 5 + 4: dmma_stage<2, 4, 128>(a_s, b_s, acc); break;
+        case 2 * 5 + 3: dmma_stage<2, 3, 128>(a_s, b_s, acc); break;
+        case 3 * 5 + 4: dmma_stage<3, 4, 128>(a_s, b_s, acc); break;
         default: break;                                              // empty range
     }
 }
@@ -162,15 +143,8 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                     const int m0 = ib * 128;
                     for (int kt = 0; kt < nk; ++kt) {
                         mbar_wait(&empty[stage], phase ^ 1);
-                        mbar_expect_tx(&full[stage], SW_STAGE_BYTES);
-                        double* sa = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES);
-                        double* sb = sa + SW_OPER_DOUBLES;
-                        const int k0 = kt * 16;
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            tma_load_2d(sa + q * 512, &tmA, k0 + 4 * q, m0, &full[stage]);
-                            tma_load_2d(sb + q * 512, &tmB, k0 + 4 * q, brow, &full[stage]);
-                        }
+                        tma_stage_load(stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES), &full[stage], &tmA, kt * 16, m0,
+                                       &tmB, kt * 16, brow);
                         if (++stage == FS_STAGES) { stage = 0; phase ^= 1; }
                     }
                 }
@@ -205,7 +179,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
             sc[e] = (k < d && gc < p.m) ? p.spec.sk(k) * p.Xc[gc * d + k] : 0.0;
         }
         bar_consumers();
-        const int nitems = ((p.dbg & 1) && j > 1) ? 0 : (int)((n + 31) / 32) * 4;
+        const int nitems = (int)((n + 31) / 32) * 4;
         auto items = [&](auto fam_tag) {
             constexpr int FAM = decltype(fam_tag)::value;
             constexpr bool PREF = DT <= 12;                           // next item's coordinates loaded one item ahead (register budget)
@@ -282,11 +256,11 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
             // k16 steps left of the diagonal block: every live row fragment; inside the diagonal block (k0 = m0 + 16 t) only the
             // rows >= k0 are non-zero in L^-1: fragments f >= 2 t, i.e. i >= ceil((2 t - q) / 4) for this warp — the
             // upper-triangle half of the diagonal tile is never multiplied (it is (T + 1) / T of the work at T row tiles)
-            const int nk_full = (rows == 128 && !(p.dbg & 2)) ? min(nk, ib * 8) : 0;
+            const int nk_full = (rows == 128) ? min(nk, ib * 8) : 0;
             for (int kt = 0; kt < nk_full; ++kt) {
                 mbar_wait(&full[stage], phase);
                 const double* st = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES);
-                fused_stage<0, 4>(st + a_off, st + b_off, acc);
+                dmma_stage<0, 4, 128>(st + a_off, st + b_off, acc);
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&empty[stage]);
                 if (++stage == FS_STAGES) { stage = 0; phase ^= 1; }
@@ -296,7 +270,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 const double* st = stage_base + (size_t)stage * (2 * SW_OPER_DOUBLES);
                 const int t = kt - ib * 8;                            // < 0 left of the diagonal block
                 const int ilo = t > 0 ? max(0, (2 * t - q + 3) >> 2) : 0;
-                if (!(p.dbg & 2)) fused_stage_range(st + a_off, st + b_off, acc, ilo, ni);
+                fused_stage_range(st + a_off, st + b_off, acc, ilo, ni);
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&empty[stage]);
                 if (++stage == FS_STAGES) { stage = 0; phase ^= 1; }

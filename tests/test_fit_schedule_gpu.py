@@ -126,7 +126,7 @@ def _check_same_bits(abo, gp, d, p, X, Y, Xc):
 
 
 # T = 31: no overlap; T = 32: the first overlapped size; T = 33, 65, 66, 129: no outer-block boundary in [b_top, T).
-# N = 16400 is also above ABO_FUSED_MAX, so its posterior takes the three-kernel sweep, not sweep_fused.
+# N = 16400 is also above FS_MAX_NPAD, so its posterior takes the three-kernel sweep (gemm_tma_kernel<EPI_COLSUMSQ>), not sweep_fused.
 @pytest.mark.parametrize("n", [pytest.param(n, id=f"T{_tiles(n, 1)}-n{n}") for n in (3900, 4096, 4097, 4224, 8193, 8400, 16400)])
 def test_standard_fit_across_overlap_schedule(abo, orc, oracle_fit, n):
     post, cond, L_ref = oracle_fit(6, n, 1)

@@ -1,7 +1,8 @@
 """Exercises the HBM-bound kernels of the path once each (for `ncu --set full` captures, profiles/ncu_hbm_kernels_r02_summary.json):
 K build at n = 8192 (kmat_p1_kernel), O(n^2) row append (kvec / trmv_lower / trmvT_lower_partial / reduce_rows / append_commit),
 copy-on-write un-share (copy_lower_tiles), the device top-k selection over 2 M scores (sel_*), the small-n fused sweep (n = 64,
-HBM side: 8 (d + 1) B per candidate) and the three-kernel GradientGP sweep (ks_build_kernel<.., true>, acq_epilogue_kernel)."""
+HBM side: 8 (d + 1) B per candidate) and the three-kernel GradientGP sweep (ks_build_kernel<.., true>, gemm_tma_kernel<EPI_COLSUMSQ>,
+acq_epilogue_kernel)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -24,6 +25,6 @@ g64.gpx.acq_eval_dev(acq.acq_id, acq.params(), Xc.data_ptr(), m, S.data_ptr(), k
 c3 = orc.make_config("C3", n=128, m=16384)
 kg = c3["scale"] * abo.with_lengthscale(abo.ApproxMatern52Kernel(), 1.0 / c3["inv_ls"])
 gg = abo.update(abo.GradientGP(kg, 11, c3["noise"]), c3["X"], c3["Y"])
-abo.ExpectedImprovement(*c3["acq_params"])(gg, c3["Xc"])                                   # ks_build<GRAD> + sweep_tma + acq_epilogue
+abo.ExpectedImprovement(*c3["acq_params"])(gg, c3["Xc"])                                   # ks_build<GRAD> + gemm_tma<EPI_COLSUMSQ> + acq_epilogue
 torch.cuda.synchronize()
 print("hbm_kernels_probe done")

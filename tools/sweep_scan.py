@@ -1,7 +1,7 @@
-"""Device-resident sweep throughput as a function of n (the fused single-kernel path vs the three-kernel path):
+"""Device-resident sweep throughput of the fused single-kernel path as a function of n:
 EI + stable top-100 over m candidates already in HBM (abo_acq_eval_dev), CUDA events on the library's stream.
     python tools/sweep_scan.py [--n 64,128,...] [--d 20] [--m 2097152] [--kind 0] [--label fused]
-Set ABO_FUSED_MAX=0 in the environment to force the three-kernel path.  Prints one JSON line per n:
+(profiles/sweep_scan_r02.jsonl also records the three-kernel path at the same n for comparison.)  Prints one JSON line per n:
 candidates/s, algorithmic TFLOP/s (n^2 and n^2 + 3nd + 4n per candidate), fraction of the measured FP64 peak,
 and the candidate-stream GB/s (8(d+1) B per candidate) for the small-n, HBM-side view."""
 import argparse, json, os, sys
@@ -16,7 +16,7 @@ ap.add_argument("--n", default="64,128,256,512,1024,2048")
 ap.add_argument("--d", type=int, default=20)
 ap.add_argument("--m", type=int, default=1 << 21)
 ap.add_argument("--kind", type=int, default=0)
-ap.add_argument("--label", default=os.environ.get("ABO_FUSED_MAX", "default"))
+ap.add_argument("--label", default="fused")
 ap.add_argument("--reps", type=int, default=3)
 args = ap.parse_args()
 KN = {0: "SqExponentialKernel", 1: "Matern52Kernel", 2: "Matern72Kernel"}
