@@ -20,7 +20,7 @@ SYMBOLS = [
     "abo_gp_clone", "abo_gp_n", "abo_gp_alpha", "abo_gp_factor", "abo_gp_posterior", "abo_gp_posterior_cov", "abo_acq_eval", "abo_acq_eval_dev", "abo_acq_eval_grad",
     "abo_nlml_batch", "abo_potrf_dev", "abo_fill_distance", "abo_nccl_unique_id", "abo_ctx_init_rank", "abo_gp_sync",
     "abo_topk_allgather", "abo_allgather_f64", "abo_ctx_ranks", "abo_ctx_trim", "abo_acq_eval_multi", "abo_standardize", "abo_gp_set_params_ard", "abo_nlml_batch_ard",
-    "abo_gp_posterior_sample",
+    "abo_gp_posterior_sample", "abo_gp_pathwise_sample", "abo_gp_pathwise_sample_dev",
 ]
 
 
@@ -79,6 +79,8 @@ def lib():
             "abo_gp_posterior": [vp, vp, i64, i32, vp, vp],
             "abo_gp_posterior_cov": [vp, vp, i64, i32, vp],
             "abo_gp_posterior_sample": [vp, vp, i64, i64, u64, dbl, vp, vp, vp, C.POINTER(C.c_double)],
+            "abo_gp_pathwise_sample": [vp, vp, i64, i64, i64, u64, vp, vp, vp],
+            "abo_gp_pathwise_sample_dev": [vp, vp, i64, i64, i64, u64, vp, vp, vp],
             "abo_acq_eval": [vp, i32, vp, vp, i64, vp, i64, vp, vp],
             "abo_acq_eval_dev": [vp, i32, vp, vp, i64, vp, i64, vp, vp],
             "abo_acq_eval_multi": [vp, i32, vp, vp, vp, vp, i64, vp, i64, vp, vp],
@@ -340,6 +342,31 @@ class GpHandle:
         check(lib().abo_gp_posterior_sample(self._h, ptr(Xc), m, S, seed, float(jitter),
                                             ptr(samples), ptr(ai), ptr(av), C.byref(tau)))
         return samples, ai[:max(S, 0)], av[:max(S, 0)], tau.value
+
+    def pathwise_sample(self, Xc, num_samples, seed, num_features=4096, want_samples=True):
+        """Pathwise posterior draws of the value output over Xc (random-Fourier-feature prior, Matheron's rule):
+        (samples (S, m) or None, argmin indices (S,), argmin values (S,))."""
+        Xc = f64(Xc)
+        if Xc.ndim != 2 or Xc.shape[1] != self.d:
+            raise DimensionMismatch(f"query points must be m x {self.d}")
+        m, S, seed = Xc.shape[0], int(num_samples), int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2^64)")
+        samples = np.empty((max(S, 0), m)) if want_samples else None
+        ai = np.empty(max(S, 1), dtype=np.int64); av = np.empty(max(S, 1))
+        check(lib().abo_gp_pathwise_sample(self._h, ptr(Xc), m, S, int(num_features), seed, ptr(samples), ptr(ai), ptr(av)))
+        return samples, ai[:max(S, 0)], av[:max(S, 0)]
+
+    def pathwise_sample_dev(self, d_xc: int, m: int, num_samples, seed, num_features=4096, d_samples: int = 0):
+        """As pathwise_sample for m device-resident candidates; the S x m draws go to d_samples when it is not 0.
+        Returns (argmin indices (S,), argmin values (S,))."""
+        S, seed = int(num_samples), int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2^64)")
+        ai = np.empty(max(S, 1), dtype=np.int64); av = np.empty(max(S, 1))
+        check(lib().abo_gp_pathwise_sample_dev(self._h, C.c_void_p(d_xc), int(m), S, int(num_features), seed,
+                                               C.c_void_p(d_samples) if d_samples else None, ptr(ai), ptr(av)))
+        return ai[:max(S, 0)], av[:max(S, 0)]
 
     def acq_eval(self, acq_id, params, Xc, k=0, want_scores=True):
         Xc = f64(Xc)

@@ -8,7 +8,7 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from .surrogates import _as_points, _get_minimum, _need_posterior, posterior_sample
+from .surrogates import _as_points, _get_minimum, _need_posterior, pathwise_sample, posterior_sample
 from .parallel import merge_topk
 
 ACQ_EI, ACQ_PI, ACQ_UCB = 0, 1, 2
@@ -96,6 +96,31 @@ class ThompsonSampling(AbstractAcquisition):
 
     def copy(self): return ThompsonSampling(self.seed)
     def update(self, ys, surrogate): return ThompsonSampling(self.seed + 1)
+
+
+@dataclass(frozen=True)
+class PathwiseThompsonSampling(AbstractAcquisition):
+    """Thompson sampling on any grid: the acquisition is minus ONE pathwise posterior draw of f (abo_gp_pathwise_sample,
+    num_features random Fourier features conditioned by Matheron's rule), so its maximiser is the minimiser of that draw.
+    The draw is a function of (seed, x), whatever else the grid holds; `update` advances the seed.  There is no cap on
+    the grid size, unlike ThompsonSampling.  A draw has no gradient here: optimize_acquisition returns the best grid point."""
+    seed: int
+    num_features: int = 4096
+    has_gradient = False
+
+    def __call__(self, surrogate, x):
+        return -pathwise_sample(surrogate, x, 1, seed=self.seed, num_features=self.num_features)[0]
+
+    def topk(self, surrogate, x, k, want_scores=True):
+        s = self(surrogate, x)
+        ti, tv = merge_topk([np.arange(len(s))], [s], k)
+        return (s if want_scores else None), ti, tv
+
+    def value_and_grad(self, surrogate, x):
+        raise TypeError("PathwiseThompsonSampling has no gradient: draws are evaluated at the grid points only")
+
+    def copy(self): return PathwiseThompsonSampling(self.seed, self.num_features)
+    def update(self, ys, surrogate): return PathwiseThompsonSampling(self.seed + 1, self.num_features)
 
 
 ACQ_GRADNORM_UCB = 3

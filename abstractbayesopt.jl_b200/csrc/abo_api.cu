@@ -1,5 +1,5 @@
 // abo_api.cu — C ABI of libabo_cuda.so (include/abo.h): handles, host drivers of the blocked
-// Cholesky / triangular inverse / candidate sweep, top-k selection, joint posterior sampling.  No CPU fallback anywhere:
+// Cholesky / triangular inverse / candidate sweep, top-k selection, joint and pathwise posterior sampling.  No CPU fallback anywhere:
 // every entry point needs a live CUDA device.
 #include <algorithm>
 #include <cmath>
@@ -1319,7 +1319,7 @@ static int gp_posterior_sample_run(abo_gp* g, const double* Xc, int64_t m, int64
         acq_epilogue_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(a, pmean, npb, nullptr, 0, Mpad, m, mu, nullptr, nullptr);
         KL(c);
     }
-    philox_normal_kernel<<<(unsigned)((Spad * Mpad / 4 + 255) / 256), 256, 0, st>>>(seed, S, m, Spad, Mpad, Z);
+    philox_normal_kernel<<<(unsigned)((Spad * Mpad / 4 + 255) / 256), 256, 0, st>>>(seed, 0, 0, 1.0, S, m, Spad, Mpad, Mpad, Z);
     KL(c);
     double tau = 0.0;
     for (int k = 0;; ++k) {
@@ -1350,7 +1350,7 @@ static int gp_posterior_sample_run(abo_gp* g, const double* Xc, int64_t m, int64
         if ((rc = launch_gemm_tma(c, tmL, tmZ, f, st))) return rc;
     }
     long long* aidx = reinterpret_cast<long long*>(amin);
-    sample_finish_kernel<<<(unsigned)S, SF_THREADS, 0, st>>>(F, Mpad, mu, m, aidx, amin + S);
+    sample_finish_kernel<<<(unsigned)S, SF_THREADS, 0, st>>>(F, Mpad, mu, 0.0, m, 0, 0, aidx, amin + S);
     KL(c);
     if (samples)
         CU(cudaMemcpy2DAsync(samples, sizeof(double) * m, F, sizeof(double) * Mpad, sizeof(double) * m, S, cudaMemcpyDeviceToHost, st));
@@ -1359,6 +1359,174 @@ static int gp_posterior_sample_run(abo_gp* g, const double* Xc, int64_t m, int64
     CU(cudaStreamSynchronize(st));
     if (jitter_used) *jitter_used = tau;
     return ABO_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// pathwise posterior draws over any number of candidates (sample.cuh), f_s(x) = mean_c + k(x, X)(alpha - v_s) + phi(x) theta'_s:
+//   once per call   features (Om, b) -> Phi(X) [Npad][Lpad], training rows in point-major output order
+//                   -> Bc[s][Npad + l] = theta'_s[l] and Rt[s][i] = eps_s[i] (Philox) -> Rt += Theta' Phi(X)^T (TMA GEMM)
+//                   -> Y = L^-1 Rt^T (TMA GEMM) -> V = L^-T Y (the cp.async DMMA GEMM, which reads L^-1 transposed)
+//                   -> Bc[s][k] = alpha[k] - V[k][s], k < Npad
+//   per chunk       K* value rows and Phi* of mc candidates -> F = Bc [K* | Phi*]^T [Spad][mc]: two TMA GEMM launches over
+//                   k in [0, Npad) and [Npad, Npad + Lpad), the second accumulating -> + mean_c, running per-draw argmin.
+// Each element of F is one fixed-order reduction over k of quantities that depend on its own candidate and draw only.
+// ------------------------------------------------------------------------------------------
+constexpr int64_t PATH_MAX_S = 4096, PATH_MAX_L = 16384;
+constexpr size_t PATH_CHUNK_BYTES = (size_t)6 << 30;     // K*, Phi* and F of one candidate chunk
+struct PathPlan {
+    int64_t Lpad, Spad, ldb, mc;
+    int npb;
+    double *Om, *bf, *Phi, *Bc, *Ks, *pmean, *F, *amin;
+    CUtensorMap tmB, tmK, tmP;
+};
+
+static int pathwise_prepare(abo_gp* g, int64_t m, int64_t S, int64_t L, uint64_t seed, PathPlan& P) {
+    abo_ctx* c = g->ctx;
+    cudaStream_t st = c->stream;
+    const int64_t Npad = g->Npad, N = g->N;
+    const int d = g->d;
+    const int64_t Lpad = (L + NB - 1) / NB * NB, Spad = (S + NB - 1) / NB * NB, ldb = Npad + Lpad;
+    // chunk: three waves of (draw tile, candidate tile) work items, K* + Phi* + F within PATH_CHUNK_BYTES
+    const int64_t ts = Spad / NB;
+    int64_t mc = NB * ((3 * c->sms + ts - 1) / ts);
+    mc = std::min<int64_t>(mc, (int64_t)(PATH_CHUNK_BYTES / (sizeof(double) * (size_t)(Npad + Lpad + Spad))) / NB * NB);
+    mc = std::max<int64_t>(NB, std::min<int64_t>(mc, (m + NB - 1) / NB * NB));
+    P.Lpad = Lpad; P.Spad = Spad; P.ldb = ldb; P.mc = mc;
+    P.npb = (int)(((Npad + g->p - 1) / g->p + 127) / 128);
+    double *R, *Y;
+    int rc;
+    if ((rc = ws_get(c, WS_PATH_FEAT, sizeof(double) * (size_t)Lpad * (d + 1), (void**)&P.Om)) ||
+        (rc = ws_get(c, WS_PATH_PHI, sizeof(double) * (size_t)std::max(Npad, mc) * Lpad, (void**)&P.Phi)) ||
+        (rc = ws_get(c, WS_PATH_COEF, sizeof(double) * (size_t)Spad * ldb, (void**)&P.Bc)) ||
+        (rc = ws_get(c, WS_PATH_R, sizeof(double) * (size_t)Spad * Npad, (void**)&R)) ||
+        (rc = ws_get(c, WS_PATH_Y, sizeof(double) * (size_t)Npad * Spad, (void**)&Y)) ||
+        (rc = ws_get(c, WS_KS, sizeof(double) * (size_t)mc * Npad, (void**)&P.Ks)) ||
+        (rc = ws_get(c, WS_PMEAN, sizeof(double) * (size_t)P.npb * mc, (void**)&P.pmean)) ||
+        (rc = ws_get(c, WS_PATH_F, sizeof(double) * (size_t)Spad * mc, (void**)&P.F)) ||
+        (rc = ws_get(c, WS_OUT_A, sizeof(double) * (size_t)2 * S, (void**)&P.amin)))
+        return rc;
+    P.bf = P.Om + Lpad * d;
+    const int kdf = g->kind == K_SE ? 0 : (g->kind == K_M52 || g->kind == K_AM52 || g->kind == K_ADM52) ? 5 : 7;
+    rff_params_kernel<<<(unsigned)(Lpad / 128), 128, 0, st>>>(seed, d, kdf, L, Lpad, P.Om, P.bf);
+    KL(c);
+    const int64_t vpts = (Npad + g->p - 1) / g->p;
+    rff_build_kernel<<<dim3((unsigned)(Lpad / 128), (unsigned)((vpts + RFF_PB - 1) / RFF_PB)), 128, 0, st>>>(
+        gp_spec(g), P.Om, P.bf, Lpad, g->dXsT, 1, g->ldx, 0, g->n, g->p, Npad, P.Phi);
+    KL(c);
+    const uint64_t draw_key = 1ull << 63;
+    philox_normal_kernel<<<(unsigned)((Spad * Lpad / 4 + 255) / 256), 256, 0, st>>>(seed, draw_key, 0, std::sqrt(2.0 * g->scale / (double)L),
+                                                                                   S, L, Spad, Lpad, ldb, P.Bc + Npad);
+    KL(c);
+    philox_normal_kernel<<<(unsigned)((Spad * Npad / 4 + 255) / 256), 256, 0, st>>>(seed, draw_key, L, std::sqrt(g->noise),
+                                                                                   S, N, Spad, Npad, Npad, R);
+    KL(c);
+    CUtensorMap tmPX;
+    if ((rc = make_tmap_k4(&P.tmB, P.Bc, ldb, Spad, ldb)) || (rc = make_tmap_k4(&tmPX, P.Phi, Lpad, Npad, Lpad))) return rc;
+    {
+        TmaGemmParams q{};                                                   // Rt = E + Theta' Phi(X)^T  [Spad][Npad]
+        q.Mt = (int)(Spad / NB); q.Nt = (int)(Npad / NB); q.batch = 1; q.K = (int)Lpad; q.a_col0 = (int)Npad;
+        q.alpha = 1.0; q.beta = 1.0; q.C = R; q.ldc = Npad;
+        if ((rc = launch_gemm_tma(c, P.tmB, tmPX, q, st))) return rc;
+    }
+    if ((rc = linv_times_ks(c, g, R, Spad, Y, st))) return rc;             // Y = L^-1 R  [Npad][Spad]
+    {
+        GemmParams z{};                                                      // V = L^-T Y  [Npad][Spad], into R's slot
+        z.A = g->dLinv; z.lda = g->ld; z.B = Y; z.ldb = Spad; z.C = R; z.ldc = Spad;
+        z.M = (int)Npad; z.N = (int)Spad; z.K = (int)Npad; z.alpha = 1.0; z.beta = 0.0; z.flags = KLO_M;
+        CU((launch_gemm(z, 1, st)));
+        KL(c);
+    }
+    pathwise_coef_kernel<<<dim3((unsigned)(Npad / 32), (unsigned)(Spad / 32)), dim3(32, 8), 0, st>>>(g->dAlpha, N, R, Npad, Spad,
+                                                                                                  P.Bc, ldb);
+    KL(c);
+    if ((rc = make_tmap_k4(&P.tmK, P.Ks, Npad, mc, Npad)) || (rc = make_tmap_k4(&P.tmP, P.Phi, Lpad, mc, Lpad))) return rc;
+    return ABO_OK;
+}
+
+// the draws at m device-resident candidates dXc, global indices off .. off + m - 1; samples (nullable) is the caller's
+// S x ldo output (host or device memory, `kind`), written at column off
+static int pathwise_chunks(abo_gp* g, const PathPlan& P, const double* dXc, int64_t m, int64_t S, int64_t off, double* samples,
+                           int64_t ldo, cudaMemcpyKind kind, int64_t* nchunk) {
+    abo_ctx* c = g->ctx;
+    cudaStream_t st = c->stream;
+    const int64_t Npad = g->Npad, mc = P.mc;
+    long long* aidx = reinterpret_cast<long long*>(P.amin);
+    int rc;
+    for (int64_t c0 = 0; c0 < m; c0 += mc) {
+        const int64_t mvalid = std::min(mc, m - c0), mc_eff = (mvalid + NB - 1) / NB * NB;
+        if ((rc = launch_ks_d(c, g, dXc, c0, m, 0, P.Ks, P.pmean, mc_eff, mc, P.npb, st))) return rc;
+        rff_build_kernel<<<dim3((unsigned)(P.Lpad / 128), (unsigned)(mc_eff / RFF_PB)), 128, 0, st>>>(
+            gp_spec(g), P.Om, P.bf, P.Lpad, dXc + c0 * g->d, g->d, 1, 1, mvalid, 1, mc_eff, P.Phi);
+        KL(c);
+        TmaGemmParams q{};                                                   // F = Bc[:, 0:Npad] K*^T   [Spad][mc]
+        q.Mt = (int)(P.Spad / NB); q.Nt = (int)(mc_eff / NB); q.batch = 1; q.K = (int)Npad;
+        q.alpha = 1.0; q.beta = 0.0; q.C = P.F; q.ldc = mc;
+        if ((rc = launch_gemm_tma(c, P.tmB, P.tmK, q, st))) return rc;
+        q.K = (int)P.Lpad; q.a_col0 = (int)Npad; q.beta = 1.0;               //   += Bc[:, Npad:] Phi*^T
+        if ((rc = launch_gemm_tma(c, P.tmB, P.tmP, q, st))) return rc;
+        sample_finish_kernel<<<(unsigned)S, SF_THREADS, 0, st>>>(P.F, mc, nullptr, g->mean_c[0], mvalid, off + c0, *nchunk > 0 ? 1 : 0,
+                                                                 aidx, P.amin + S);
+        KL(c);
+        if (samples)
+            CU(cudaMemcpy2DAsync(samples + off + c0, sizeof(double) * ldo, P.F, sizeof(double) * mc, sizeof(double) * mvalid, S,
+                                 kind, st));
+        ++*nchunk;
+    }
+    return ABO_OK;
+}
+
+static int gp_pathwise_run(abo_gp* g, const double* Xc, bool dev, int64_t m, int64_t S, int64_t L, uint64_t seed, double* samples,
+                           int64_t* argmin_idx, double* argmin_val) {
+    if (!g || !Xc) return abo_fail(ABO_ERR_INVALID, "null argument");
+    if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
+    if (S > PATH_MAX_S || L < 1 || L > PATH_MAX_L)
+        return abo_fail(ABO_ERR_INVALID, "pathwise samples need S <= %lld draws and 1 <= L <= %lld features", (long long)PATH_MAX_S,
+                        (long long)PATH_MAX_L);
+    if (g->d > RFF_MAXD) return abo_fail(ABO_ERR_INVALID, "pathwise samples support d <= %d", RFF_MAXD);
+    if (m <= 0 || S <= 0) return ABO_OK;
+    abo_ctx* c = g->ctx;
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    PathPlan P;
+    int rc;
+    if ((rc = pathwise_prepare(g, dev ? m : std::min(m, HOST_PIECE), S, L, seed, P))) return rc;
+    int64_t nchunk = 0;
+    if (dev) {
+        if ((rc = pathwise_chunks(g, P, Xc, m, S, 0, samples, m, cudaMemcpyDeviceToDevice, &nchunk))) return rc;
+    } else {
+        double* dXc;
+        if ((rc = ws_get(c, WS_CAND, sizeof(double) * (size_t)std::min(m, HOST_PIECE) * g->d, (void**)&dXc))) return rc;
+        for (int64_t off = 0; off < m; off += HOST_PIECE) {                 // stream order: piece i + 1 overwrites dXc after piece i
+            const int64_t cnt = std::min(HOST_PIECE, m - off);
+            CU(cudaMemcpyAsync(dXc, Xc + off * g->d, sizeof(double) * cnt * g->d, cudaMemcpyHostToDevice, st));
+            if ((rc = pathwise_chunks(g, P, dXc, cnt, S, off, samples, m, cudaMemcpyDeviceToHost, &nchunk))) return rc;
+        }
+    }
+    if (argmin_idx) CU(cudaMemcpyAsync(argmin_idx, P.amin, sizeof(int64_t) * S, cudaMemcpyDeviceToHost, st));
+    if (argmin_val) CU(cudaMemcpyAsync(argmin_val, P.amin + S, sizeof(double) * S, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return ABO_OK;
+}
+
+static int pathwise_entry(abo_gp* g, const double* Xc, bool dev, int64_t m, int64_t S, int64_t L, uint64_t seed, double* samples,
+                          int64_t* argmin_idx, double* argmin_val) {
+    const int rc = gp_pathwise_run(g, Xc, dev, m, S, L, seed, samples, argmin_idx, argmin_val);
+    if (rc && g && g->ctx) {
+        // as abo_gp_posterior_sample: nothing may still be writing workspace slots or the caller's buffers
+        const std::string keep = g_err;
+        ctx_sync_all(g->ctx);
+        cudaGetLastError();
+        g_err = keep;
+    }
+    return rc;
+}
+extern "C" int32_t abo_gp_pathwise_sample(abo_gp* g, const double* Xc, int64_t m, int64_t S, int64_t L, uint64_t seed,
+                                          double* samples, int64_t* argmin_idx, double* argmin_val) {
+    return pathwise_entry(g, Xc, false, m, S, L, seed, samples, argmin_idx, argmin_val);
+}
+extern "C" int32_t abo_gp_pathwise_sample_dev(abo_gp* g, const double* d_Xc, int64_t m, int64_t S, int64_t L, uint64_t seed,
+                                              double* d_samples, int64_t* argmin_idx, double* argmin_val) {
+    return pathwise_entry(g, d_Xc, true, m, S, L, seed, d_samples, argmin_idx, argmin_val);
 }
 
 // ---- stable descending top-k with Julia isless semantics (NaN largest, -0.0 < 0.0)

@@ -3,9 +3,13 @@
 // the standard normals z from a counter-based Philox4x64-10 stream that is pinned to NumPy's `Philox` bit generator, and
 // a per-draw epilogue that adds the mean and finds the minimising candidate.  The O(m^3) / O(m^2 S) products run on the
 // persistent TMA GEMM (gemm_tma.cuh) and the look-ahead Cholesky; see the driver in abo_api.cu.
+// Also the feature generator, feature builder and coefficient transpose of the pathwise sampler (abo_gp_pathwise_sample).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
+#include <math_constants.h>
+
+#include "kernels.cuh"
 
 namespace abo {
 
@@ -26,29 +30,47 @@ __device__ __forceinline__ void philox4x64_10(uint64_t c[4], uint64_t k0, uint64
 // uniform in (0, 1): the top 53 bits, centred in their interval (never 0, so the logarithm below is finite)
 __device__ __forceinline__ double philox_u01(uint64_t w) { return ((double)(w >> 11) + 0.5) * 0x1.0p-53; }
 
-// Z^T [Spad][ld]: Z[s][i] for draw s < S and candidate i < m, zero elsewhere.  Block j of draw s is Philox with
-// key (seed, s) and counter (j + 1, 0, 0, 0) -- the words np.random.Philox(key=[seed, s]).random_raw() returns at
-// positions 4j .. 4j+3, since NumPy increments the counter before each block.  Its four words give candidates 4j .. 4j+3
-// by two Box-Muller pairs: (r0 cos 2 pi u1, r0 sin 2 pi u1, r2 cos 2 pi u3, r2 sin 2 pi u3), r = sqrt(-2 ln u).
-// Z[s][i] depends on (seed, s, i) only.  One thread per block of four; ld is a multiple of 4.
-__global__ void philox_normal_kernel(uint64_t seed, int64_t S, int64_t m, int64_t Spad, int64_t ld, double* __restrict__ Z) {
-    const int64_t nblk = ld / 4;
+// Normals 4j .. 4j+3 of the stream with key (k0, k1): Philox block j, counter (j + 1, 0, 0, 0) -- the words
+// np.random.Philox(key=[k0, k1]).random_raw() returns at positions 4j .. 4j+3, since NumPy increments the counter before
+// each block -- turned into (r0 cos 2 pi u1, r0 sin 2 pi u1, r2 cos 2 pi u3, r2 sin 2 pi u3), r = sqrt(-2 ln u).
+__device__ __forceinline__ void philox_normal4(uint64_t k0, uint64_t k1, uint64_t j, double z[4]) {
+    uint64_t c[4] = {j + 1, 0, 0, 0};
+    philox4x64_10(c, k0, k1);
+    double sn, cs;
+    const double r0 = sqrt(-2.0 * log(philox_u01(c[0])));
+    sincospi(2.0 * philox_u01(c[1]), &sn, &cs);
+    z[0] = r0 * cs; z[1] = r0 * sn;
+    const double r2 = sqrt(-2.0 * log(philox_u01(c[2])));
+    sincospi(2.0 * philox_u01(c[3]), &sn, &cs);
+    z[2] = r2 * cs; z[3] = r2 * sn;
+}
+
+// Z [Spad][ld], columns [0, width): Z[s][i] = scale * normal (idx_off + i) of the stream with key (seed, key_off + s), for
+// draw s < S and i < m, zero elsewhere.  Z[s][i] depends on (seed, key_off + s, idx_off + i) only.  One thread per four
+// columns; width and ld are multiples of 4.  The joint sampler uses key_off = idx_off = 0 and scale = 1.
+__global__ void philox_normal_kernel(uint64_t seed, uint64_t key_off, int64_t idx_off, double scale, int64_t S, int64_t m,
+                                     int64_t Spad, int64_t width, int64_t ld, double* __restrict__ Z) {
+    const int64_t nblk = width / 4;
     const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (t >= Spad * nblk) return;
     const int64_t s = t / nblk, j = t % nblk;
     double z[4] = {0.0, 0.0, 0.0, 0.0};
     if (s < S && 4 * j < m) {
-        uint64_t c[4] = {(uint64_t)j + 1, 0, 0, 0};
-        philox4x64_10(c, seed, (uint64_t)s);
-        double sn, cs;
-        const double r0 = sqrt(-2.0 * log(philox_u01(c[0])));
-        sincospi(2.0 * philox_u01(c[1]), &sn, &cs);
-        z[0] = r0 * cs; z[1] = r0 * sn;
-        const double r2 = sqrt(-2.0 * log(philox_u01(c[2])));
-        sincospi(2.0 * philox_u01(c[3]), &sn, &cs);
-        z[2] = r2 * cs; z[3] = r2 * sn;
+        const uint64_t key = key_off + (uint64_t)s;
+        const int64_t q0 = idx_off + 4 * j, b0 = q0 / 4, sh = q0 % 4;
+        double a[4];
+        philox_normal4(seed, key, (uint64_t)b0, a);
+        if (sh == 0) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) if (4 * j + q >= m) z[q] = 0.0;
+            for (int q = 0; q < 4; ++q) z[q] = a[q];
+        } else {                                      // the four normals straddle two blocks
+            double b[4];
+            philox_normal4(seed, key, (uint64_t)b0 + 1, b);
+#pragma unroll
+            for (int q = 0; q < 4; ++q) z[q] = (q + sh < 4) ? a[q + sh] : b[q + sh - 4];
+        }
+#pragma unroll
+        for (int q = 0; q < 4; ++q) z[q] = (4 * j + q < m) ? z[q] * scale : 0.0;
     }
     double2* dst = reinterpret_cast<double2*>(Z + s * ld + 4 * j);
     dst[0] = make_double2(z[0], z[1]);
@@ -73,18 +95,21 @@ __device__ __forceinline__ uint64_t findmin_key(double v) {
     return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
 }
 
-// One CTA per draw s: F[s][i] += mu[i] in place for i < m (the draw, sample-major), and the draw's minimiser in that
-// order, ties to the smallest index, written to idx[s] / val[s].  The reduction tree is fixed, so the result is too.
+// One CTA per draw s: F[s][i] += mu[i] (or + mu_c when mu is null) in place for i < m (the draw, sample-major), and the
+// draw's minimiser in that order, ties to the smallest index, written to idx[s] / val[s] as off + i.  With carry, the
+// chunk's minimiser replaces the (idx[s], val[s]) of the earlier chunks only when it is strictly smaller in that order: the
+// earlier chunks hold the smaller indices.  The reduction tree is fixed, so the result is too.
 constexpr int SF_THREADS = 256;
 __global__ void __launch_bounds__(SF_THREADS) sample_finish_kernel(double* __restrict__ F, int64_t ld, const double* __restrict__ mu,
-                                                                   int64_t m, long long* __restrict__ idx, double* __restrict__ val) {
+                                                                   double mu_c, int64_t m, int64_t off, int carry,
+                                                                   long long* __restrict__ idx, double* __restrict__ val) {
     __shared__ uint64_t sk[SF_THREADS];
     __shared__ long long si[SF_THREADS];
     double* row = F + (int64_t)blockIdx.x * ld;
     uint64_t bk = ~0ull;
     long long bi = -1;
     for (int64_t i = threadIdx.x; i < m; i += SF_THREADS) {
-        const double v = row[i] + mu[i];
+        const double v = mu ? row[i] + mu[i] : row[i] + mu_c;
         row[i] = v;
         const uint64_t k = findmin_key(v);
         if (bi < 0 || k < bk) { bk = k; bi = i; }       // indices ascend per thread: strict < keeps the first
@@ -102,8 +127,109 @@ __global__ void __launch_bounds__(SF_THREADS) sample_finish_kernel(double* __res
         __syncthreads();
     }
     if (threadIdx.x == 0) {
-        idx[blockIdx.x] = si[0];
-        val[blockIdx.x] = row[si[0]];
+        const double v = row[si[0]];
+        if (!carry || findmin_key(v) < findmin_key(val[blockIdx.x])) {
+            idx[blockIdx.x] = off + si[0];
+            val[blockIdx.x] = v;
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// pathwise posterior draws (abo_gp_pathwise_sample): random-Fourier-feature prior draws conditioned by Matheron's rule,
+//     f_s(x) = mean_c + k(x, X) (alpha - v_s) + phi(x) . theta'_s,      v_s = (K + noise I)^-1 (phi(X) theta'_s + eps_s).
+// The library stores coordinates scaled, s (.) x, so the device keeps each frequency in those coordinates:
+// Om[l][k] = z_lk t_l, and omega_l . x = Om_l . (s (.) x).  A derivative output d/dx_k carries the factor s_k Om[l][k].
+// ------------------------------------------------------------------------------------------
+
+// Feature l < L: the stream with key (seed, 2^64 - 1 - l).  Normals [0, d) are z_l, normals [d, d + kdf) are g_l, and the
+// phase is b_l = 2 pi u01(word 0 of the first block after them).  t_l = 1 (SE, kdf = 0) or sqrt(kdf / |g_l|^2) (Matern,
+// a Student-t frequency with kdf = 2 nu degrees of freedom).  Features l in [L, Lpad) have Om = 0 and b = 0; their weights
+// theta' are 0.  One thread per feature.  Om [Lpad][d], b [Lpad].
+__global__ void rff_params_kernel(uint64_t seed, int d, int kdf, int64_t L, int64_t Lpad, double* __restrict__ Om,
+                                  double* __restrict__ b) {
+    const int64_t l = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (l >= Lpad) return;
+    double* om = Om + l * d;
+    if (l >= L) {
+        for (int k = 0; k < d; ++k) om[k] = 0.0;
+        b[l] = 0.0;
+        return;
+    }
+    const uint64_t key = ~0ull - (uint64_t)l;
+    const int nz = d + kdf, nblk = (nz + 3) / 4;
+    double g2 = 0.0;
+    for (int j = 0; j < nblk; ++j) {
+        double z[4];
+        philox_normal4(seed, key, (uint64_t)j, z);
+        for (int q = 0; q < 4; ++q) {
+            const int i = 4 * j + q;
+            if (i < d) om[i] = z[q];
+            else if (i < nz) g2 = fma(z[q], z[q], g2);
+        }
+    }
+    if (kdf > 0) {
+        const double t = sqrt((double)kdf / g2);
+        for (int k = 0; k < d; ++k) om[k] *= t;
+    }
+    uint64_t c[4] = {(uint64_t)nblk + 1, 0, 0, 0};
+    philox4x64_10(c, seed, key);
+    b[l] = 2.0 * CUDART_PI * philox_u01(c[0]);
+}
+
+// Feature rows of `count` points: Phi[r][l] for l < Lpad, k-contiguous (ld = Lpad), for the GEMM operands.
+//   Point i's scaled coordinates are xs_k = X[i xi + k xk] * (scale_in ? s_k : 1): raw candidates (xi = d, xk = 1,
+//   scale_in) or the library's XsT (xi = 1, xk = ldx).  ph = (sum_k Om[l][k] xs_k, in k order) + b_l.
+//   p = 1: row i = cos(ph).  p = d + 1 (training side of a GradientGP): rows i p + a in the library's point-major order,
+//   a = 0 cos(ph), a >= 1 -s_{a-1} Om[l][a-1] sin(ph).  Rows of points i >= count, up to rows_out, are zero.
+// Every element is evaluated alone in a fixed order, so a point's features do not depend on the set it is in.
+// grid (Lpad / 128, ceil(rows_out / p / RFF_PB)), 128 threads = 128 features; the points of a CTA are staged in shared memory.
+constexpr int RFF_PB = 16, RFF_MAXD = 64;
+__global__ void __launch_bounds__(128) rff_build_kernel(KSpec spec, const double* __restrict__ Om, const double* __restrict__ b,
+                                                        int64_t Lpad, const double* __restrict__ X, int64_t xi, int64_t xk,
+                                                        int scale_in, int64_t count, int p, int64_t rows_out,
+                                                        double* __restrict__ Phi) {
+    __shared__ double xs[RFF_PB][RFF_MAXD];
+    const int d = spec.d;
+    const int64_t l = blockIdx.x * 128LL + threadIdx.x;
+    const int64_t i0 = (int64_t)blockIdx.y * RFF_PB;
+    for (int e = threadIdx.x; e < RFF_PB * d; e += 128) {
+        const int c = e / d, k = e - c * d;
+        const int64_t i = i0 + c;
+        xs[c][k] = (i < count) ? (scale_in ? spec.sk(k) * X[i * xi + k * xk] : X[i * xi + k * xk]) : 0.0;
+    }
+    __syncthreads();
+    const double* om = Om + l * d;
+    const double bl = b[l];
+    for (int c = 0; c < RFF_PB; ++c) {
+        const int64_t i = i0 + c;
+        if (i * p >= rows_out) break;
+        double* dst = Phi + i * p * Lpad + l;
+        if (i >= count) {
+            for (int a = 0; a < p; ++a) if (i * p + a < rows_out) dst[a * Lpad] = 0.0;
+            continue;
+        }
+        double ph = 0.0;
+        for (int k = 0; k < d; ++k) ph = fma(om[k], xs[c][k], ph);
+        ph += bl;
+        double sn, cs;
+        sincos(ph, &sn, &cs);
+        dst[0] = cs;
+        for (int a = 1; a < p; ++a) dst[a * Lpad] = -(spec.sk(a - 1) * om[a - 1]) * sn;
+    }
+}
+
+// Bc [Spad][ldb], columns [0, Npad): Bc[s][k] = (k < N ? alpha[k] : 0) - V[k][s], V [Npad][Spad] (the transpose, through a
+// 32 x 32 shared tile).  grid (Npad / 32, Spad / 32), block (32, 8).
+__global__ void pathwise_coef_kernel(const double* __restrict__ alpha, int64_t N, const double* __restrict__ V, int64_t Npad,
+                                     int64_t Spad, double* __restrict__ Bc, int64_t ldb) {
+    __shared__ double t[32][33];
+    const int64_t k0 = blockIdx.x * 32LL, s0 = blockIdx.y * 32LL;
+    for (int r = threadIdx.y; r < 32; r += 8) t[r][threadIdx.x] = V[(k0 + r) * Spad + s0 + threadIdx.x];
+    __syncthreads();
+    for (int r = threadIdx.y; r < 32; r += 8) {
+        const int64_t k = k0 + threadIdx.x;
+        Bc[(s0 + r) * ldb + k] = (k < N ? alpha[k] : 0.0) - t[threadIdx.x][r];
     }
 }
 

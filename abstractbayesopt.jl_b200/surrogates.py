@@ -235,6 +235,22 @@ def thompson_batch(model, x, q, *, seed, jitter=1e-10):
     return h.posterior_sample(_as_points(x, h.d), q, seed, jitter, want_samples=False)[1]
 
 
+def pathwise_sample(model, x, num_samples, *, seed, num_features=4096):
+    """Pathwise posterior draws of the latent value f over the points x: an (S, m) array, row s = draw s.  Each draw is a
+    function of x (a random-Fourier-feature prior draw with num_features features, conditioned by Matheron's rule): its
+    value at a point does not depend on the other points of x, and the first S' rows of S > S' draws are the S' draws.
+    Unlike posterior_sample there is no cap on the number of points; the features make the prior draw approximate."""
+    h = _need_posterior(model)
+    return h.pathwise_sample(_as_points(x, h.d), num_samples, seed, num_features)[0]
+
+
+def pathwise_thompson_batch(model, x, q, *, seed, num_features=4096):
+    """q candidate indices (0-based) into x: the minimiser of each of q pathwise posterior draws, a Thompson-sampling
+    batch drawn with replacement.  Only the q indices leave the device."""
+    h = _need_posterior(model)
+    return h.pathwise_sample(_as_points(x, h.d), q, seed, num_features, want_samples=False)[1]
+
+
 def unstandardized_mean_and_var(model, xs, params):
     """StandardGP.jl:395-404 / GradientGP.jl:1019-1030."""
     h = _need_posterior(model)

@@ -147,6 +147,45 @@ int32_t abo_gp_posterior_cov(abo_gp* gp, const double* Xc, int64_t m, int32_t ou
 int32_t abo_gp_posterior_sample(abo_gp* gp, const double* Xc, int64_t m, int64_t S, uint64_t seed, double jitter,
                                 double* samples, int64_t* argmin_idx, double* argmin_val, double* jitter_used);
 
+/* Pathwise posterior draws of the latent value f over any number of candidates (Wilson et al., ICML 2020, "Efficiently
+ * sampling functions from Gaussian process posteriors"; BoTorch draw_matheron_paths): a prior draw with L random Fourier
+ * features, conditioned by Matheron's rule,
+ *     f_s(x) = mu(x) + f~_s(x) - k(x, X) v_s,        v_s = (K + noise I)^-1 (f~_s(X) + eps_s),
+ *     f~_s(x) = sqrt(2 sigma^2 / L) sum_l theta_{s,l} cos(omega_l . x + b_l),   eps_s ~ N(0, noise I),
+ * computed as mean_c + k(x, X)(alpha - v_s) + f~_s(x). The cost is O((n p + L) S) per candidate, with no m x m matrix.
+ * The draws are exact given the features and the prior draw is the feature approximation; for a small set, the exact
+ * joint distribution is abo_gp_posterior_sample. Value output, in the model's units (those of abo_gp_posterior's mean),
+ * for StandardGP (isotropic or ARD) and GradientGP (f~_s(X) then holds the derivative outputs too, d f~ / dx_k =
+ * -sqrt(2 sigma^2 / L) sum_l theta_{s,l} omega_{l,k} sin(omega_l . x + b_l)).
+ * samples: S x m, sample-major, as abo_gp_posterior_sample. Nullable. argmin_idx / argmin_val: per draw, in Julia findmin
+ * order (the first NaN if any, otherwise the first smallest value). Both nullable; they do not depend on whether samples
+ * is NULL.
+ * 1 <= S <= 4096, 1 <= L <= 16384, d <= 64; no cap on m. m <= 0 or S <= 0 is a no-op. Host sets above 262144 candidates
+ * are staged in pieces; the per-draw argmin is carried across pieces. The posterior held by gp is only read.
+ * The random stream (Philox4x64-10; "normal i of key K" is block i/4 of np.random.Philox(key=K), counter
+ * (i/4 + 1, 0, 0, 0), its four words turned into normals 4(i/4) .. 4(i/4) + 3 by two Box-Muller pairs, as
+ * abo_gp_posterior_sample):
+ *   draw s:    key (seed, 2^63 + s). Normals [0, L) are theta_s; normals [L, L + N) are eps_s / sqrt(noise_var), indexed
+ *              in the library's point-major system order i*p + out (N = n p), so that a GradientGP's derivative rows get
+ *              noise where the fit adds it.
+ *   feature l: key (seed, 2^64 - 1 - l). Normals [0, d) are z_l and normals [d, d + k) are g_l, with k = 0 for SE, 5 for
+ *              the Matern-5/2 family and 7 for the Matern-7/2 family (Approx and AD Matern included). b_l = 2 pi u, u the
+ *              uniform of word 0 of the first block after those normals, ((w >> 11) + 0.5) 2^-53.
+ *              omega_l = s (.) z_l (SE) or s (.) z_l sqrt(k / |g_l|^2) (Matern: a Student-t frequency with 2 nu degrees of
+ *              freedom, the Matern spectral density), s the per-dimension inverse length scales.
+ * Guarantees: a draw's value at a candidate is bit-identical whatever set it is evaluated in (any m, any piece boundary,
+ * this entry or abo_gp_pathwise_sample_dev); the first S' draws of a call equal those of a call with S'; the same
+ * arguments give the same bits.
+ * Device workspace, with Lp = L, Sp = S and N rounded up to 128 and c the candidate chunk (three waves of 128 x 128 draw x
+ * candidate tiles, bounded by 6 GB for K*, the features and the draws): about
+ * 8 (max(N, c) Lp + Sp (3 N + Lp) + c (N + Sp)) bytes, 5.7 GB at n p = 8192, L = 4096, S = 128 (abo_ctx_trim releases it). */
+int32_t abo_gp_pathwise_sample(abo_gp* gp, const double* Xc, int64_t m, int64_t S, int64_t L, uint64_t seed,
+                               double* samples, int64_t* argmin_idx, double* argmin_val);
+/* The same for m candidates in device memory; d_samples (nullable) is an S x m device buffer; the argmins go to host
+ * memory. */
+int32_t abo_gp_pathwise_sample_dev(abo_gp* gp, const double* d_Xc, int64_t m, int64_t S, int64_t L, uint64_t seed,
+                                   double* d_samples, int64_t* argmin_idx, double* argmin_val);
+
 /* fused acquisition sweep: scores = acq(surrogate, Xc) (ExpectedImprovement.jl:40-45 etc.) and
  * sortperm(scores; rev=true)[1:k] (acq_utils.jl:50-52): stable, descending, NaN first.
  * scores (m) may be NULL — then only the k selected (index, value) pairs leave the device (the

@@ -406,6 +406,19 @@ function posterior_sample(m::Union{CuStandardGP,CuGradientGP}, xs, S::Integer; s
     out
 end
 
+# Pathwise posterior draws of the latent value over xs (random-Fourier-feature prior with num_features features,
+# conditioned by Matheron's rule): an m x S matrix, column s = draw s.  No cap on the number of points; a draw's value at
+# a point does not depend on the other points.  Thompson sampling proposes argmin of each column.
+function pathwise_sample(m::Union{CuStandardGP,CuGradientGP}, xs, S::Integer; seed::Integer, num_features::Integer=4096)
+    m.gpx === nothing && error("surrogate has no posterior: call update(model, xs, ys) first")
+    Xc = Matrix{Float64}(points(collect(xs))); mcount = size(Xc, 2)
+    out = Matrix{Float64}(undef, mcount, S)
+    check(GC.@preserve Xc out ccall((:abo_gp_pathwise_sample, LIB), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, UInt64, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}),
+        m.gpx.h, Xc, mcount, S, num_features, UInt64(seed), out, C_NULL, C_NULL))
+    out
+end
+
 # monte_carlo_fill_distance (src/BO_utils.jl:140-159) on the device; the caller draws the uniform samples
 function fill_distance(X::Matrix{Float64}, S::Matrix{Float64})         # both d x count, column-major = point-major
     out = Ref{Float64}(0.0)
