@@ -4,6 +4,7 @@ library or a CUDA device is missing every call raises."""
 from __future__ import annotations
 
 import ctypes as C
+import itertools
 import os
 
 import numpy as np
@@ -237,6 +238,11 @@ def nccl_unique_id() -> bytes:
 
 _default_ctx = {}
 
+# posterior tokens: a handle takes a fresh one whenever its posterior may change (create, set_params, fit, append, the
+# receiving side of sync), so a token names one posterior state for the life of the process (ids of dead handles are
+# reused, tokens are not)
+_TOKENS = itertools.count(1)
+
 
 def default_context(device: int | None = None) -> Context:
     if device is None:
@@ -256,8 +262,10 @@ class GpHandle:
             check(lib().abo_gp_create(ctx.handle, kernel_id, d, p, C.byref(h)))
             _h = h
         self._h = _h
+        self.token = next(_TOKENS)
 
     def set_params(self, inv_ls, scale, noise, mean_c=None):
+        self.token = next(_TOKENS)
         mc = None if mean_c is None else f64(np.atleast_1d(mean_c))
         if mc is not None and mc.size != self.p:
             raise DimensionMismatch("mean_c must have p entries")
@@ -277,6 +285,7 @@ class GpHandle:
         if y.size != n * self.p:
             raise DimensionMismatch("ys length does not match xs")
         info = C.c_int64(0)
+        self.token = next(_TOKENS)
         rc = lib().abo_gp_fit(self._h, ptr(X), ptr(y), n, C.byref(info))
         check(rc, info.value)
 
@@ -285,6 +294,7 @@ class GpHandle:
         if x.size != self.d or y.size != self.p:
             raise DimensionMismatch("appended observation has the wrong dimension")
         info = C.c_int64(0)
+        self.token = next(_TOKENS)
         rc = lib().abo_gp_append(self._h, ptr(x), ptr(y), C.byref(info))
         check(rc, info.value)
 
@@ -431,6 +441,7 @@ class GpHandle:
         return val, grad, info
 
     def sync(self, root=0):
+        self.token = next(_TOKENS)
         check(lib().abo_gp_sync(self._h, root))
 
     def close(self):

@@ -4,14 +4,15 @@ For the GPU surrogates the posterior mean, variance and the formula are evaluate
 sweep (abo_acq_eval) instead of two posterior passes (ExpectedImprovement.jl:41-42)."""
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 
 import numpy as np
 
-from .surrogates import _as_points, _get_minimum, _need_posterior, pathwise_sample, posterior_sample
+from .surrogates import _as_points, _get_minimum, _max_value_samples, _need_posterior, pathwise_sample, posterior_sample
 from .parallel import merge_topk
 
 ACQ_EI, ACQ_PI, ACQ_UCB = 0, 1, 2
+ACQ_MES = 4
 
 
 class AbstractAcquisition:
@@ -123,6 +124,82 @@ class PathwiseThompsonSampling(AbstractAcquisition):
     def update(self, ys, surrogate): return PathwiseThompsonSampling(self.seed + 1, self.num_features)
 
 
+@dataclass(frozen=True)
+class MaxValueEntropySearch(AbstractAcquisition):
+    """Max-value entropy search (Wang & Jegelka, ICML 2017; BoTorch qMaxValueEntropy), minimising: the expected reduction
+    of the entropy of the minimum value f* from observing x, averaged over num_max_values sampled values y*_k
+    (ABO_ACQ_MES in include/abo.h: (1/K) sum_k h((mu - y*_k) / sigma), evaluated in the fused sweep, with an analytic
+    gradient).  y*_k = min(argmin_val_k, best_y), the minimum of pathwise posterior draw k over the grid clamped at the
+    incumbent (max_value_samples); the draws depend on seed, which `update` advances with the incumbent.
+    topk(surrogate, grid, k) draws y* over the grid, the standard discretisation.  __call__ and value_and_grad reuse the
+    y* of the last topk on the same posterior (the refinement and the reported acquisition value then optimise the
+    function the grid was ranked by); without such a draw they draw over the points they evaluate."""
+    seed: int
+    best_y: float
+    num_max_values: int = 16
+    num_features: int = 4096
+    _cache: dict = field(default_factory=dict, init=False, compare=False, repr=False)
+    acq_id = ACQ_MES
+
+    @staticmethod
+    def _params(ys):
+        return np.concatenate([[float(len(ys))], ys])
+
+    def _draw(self, h, X, best_y):
+        return _max_value_samples(h, X, self.num_max_values, self.seed, self.num_features, best_y)
+
+    def _keep(self, h, ys):
+        self._cache.clear()
+        self._cache.update(token=h.token, ystar=ys)
+
+    def _ystar(self, h, X):
+        if self._cache.get("token") == h.token:
+            return self._cache["ystar"]
+        return self._draw(h, X, self.best_y)
+
+    def __call__(self, surrogate, x):
+        h = _need_posterior(surrogate)
+        X = _as_points(x, h.d)
+        return h.acq_eval(ACQ_MES, self._params(self._ystar(h, X)), X, k=0)[0]
+
+    def value_and_grad(self, surrogate, x):
+        h = _need_posterior(surrogate)
+        X = _as_points(x, h.d)
+        return h.acq_eval_grad(ACQ_MES, self._params(self._ystar(h, X)), X)
+
+    def topk(self, surrogate, x, k, want_scores=True):
+        h = _need_posterior(surrogate)
+        X = _as_points(x, h.d)
+        ys = self._draw(h, X, self.best_y)
+        self._keep(h, ys)
+        return h.acq_eval(ACQ_MES, self._params(ys), X, k=k, want_scores=want_scores)
+
+    def shard_topk(self, surrogate, shard, k, gather):
+        """topk of one rank's shard of a candidate set split over ranks, with the y* of the WHOLE set: each rank draws the
+        per-draw minima over its shard, `gather(values)` returns every rank's values in rank order, and their
+        NaN-propagating elementwise minimum is what one GPU draws over the whole set (a draw's value at a point does not
+        depend on the rest of the set, and min is exact).  Sharded top-k lists then merge to the single-GPU top-k."""
+        h = _need_posterior(surrogate)
+        X = _as_points(shard, h.d)
+        ys = np.minimum(nan_min_reduce(gather(self._draw(h, X, None))), float(self.best_y))
+        self._keep(h, ys)
+        return h.acq_eval(ACQ_MES, self._params(ys), X, k=k)
+
+    def copy(self):
+        return MaxValueEntropySearch(self.seed, self.best_y, self.num_max_values, self.num_features)
+
+    def update(self, ys, surrogate):
+        return MaxValueEntropySearch(self.seed + 1, _get_minimum(surrogate, ys), self.num_max_values, self.num_features)
+
+
+def nan_min_reduce(arrays):
+    """Elementwise minimum of equally long arrays; a NaN in any of them gives NaN there (np.minimum)."""
+    out = np.asarray(arrays[0], dtype=np.float64)
+    for a in arrays[1:]:
+        out = np.minimum(out, np.asarray(a, dtype=np.float64))
+    return out
+
+
 ACQ_GRADNORM_UCB = 3
 
 
@@ -193,12 +270,14 @@ class EnsembleAcquisition(AbstractAcquisition):
         return len(self.acquisitions) <= 8 and all(getattr(a, "acq_id", -1) in (0, 1, 2, 3) and not isinstance(a, EnsembleAcquisition)
                                                    for a in self.acquisitions)
 
-    def _eval(self, surrogate, x, k=0, want_scores=True):
+    def _eval(self, surrogate, x, k=0, want_scores=True, grid=False):
         h = _need_posterior(surrogate)
         if self._fusable():
             return h.acq_eval_multi([a.acq_id for a in self.acquisitions], self.weights, [a.params() for a in self.acquisitions],
                                     _as_points(x, h.d), k=k, want_scores=want_scores)
-        s = sum(w * a(surrogate, x) for w, a in zip(self.weights, self.acquisitions))
+        # the grid sweep of the sequential path is every member's own grid sweep (topk, same scores as the functor), so
+        # that a member which draws per grid (MaxValueEntropySearch) keeps that draw for the refinement
+        s = sum(w * (a.topk(surrogate, x, 0)[0] if grid else a(surrogate, x)) for w, a in zip(self.weights, self.acquisitions))
         ti, tv = merge_topk([np.arange(len(s))], [s], k)
         return s, ti, tv
 
@@ -206,7 +285,7 @@ class EnsembleAcquisition(AbstractAcquisition):
         return self._eval(surrogate, x)[0]
 
     def topk(self, surrogate, x, k, want_scores=True):
-        return self._eval(surrogate, x, k=k, want_scores=want_scores)
+        return self._eval(surrogate, x, k=k, want_scores=want_scores, grid=True)
 
     def value_and_grad(self, surrogate, x):
         return _fd_value_and_grad(self, surrogate, _as_points(x, _need_posterior(surrogate).d))

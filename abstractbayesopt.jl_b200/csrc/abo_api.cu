@@ -56,7 +56,8 @@ static int configure_kernels() {
     CU(cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SY_SMEM_BYTES));
     CU(cudaFuncSetAttribute(gemm_tma_kernel<EPI_STORE>, cudaFuncAttributeMaxDynamicSharedMemorySize, tg_smem_bytes<EPI_STORE>()));
     CU(cudaFuncSetAttribute(gemm_tma_kernel<EPI_COLSUMSQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, tg_smem_bytes<EPI_COLSUMSQ>()));
-#define ABO_FS_CFG(DT) CU(cudaFuncSetAttribute(sweep_fused_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, fused_smem_bytes<DT>()))
+#define ABO_FS_CFG(DT) CU(cudaFuncSetAttribute(sweep_fused_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, fused_smem_bytes<DT>())); \
+    CU(cudaFuncSetAttribute(sweep_fused_kernel<DT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fused_smem_bytes<DT>()))
     ABO_FS_CFG(4); ABO_FS_CFG(8); ABO_FS_CFG(12); ABO_FS_CFG(16); ABO_FS_CFG(20); ABO_FS_CFG(24); ABO_FS_CFG(32);
 #undef ABO_FS_CFG
     return ABO_OK;
@@ -991,8 +992,8 @@ static double phi_prime0(int kind) {
 static bool fused_applies(const abo_gp* g, int bo) {
     return g->p == 1 && bo == 0 && g->d <= 32 && g->Npad <= FS_MAX_NPAD;
 }
-static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const AcqSpec& a, double* d_mean, double* d_var,
-                              double* d_score) {
+static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const AcqSpec& a, const MesSpec* mes, double* d_mean,
+                              double* d_var, double* d_score) {
     abo_ctx* c = g->ctx;
     cudaStream_t st = c->stream;
     FusedParams fp;
@@ -1012,7 +1013,11 @@ static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const Acq
     if ((rc = make_tmap_k4(&tmB, fp.scratch, fp.Kld, (int64_t)c->sms * 2 * NB, fp.Kld))) return rc;
     if ((rc = prof_mark(c)) || (rc = prof_mark(c))) return rc;            // class 0 (K* builder): inside the fused kernel
     if ((rc = prof_mark(c))) return rc;
-#define ABO_FS_RUN(DT) sweep_fused_kernel<DT><<<grid, FS_THREADS, fused_smem_bytes<DT>(), st>>>(tmA, tmB, fp)
+#define ABO_FS_RUN(DT)                                                                                           \
+    do {                                                                                                         \
+        if (mes) sweep_fused_kernel<DT, true><<<grid, FS_THREADS, fused_smem_bytes<DT>(), st>>>(tmA, tmB, fp, *mes); \
+        else sweep_fused_kernel<DT><<<grid, FS_THREADS, fused_smem_bytes<DT>(), st>>>(tmA, tmB, fp, NoMes{});       \
+    } while (0)
     const int d = g->d;
     if (d <= 4) ABO_FS_RUN(4); else if (d <= 8) ABO_FS_RUN(8); else if (d <= 12) ABO_FS_RUN(12); else if (d <= 16) ABO_FS_RUN(16);
     else if (d <= 20) ABO_FS_RUN(20); else if (d <= 24) ABO_FS_RUN(24); else ABO_FS_RUN(32);
@@ -1027,12 +1032,28 @@ static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const Acq
     return ABO_OK;
 }
 
+// ABO_ACQ_MES params = {K, y*_1 .. y*_K}: K an integer-valued double in [1, MES_MAX_K], every y* finite
+static int mes_spec(const double* params, MesSpec* out) {
+    const double K = params[0];
+    if (!(K >= 1.0 && K <= (double)MES_MAX_K && K == std::floor(K)))
+        return abo_fail(ABO_ERR_INVALID, "MES needs params[0] = K, an integer in [1, %d]", MES_MAX_K);
+    out->K = (int)K;
+    for (int k = 0; k < out->K; ++k) {
+        if (!std::isfinite(params[1 + k])) return abo_fail(ABO_ERR_INVALID, "MES y*[%d] is not finite", k);
+        out->ystar[k] = params[1 + k];
+    }
+    return ABO_OK;
+}
+
 // mean / var / scores for m device-resident candidates and candidate output bo; any of the
 // three outputs may be null (device pointers, length m)
 int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const double* params, double* d_mean,
                  double* d_var, double* d_score) {
     abo_ctx* c = g->ctx;
     cudaStream_t st = c->stream;
+    MesSpec mes;                                                     // by value in the kernel parameters: no upload
+    if (acq == ACQ_MES) { const int rc = mes_spec(params, &mes); if (rc) return rc; }
+    const MesSpec* mesp = acq == ACQ_MES ? &mes : nullptr;
     {
         AcqSpec a0;
         a0.acq = acq;
@@ -1040,7 +1061,7 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
         a0.p1 = (params && acq != ACQ_UCB && acq >= 0) ? params[1] : 0.0;
         a0.mean_c = g->mean_c[bo];
         a0.kss = g->scale;
-        if (fused_applies(g, bo)) return sweep_fused_device(g, dXc, m, a0, d_mean, d_var, d_score);
+        if (fused_applies(g, bo)) return sweep_fused_device(g, dXc, m, a0, mesp, d_mean, d_var, d_score);
     }
     const int64_t Npad = g->Npad;
     const int T = (int)(Npad / NB);
@@ -1082,9 +1103,14 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
         if ((rc = launch_gemm_tma<EPI_COLSUMSQ>(c, tmA, tmB, sp, st))) return rc;
         if ((rc = prof_mark(c))) return rc;
         if ((rc = prof_mark(c))) return rc;
-        acq_epilogue_kernel<<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
-            a, pmean, npb, sumsq, T, mc, mvalid, d_mean ? d_mean + c0 : nullptr, d_var ? d_var + c0 : nullptr,
-            d_score ? d_score + c0 : nullptr);
+        if (mesp)
+            mes_epilogue_kernel<<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
+                a, *mesp, pmean, npb, sumsq, T, mc, mvalid, d_mean ? d_mean + c0 : nullptr, d_var ? d_var + c0 : nullptr,
+                d_score ? d_score + c0 : nullptr);
+        else
+            acq_epilogue_kernel<<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
+                a, pmean, npb, sumsq, T, mc, mvalid, d_mean ? d_mean + c0 : nullptr, d_var ? d_var + c0 : nullptr,
+                d_score ? d_score + c0 : nullptr);
         KL(c);
         if ((rc = prof_mark(c))) return rc;
         if (c->profile && c->prof_used >= 6 * 512) {       // bound the event pool
@@ -1145,7 +1171,9 @@ extern "C" int32_t abo_acq_eval_grad(abo_gp* g, int32_t acq_id, const double* pa
                                      double* scores, double* grad, double* mean, double* var) {
     if (!g || !Xc || !params || !scores || !grad) return abo_fail(ABO_ERR_INVALID, "null argument");
     if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
-    if (acq_id < 0 || acq_id > 2) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
+    if ((acq_id < 0 || acq_id > 2) && acq_id != ACQ_MES) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
+    MesSpec mes;
+    if (acq_id == ACQ_MES) { const int rc = mes_spec(params, &mes); if (rc) return rc; }
     if (g->d > AG_MAXD) return abo_fail(ABO_ERR_INVALID, "abo_acq_eval_grad supports d <= %d", AG_MAXD);
     if (m <= 0) return ABO_OK;
     abo_ctx* c = g->ctx;
@@ -1191,8 +1219,13 @@ extern "C" int32_t abo_acq_eval_grad(abo_gp* g, int32_t acq_id, const double* pa
         acq_grad_partial_kernel<<<dim3(npbg, (unsigned)mpad), 128, 0, st>>>(gp_spec(g), g->dXsT, g->ldx, g->n, g->dAlpha, Z,
                                                                            mpad, dXc + c0 * d, mvalid, part);
         KL(c);
-        acq_grad_finish_kernel<<<(unsigned)((mvalid + 127) / 128), 128, 0, st>>>(a, d, pmean, npb, colsq, part, npbg, mc, mpad,
-                                                                                 mvalid, dS + c0, dG + c0 * d, dM + c0, dV + c0);
+        if (acq_id == ACQ_MES)
+            mes_grad_finish_kernel<<<(unsigned)((mvalid + 127) / 128), 128, 0, st>>>(a, mes, d, pmean, npb, colsq, part, npbg, mc,
+                                                                                     mpad, mvalid, dS + c0, dG + c0 * d, dM + c0,
+                                                                                     dV + c0);
+        else
+            acq_grad_finish_kernel<<<(unsigned)((mvalid + 127) / 128), 128, 0, st>>>(a, d, pmean, npb, colsq, part, npbg, mc, mpad,
+                                                                                     mvalid, dS + c0, dG + c0 * d, dM + c0, dV + c0);
         KL(c);
     }
     CU(cudaMemcpyAsync(scores, dS, sizeof(double) * m, cudaMemcpyDeviceToHost, st));
@@ -1648,7 +1681,12 @@ static int acq_check(abo_gp* g, int acq_id, const double* params, const void* Xc
                      int64_t* top_idx, double* top_val) {
     if (!g || !Xc || !params) return abo_fail(ABO_ERR_INVALID, "null argument");
     if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
-    if (acq_id < 0 || acq_id > 2) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
+    if ((acq_id < 0 || acq_id > 2) && acq_id != ACQ_MES) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
+    if (acq_id == ACQ_MES) {
+        MesSpec mes;
+        const int rc = mes_spec(params, &mes);
+        if (rc) return rc;
+    }
     if (m < 0 || k < 0) return abo_fail(ABO_ERR_INVALID, "negative size");
     if (k > 0 && (!top_idx || !top_val)) return abo_fail(ABO_ERR_INVALID, "top-k buffers are NULL");
     return ABO_OK;

@@ -12,6 +12,7 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 #include <math_constants.h>
+#include <type_traits>
 
 #include "gemm_dmma.cuh"
 
@@ -21,7 +22,7 @@ constexpr int NB = 128;                 // tile / panel width everywhere
 constexpr double JITTER = 1e-18;        // AbstractGPs default_σ² (StandardGP.jl:361-379 via FiniteGP)
 
 enum KernelId { K_SE = 0, K_M52 = 1, K_M72 = 2, K_AM52 = 3, K_AM72 = 4, K_ADM52 = 5, K_ADM72 = 6 };
-enum AcqId { ACQ_EI = 0, ACQ_PI = 1, ACQ_UCB = 2 };
+enum AcqId { ACQ_EI = 0, ACQ_PI = 1, ACQ_UCB = 2, ACQ_MES = 4 };
 
 constexpr int ARD_MAXD = 32;
 struct KSpec {
@@ -742,6 +743,83 @@ __device__ __forceinline__ double acq_value(const AcqSpec& a, double mu, double 
     return normcdf_ref(z);
 }
 
+// ------------------------------------------------------------------------------------------
+// max-value entropy search (Wang & Jegelka, ICML 2017), minimising: for K sampled minimum values y*_k,
+//   MES = (1/K) sum_k h(gamma_k),  gamma_k = (mu - y*_k) / sigma,  h(g) = g r(g) / 2 - log Phi(g),  r = phi / Phi,
+// 0 where var <= 1e-12 (the threshold of acq_value).  The y* travel by value in the kernel parameters (2 KB): every
+// thread walks k in the same order, so the reads are constant-bank broadcasts.
+// h is formed with erfc / erfcx so that nothing overflows or cancels early; in the left tail (gamma <= -4) the leading
+// g^2 / 2 terms of g r / 2 and -log Phi still cancel, the error grows like eps g^2 (1e-13 relative at |g| = 40).
+// h' = -(r / 2)(1 + g (g + r)) cancels twice in that tail, so there it comes from the Mills ratio R(u) = Phi(-u) / phi(u),
+// u = -g, and its continued fraction rho_k = k / (u + rho_{k+1}) (Laplace): R = 1 / (u + rho_1) and
+// (1 + u^2) R - u = R rho_1 rho_2, so h' = -rho_1 rho_2 (u + rho_1) / 2.  32 levels reach 1e-13 at u >= 4.
+// ------------------------------------------------------------------------------------------
+constexpr int MES_MAX_K = 256;
+constexpr double MES_TAIL = -4.0;
+constexpr int MES_CF_DEPTH = 32;
+struct MesSpec {
+    int K;
+    double ystar[MES_MAX_K];
+};
+struct NoMes {};
+template <bool MES> using MesArg = typename std::conditional<MES, MesSpec, NoMes>::type;
+
+__device__ __forceinline__ double mes_h(double g) {
+    if (g >= 0.0) {
+        const double e = erfc(g * 0.70710678118654752440);                 // 2 (1 - Phi)
+        const double r = normpdf_ref(g) / (1.0 - e / 2);
+        return g * r / 2 - log1p(-e / 2);
+    }
+    const double t = -g * 0.70710678118654752440;
+    const double ex = erfcx(t);                                             // Phi(g) = ex e^{-t^2} / 2
+    const double r = 0.79788456080286535588 / ex;                           // sqrt(2 / pi) / erfcx(t)
+    return g * r / 2 - (log(ex / 2) - t * t);
+}
+
+__device__ __forceinline__ double mes_hprime(double g) {
+    if (g > MES_TAIL) {
+        double r;
+        if (g >= 0.0) r = normpdf_ref(g) / (1.0 - erfc(g * 0.70710678118654752440) / 2);
+        else r = 0.79788456080286535588 / erfcx(-g * 0.70710678118654752440);
+        return -(r / 2) * (1.0 + g * (g + r));
+    }
+    const double u = -g;
+    double rho = 0.0, rho2 = 0.0;
+#pragma unroll 1
+    for (int k = MES_CF_DEPTH; k >= 1; --k) {
+        rho = k / (u + rho);
+        if (k == 2) rho2 = rho;
+    }
+    return -(rho * rho2) * (u + rho) / 2;
+}
+
+// a called function, not inlined: inlined into sweep_fused_kernel<32, true> it costs 176 more spill bytes in the hot loops
+__device__ __noinline__ double mes_value(const MesSpec& s, double mu, double var) {
+    if (var <= 1e-12) return 0.0;
+    const double sig = sqrt(var);
+    double acc = 0.0;
+    for (int k = 0; k < s.K; ++k) acc += mes_h((mu - s.ystar[k]) / sig);
+    return acc / s.K;
+}
+
+// d MES / d mu = (1/K) sum h'(g_k) / sigma,  d MES / d var = -(1/K) sum h'(g_k) g_k / (2 var)
+__device__ __forceinline__ double mes_value_grad(const MesSpec& s, double mu, double var, double& dmu, double& dvar) {
+    dmu = 0.0; dvar = 0.0;
+    if (var <= 1e-12) return 0.0;
+    const double sig = sqrt(var);
+    double acc = 0.0, sd = 0.0, sdg = 0.0;
+    for (int k = 0; k < s.K; ++k) {
+        const double g = (mu - s.ystar[k]) / sig;
+        const double hp = mes_hprime(g);
+        acc += mes_h(g);
+        sd += hp;
+        sdg += hp * g;
+    }
+    dmu = (sd / s.K) / sig;
+    dvar = -(sdg / s.K) / (2 * var);
+    return acc / s.K;
+}
+
 __global__ void acq_epilogue_kernel(AcqSpec a, const double* __restrict__ pmean, int npb,
                                     const double* __restrict__ sumsq, int ntile, int64_t mc, int64_t mvalid,
                                     double* __restrict__ mean_out, double* __restrict__ var_out,
@@ -757,6 +835,24 @@ __global__ void acq_epilogue_kernel(AcqSpec a, const double* __restrict__ pmean,
     if (mean_out) mean_out[c] = mu;
     if (var_out) var_out[c] = var;
     if (score_out && a.acq >= 0) score_out[c] = acq_value(a, mu, var);
+}
+
+// the same for MES: acq_epilogue_kernel's mean / variance, then mes_value
+__global__ void mes_epilogue_kernel(AcqSpec a, const __grid_constant__ MesSpec mes, const double* __restrict__ pmean, int npb,
+                                    const double* __restrict__ sumsq, int ntile, int64_t mc, int64_t mvalid,
+                                    double* __restrict__ mean_out, double* __restrict__ var_out,
+                                    double* __restrict__ score_out) {
+    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (c >= mvalid) return;
+    double mu = 0.0;
+    for (int b = 0; b < npb; ++b) mu += pmean[(int64_t)b * mc + c];
+    mu += a.mean_c;
+    double q = 0.0;
+    for (int t = 0; t < ntile; ++t) q += sumsq[(int64_t)t * mc + c];
+    const double var = (a.kss - q) + JITTER;
+    if (mean_out) mean_out[c] = mu;
+    if (var_out) var_out[c] = var;
+    if (score_out) score_out[c] = mes_value(mes, mu, var);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1568,6 +1664,32 @@ __global__ void acq_grad_finish_kernel(AcqSpec a, int d, const double* __restric
             else { dmu = -normpdf_ref(z) / sig; dvar = -normpdf_ref(z) * z * 0.5 / var; }
         }
     }
+    for (int b = 0; b < d; ++b) {
+        double gm = 0.0, gv = 0.0;
+        for (int pb = 0; pb < npb; ++pb) {
+            gm += part[(((int64_t)pb * mpad + c) * 2 + 0) * AG_MAXD + b];
+            gv += part[(((int64_t)pb * mpad + c) * 2 + 1) * AG_MAXD + b];
+        }
+        grad[c * d + b] = dmu * gm + dvar * (-2.0 * gv);
+    }
+}
+
+// the same for MES (d MES / d mu, d MES / d var from mes_value_grad)
+__global__ void mes_grad_finish_kernel(AcqSpec a, const __grid_constant__ MesSpec mes, int d, const double* __restrict__ pmean,
+                                       int npb_mean, const double* __restrict__ colsq, const double* __restrict__ part, int npb,
+                                       int64_t mc, int64_t mpad, int64_t m, double* __restrict__ score,
+                                       double* __restrict__ grad, double* __restrict__ mean_out,
+                                       double* __restrict__ var_out) {
+    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (c >= m) return;
+    double mu = 0.0;
+    for (int b = 0; b < npb_mean; ++b) mu += pmean[(int64_t)b * mc + c];
+    mu += a.mean_c;
+    const double var = (a.kss - colsq[c]) + JITTER;
+    if (mean_out) mean_out[c] = mu;
+    if (var_out) var_out[c] = var;
+    double dmu, dvar;
+    score[c] = mes_value_grad(mes, mu, var, dmu, dvar);
     for (int b = 0; b < d; ++b) {
         double gm = 0.0, gv = 0.0;
         for (int pb = 0; pb < npb; ++pb) {

@@ -1,6 +1,6 @@
 // sweep_fused.cuh — ONE kernel for the whole candidate sweep of a scalar GP (p = 1):
 //     K(X*, X) tile  ->  W = L^-1 K*^T on the FP64 tensor pipe  ->  sum_i W_ic^2 (variance) and sum_i W_ic beta_i
-//     (mean: k*^T alpha = (L^-1 k*)^T (L^-1 delta))  ->  EI / PI / UCB  ->  scores
+//     (mean: k*^T alpha = (L^-1 k*)^T (L^-1 delta))  ->  EI / PI / UCB or MES  ->  scores
 // replacing the three launches per chunk of the large-n path (ks_build_kernel, gemm_tma_kernel<EPI_COLSUMSQ>,
 // acq_epilogue_kernel) and the HBM round trip of the K* chunk between them.
 // Reference call sites: acq(surrogate, grid) in optimize_acquisition (acq_utils.jl:44-52) ->
@@ -104,9 +104,12 @@ __device__ __forceinline__ double phi_value(int kind, double u) {
     return (kind == K_AM72 && u < 1e-10) ? 1.0 - (7.0 / 10.0) * u : v;
 }
 
-template <int DT>
+// MES = true: the candidate-tile epilogue evaluates max-value entropy search for the y* in `mes` (mes_value) instead of
+// acq_value; the EI / PI / UCB instantiations take an empty last parameter and are unchanged.
+template <int DT, bool MES = false>
 __global__ void __launch_bounds__(FS_THREADS, 1)
-sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const FusedParams p) {
+sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const FusedParams p,
+                   const __grid_constant__ MesArg<MES> mes) {
     extern __shared__ __align__(128) unsigned char fs_smem[];
     double* stage_base = reinterpret_cast<double*>(fs_smem);
     double* sc = reinterpret_cast<double*>(fs_smem + FS_STAGES * SW_STAGE_BYTES);        // [128][DT] scaled candidate coordinates
@@ -311,7 +314,11 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 const double var = (p.acq.kss - qacc[tid]) + JITTER;
                 if (p.mean_out) p.mean_out[gc] = mu;
                 if (p.var_out) p.var_out[gc] = var;
-                if (p.score_out && p.acq.acq >= 0) p.score_out[gc] = acq_value(p.acq, mu, var);
+                if constexpr (MES) {
+                    if (p.score_out) p.score_out[gc] = mes_value(mes, mu, var);
+                } else {
+                    if (p.score_out && p.acq.acq >= 0) p.score_out[gc] = acq_value(p.acq, mu, var);
+                }
             }
             qacc[tid] = 0.0; macc[tid] = 0.0;
         }

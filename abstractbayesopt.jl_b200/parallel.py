@@ -41,11 +41,17 @@ def sharded_topk(acq, surrogate, candidates, k: int, group=None):
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     lo, hi = shard_range(len(candidates), rank, world)
-    _, ti, tv = acq.topk(surrogate, candidates[lo:hi], k)
+    ctx = getattr(surrogate, "ctx", None)
+    shard_topk = getattr(acq, "shard_topk", None)
+    if shard_topk is not None:
+        # an acquisition whose parameters depend on the whole set (MaxValueEntropySearch: the sampled minimum values)
+        # exchanges what it needs through `gather` before it sweeps its shard
+        _, ti, tv = shard_topk(surrogate, candidates[lo:hi], k, lambda v: _allgather(v, world, group, ctx))
+    else:
+        _, ti, tv = acq.topk(surrogate, candidates[lo:hi], k)
     mine = (np.asarray(ti, dtype=np.int64) + lo, np.asarray(tv))
     if world == 1:
         return merge_topk([mine[0]], [mine[1]], k)
-    ctx = getattr(surrogate, "ctx", None)
     if _nccl_spans(ctx, world):
         # abo_topk_allgather: one NCCL all-gather of the (count, index, value) records + the same
         # (value desc, index asc, NaN first) merge inside the library
@@ -53,6 +59,20 @@ def sharded_topk(acq, surrogate, candidates, k: int, group=None):
     gathered = [None] * world
     dist.all_gather_object(gathered, mine, group=group)
     return merge_topk([g[0] for g in gathered], [g[1] for g in gathered], k)
+
+
+def _allgather(values, world: int, group=None, ctx=None):
+    """Every rank's equally long float64 array, in rank order: NCCL through `ctx` when it spans the job, else the
+    torch.distributed group."""
+    values = np.ascontiguousarray(values, dtype=np.float64)
+    if world == 1:
+        return [values]
+    if _nccl_spans(ctx, world):
+        return list(ctx.allgather_f64(values, world))
+    import torch.distributed as dist
+    gathered = [None] * world
+    dist.all_gather_object(gathered, values, group=group)
+    return [np.asarray(g, dtype=np.float64) for g in gathered]
 
 
 def _nccl_spans(ctx, world: int) -> bool:

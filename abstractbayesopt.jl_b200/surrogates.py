@@ -251,6 +251,24 @@ def pathwise_thompson_batch(model, x, q, *, seed, num_features=4096):
     return h.pathwise_sample(_as_points(x, h.d), q, seed, num_features, want_samples=False)[1]
 
 
+def max_value_samples(model, x, K, *, seed, num_features=4096, best_y=None):
+    """K sampled values of the minimum of f over the points x, for max-value entropy search: the minimum value of each of
+    K pathwise posterior draws (argmin_val of abo_gp_pathwise_sample; one call, only the argmins leave the device),
+    clamped at the incumbent best_y when given: y*_k = min(argmin_val_k, best_y), in draw order.  The first K' values
+    equal those of a call with K'."""
+    h = _need_posterior(model)
+    return _max_value_samples(h, _as_points(x, h.d), K, seed, num_features, best_y)
+
+
+def _max_value_samples(h, X, K, seed, num_features, best_y):
+    """max_value_samples on a posterior handle and an (m, d) array; an empty set has minimum +inf."""
+    if X.shape[0] == 0:
+        v = np.full(int(K), math.inf)
+    else:
+        v = h.pathwise_sample(X, int(K), seed, num_features, want_samples=False)[2]
+    return v if best_y is None else np.minimum(v, float(best_y))
+
+
 def unstandardized_mean_and_var(model, xs, params):
     """StandardGP.jl:395-404 / GradientGP.jl:1019-1030."""
     h = _need_posterior(model)

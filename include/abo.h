@@ -49,8 +49,26 @@ typedef enum {
 } abo_kernel;
 
 /* acquisition functions (src/acquisition_functions/{ExpectedImprovement,ProbabilityImprovement,
- * UpperConfidenceBound,gradNormUCB}.jl).  params: EI/PI = {xi, best_y}; UCB / GradientNormUCB = {beta}. */
-typedef enum { ABO_ACQ_EI = 0, ABO_ACQ_PI = 1, ABO_ACQ_UCB = 2, ABO_ACQ_GRADNORM_UCB = 3 /* abo_acq_eval_multi only */ } abo_acq;
+ * UpperConfidenceBound,gradNormUCB}.jl).  params: EI/PI = {xi, best_y}; UCB / GradientNormUCB = {beta}.
+ *
+ * ABO_ACQ_MES, max-value entropy search (Wang & Jegelka, ICML 2017; BoTorch qMaxValueEntropy), for a minimiser:
+ * params = {K, y*_1, ..., y*_K}, K sampled values of the global minimum f*.  K must be an integer-valued double with
+ * 1 <= K <= 256 and every y* finite, otherwise ABO_ERR_INVALID.  With the posterior mean mu and variance var of the value
+ * output (var includes the 1e-18 of abo_gp_posterior):
+ *     MES = 0                                   if var <= 1e-12 (no information where nothing is uncertain; the
+ *                                               threshold EI / PI use),
+ *     MES = (1/K) sum_{k=1..K} h(gamma_k)        otherwise, gamma_k = (mu - y*_k) / sqrt(var),
+ *     h(g) = g r(g) / 2 - log Phi(g),  r = phi / Phi,   h >= 0, h -> 0 as g -> +inf,
+ * the sum taken in ascending k and then divided by K.  h and its derivative h' = -(r/2)(1 + g (g + r)) are accurate to
+ * 1e-12 relative for g in [-40, 40] (erfc / erfcx forms; a continued fraction of the Mills ratio for h' at g <= -4);
+ * beyond |g| = 40 the error of h grows like eps g^2 and only finite, non-negative values are promised.
+ * MES is in the model's units, those of abo_gp_posterior's mean and of the pathwise draws.  It applies to StandardGP
+ * (isotropic or ARD) and to the value output of a GradientGP, through abo_acq_eval, abo_acq_eval_dev and
+ * abo_acq_eval_grad (d MES / d mu = (1/K) sum h'(gamma_k) / sigma, d MES / d var = -(1/K) sum h'(gamma_k) gamma_k / (2 var));
+ * abo_acq_eval_multi does not take it.  The caller supplies y*; the intended source is argmin_val of
+ * abo_gp_pathwise_sample(_dev) over the candidate set, clamped at the incumbent: y*_k = min(argmin_val_k, best_y). */
+typedef enum { ABO_ACQ_EI = 0, ABO_ACQ_PI = 1, ABO_ACQ_UCB = 2, ABO_ACQ_GRADNORM_UCB = 3 /* abo_acq_eval_multi only */,
+               ABO_ACQ_MES = 4 /* not in abo_acq_eval_multi */ } abo_acq;
 
 int32_t abo_version(void);
 const char* abo_last_error(void);          /* thread-local message of the last failure */

@@ -419,6 +419,28 @@ function pathwise_sample(m::Union{CuStandardGP,CuGradientGP}, xs, S::Integer; se
     out
 end
 
+# K sampled minimum values for max-value entropy search: min(argmin_val_k, best_y) of K pathwise draws over xs, in draw
+# order (abo_gp_pathwise_sample with no samples buffer: only the argmins leave the device)
+function max_value_samples(m::Union{CuStandardGP,CuGradientGP}, xs, K::Integer; seed::Integer, num_features::Integer=4096,
+                           best_y::Real=Inf)
+    m.gpx === nothing && error("surrogate has no posterior: call update(model, xs, ys) first")
+    Xc = Matrix{Float64}(points(collect(xs))); mcount = size(Xc, 2)
+    ai = Vector{Int64}(undef, K); av = Vector{Float64}(undef, K)
+    check(GC.@preserve Xc ai av ccall((:abo_gp_pathwise_sample, LIB), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, UInt64, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}),
+        m.gpx.h, Xc, mcount, K, num_features, UInt64(seed), C_NULL, ai, av))
+    min.(av, Float64(best_y))
+end
+
+# max-value entropy search (ABO_ACQ_MES, include/abo.h) for the sampled minimum values `max_values` (1 to 256 of them,
+# e.g. from max_value_samples over the grid): evaluated in the fused sweep; acq_value_grad gives its analytic gradient
+struct MaxValueEntropy <: AbstractAcquisition
+    max_values::Vector{Float64}
+end
+acq_id(::MaxValueEntropy) = Int32(4); acq_params(a::MaxValueEntropy) = Float64[length(a.max_values); a.max_values]
+(a::MaxValueEntropy)(m::CuStandardGP, x::AbstractVector) = acq_eval(a, m, x)[1]
+(a::MaxValueEntropy)(m::CuGradientGP, x::AbstractVector) = acq_eval(a, m, x)[1]
+
 # monte_carlo_fill_distance (src/BO_utils.jl:140-159) on the device; the caller draws the uniform samples
 function fill_distance(X::Matrix{Float64}, S::Matrix{Float64})         # both d x count, column-major = point-major
     out = Ref{Float64}(0.0)
