@@ -11,8 +11,7 @@ import numpy as np
 from .surrogates import _as_points, _get_minimum, _max_value_samples, _need_posterior, pathwise_sample, posterior_sample
 from .parallel import merge_topk
 
-ACQ_EI, ACQ_PI, ACQ_UCB = 0, 1, 2
-ACQ_MES = 4
+ACQ_EI, ACQ_PI, ACQ_UCB, ACQ_GRADNORM_UCB, ACQ_MES = 0, 1, 2, 3, 4
 
 
 class AbstractAcquisition:
@@ -200,9 +199,6 @@ def nan_min_reduce(arrays):
     return out
 
 
-ACQ_GRADNORM_UCB = 3
-
-
 def _fd_value_and_grad(acq, surrogate, x, rel_step=6.0554544523933395e-06):
     """Value and central-difference gradient for a batch of points in ONE batched evaluation of m (2 d + 1) points
     (what Optim's finite-difference default does one point and one coordinate at a time, acq_utils.jl:55-63);
@@ -267,7 +263,8 @@ class EnsembleAcquisition(AbstractAcquisition):
     def update(self, ys, surrogate): return EnsembleAcquisition(self.weights, [a.update(ys, surrogate) for a in self.acquisitions])
 
     def _fusable(self):
-        return len(self.acquisitions) <= 8 and all(getattr(a, "acq_id", -1) in (0, 1, 2, 3) and not isinstance(a, EnsembleAcquisition)
+        return len(self.acquisitions) <= 8 and all(getattr(a, "acq_id", -1) in (ACQ_EI, ACQ_PI, ACQ_UCB, ACQ_GRADNORM_UCB)
+                                                   and not isinstance(a, EnsembleAcquisition)
                                                    for a in self.acquisitions)
 
     def _eval(self, surrogate, x, k=0, want_scores=True, grid=False):

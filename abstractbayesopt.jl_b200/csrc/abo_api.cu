@@ -992,12 +992,54 @@ static double phi_prime0(int kind) {
 static bool fused_applies(const abo_gp* g, int bo) {
     return g->p == 1 && bo == 0 && g->d <= 32 && g->Npad <= FS_MAX_NPAD;
 }
-static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const AcqSpec& a, const MesSpec* mes, double* d_mean,
-                              double* d_var, double* d_score) {
+
+// The acquisition of one sweep over a candidate output: its AcqSpec and, for ABO_ACQ_MES, the y*.  The MesSpec travels by
+// value in the kernel parameters: no upload.
+struct AcqSweep {
+    AcqSpec a;
+    MesSpec mes;                                                     // ABO_ACQ_MES only
+};
+
+// posterior mean / variance only (acq = -1) of candidate output bo: its prior mean and variance, -2 s_b^2 sigma^2 phi'(0) for
+// the derivative output b of a GradientGP
+static AcqSpec prior_spec(const abo_gp* g, int bo) {
+    const double sb = (bo > 0 && bo - 1 < (int)g->sv.size() && g->d <= ARD_MAXD) ? g->sv[bo - 1] : g->s;
+    return AcqSpec{-1, 0.0, 0.0, g->mean_c[bo], (bo == 0) ? g->scale : -2.0 * sb * sb * g->scale * phi_prime0(g->kind)};
+}
+
+// `a` with the acquisition acq_id: EI / PI params = {xi, best_y}, UCB {beta} (p1 = 0), MES {K, y*_1 .. y*_K} (the y* go to
+// the MesSpec), GradientNormUCB {beta, unused}
+static AcqSpec with_acq(AcqSpec a, int acq_id, const double* params) {
+    a.acq = acq_id;
+    a.p0 = params[0];
+    a.p1 = (acq_id != ACQ_UCB) ? params[1] : 0.0;
+    return a;
+}
+
+// (acq_id, params) of abo_acq_eval[_dev] / abo_acq_eval_grad, for candidate output bo.  ABO_ACQ_MES: K an integer-valued
+// double in [1, MES_MAX_K], every y* finite.
+static int acq_parse(const abo_gp* g, int acq_id, const double* params, int bo, AcqSweep* s) {
+    if ((acq_id < ACQ_EI || acq_id > ACQ_UCB) && acq_id != ACQ_MES) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
+    if (acq_id == ACQ_MES) {
+        const double K = params[0];
+        if (!(K >= 1.0 && K <= (double)MES_MAX_K && K == std::floor(K)))
+            return abo_fail(ABO_ERR_INVALID, "MES needs params[0] = K, an integer in [1, %d]", MES_MAX_K);
+        s->mes.K = (int)K;
+        for (int k = 0; k < s->mes.K; ++k) {
+            if (!std::isfinite(params[1 + k])) return abo_fail(ABO_ERR_INVALID, "MES y*[%d] is not finite", k);
+            s->mes.ystar[k] = params[1 + k];
+        }
+    }
+    s->a = with_acq(prior_spec(g, bo), acq_id, params);
+    return ABO_OK;
+}
+
+static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const AcqSweep& s, double* d_mean, double* d_var,
+                              double* d_score) {
     abo_ctx* c = g->ctx;
     cudaStream_t st = c->stream;
     FusedParams fp;
-    fp.spec = gp_spec(g); fp.acq = a;
+    fp.spec = gp_spec(g); fp.acq = s.a;
     fp.XsT = g->dXsT; fp.ldx = g->ldx; fp.n = g->n;
     fp.T = (int)((g->n + NB - 1) / NB);
     fp.Kld = (int)((g->n + 15) / 16 * 16);
@@ -1013,15 +1055,15 @@ static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const Acq
     if ((rc = make_tmap_k4(&tmB, fp.scratch, fp.Kld, (int64_t)c->sms * 2 * NB, fp.Kld))) return rc;
     if ((rc = prof_mark(c)) || (rc = prof_mark(c))) return rc;            // class 0 (K* builder): inside the fused kernel
     if ((rc = prof_mark(c))) return rc;
-#define ABO_FS_RUN(DT)                                                                                           \
-    do {                                                                                                         \
-        if (mes) sweep_fused_kernel<DT, true><<<grid, FS_THREADS, fused_smem_bytes<DT>(), st>>>(tmA, tmB, fp, *mes); \
-        else sweep_fused_kernel<DT><<<grid, FS_THREADS, fused_smem_bytes<DT>(), st>>>(tmA, tmB, fp, NoMes{});       \
-    } while (0)
-    const int d = g->d;
-    if (d <= 4) ABO_FS_RUN(4); else if (d <= 8) ABO_FS_RUN(8); else if (d <= 12) ABO_FS_RUN(12); else if (d <= 16) ABO_FS_RUN(16);
-    else if (d <= 20) ABO_FS_RUN(20); else if (d <= 24) ABO_FS_RUN(24); else ABO_FS_RUN(32);
+    const auto run = [&](auto mes) {
+        constexpr bool MES = std::is_same<decltype(mes), MesSpec>::value;
+#define ABO_FS_RUN(DT) sweep_fused_kernel<DT, MES><<<grid, FS_THREADS, fused_smem_bytes<DT>(), st>>>(tmA, tmB, fp, mes)
+        const int d = g->d;
+        if (d <= 4) ABO_FS_RUN(4); else if (d <= 8) ABO_FS_RUN(8); else if (d <= 12) ABO_FS_RUN(12); else if (d <= 16) ABO_FS_RUN(16);
+        else if (d <= 20) ABO_FS_RUN(20); else if (d <= 24) ABO_FS_RUN(24); else ABO_FS_RUN(32);
 #undef ABO_FS_RUN
+    };
+    if (s.a.acq == ACQ_MES) run(s.mes); else run(NoMes{});
     KL(c);
     if ((rc = prof_mark(c))) return rc;
     if ((rc = prof_mark(c)) || (rc = prof_mark(c))) return rc;            // class 2 (epilogue): inside the fused kernel
@@ -1032,37 +1074,13 @@ static int sweep_fused_device(abo_gp* g, const double* dXc, int64_t m, const Acq
     return ABO_OK;
 }
 
-// ABO_ACQ_MES params = {K, y*_1 .. y*_K}: K an integer-valued double in [1, MES_MAX_K], every y* finite
-static int mes_spec(const double* params, MesSpec* out) {
-    const double K = params[0];
-    if (!(K >= 1.0 && K <= (double)MES_MAX_K && K == std::floor(K)))
-        return abo_fail(ABO_ERR_INVALID, "MES needs params[0] = K, an integer in [1, %d]", MES_MAX_K);
-    out->K = (int)K;
-    for (int k = 0; k < out->K; ++k) {
-        if (!std::isfinite(params[1 + k])) return abo_fail(ABO_ERR_INVALID, "MES y*[%d] is not finite", k);
-        out->ystar[k] = params[1 + k];
-    }
-    return ABO_OK;
-}
-
-// mean / var / scores for m device-resident candidates and candidate output bo; any of the
+// mean / var / scores for m device-resident candidates and candidate output bo, `s` the acquisition of output bo; any of the
 // three outputs may be null (device pointers, length m)
-int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const double* params, double* d_mean,
-                 double* d_var, double* d_score) {
+int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, const AcqSweep& s, double* d_mean, double* d_var,
+                 double* d_score) {
+    if (fused_applies(g, bo)) return sweep_fused_device(g, dXc, m, s, d_mean, d_var, d_score);
     abo_ctx* c = g->ctx;
     cudaStream_t st = c->stream;
-    MesSpec mes;                                                     // by value in the kernel parameters: no upload
-    if (acq == ACQ_MES) { const int rc = mes_spec(params, &mes); if (rc) return rc; }
-    const MesSpec* mesp = acq == ACQ_MES ? &mes : nullptr;
-    {
-        AcqSpec a0;
-        a0.acq = acq;
-        a0.p0 = params ? params[0] : 0.0;
-        a0.p1 = (params && acq != ACQ_UCB && acq >= 0) ? params[1] : 0.0;
-        a0.mean_c = g->mean_c[bo];
-        a0.kss = g->scale;
-        if (fused_applies(g, bo)) return sweep_fused_device(g, dXc, m, a0, mesp, d_mean, d_var, d_score);
-    }
     const int64_t Npad = g->Npad;
     const int T = (int)(Npad / NB);
     // chunk: enough tiles per launch (>= ~2048) that the persistent kernel's tail is small, K* buffer
@@ -1083,13 +1101,6 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
     CUtensorMap tmA, tmB;
     if ((rc = make_tmap_k4(&tmA, g->dLinv, Npad, Npad, g->ld))) return rc;
     if ((rc = make_tmap_k4(&tmB, Ks, Npad, mc, Npad))) return rc;
-    AcqSpec a;
-    a.acq = acq;
-    a.p0 = params ? params[0] : 0.0;
-    a.p1 = (params && acq != ACQ_UCB && acq >= 0) ? params[1] : 0.0;
-    a.mean_c = g->mean_c[bo];
-    const double sb_ = (bo > 0 && bo - 1 < (int)g->sv.size() && g->d <= ARD_MAXD) ? g->sv[bo - 1] : g->s;
-    a.kss = (bo == 0) ? g->scale : -2.0 * sb_ * sb_ * g->scale * phi_prime0(g->kind);
     for (int64_t c0 = 0; c0 < m; c0 += mc) {
         const int64_t mvalid = std::min(mc, m - c0);
         const int64_t mc_eff = (mvalid + NB - 1) / NB * NB;
@@ -1103,14 +1114,12 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
         if ((rc = launch_gemm_tma<EPI_COLSUMSQ>(c, tmA, tmB, sp, st))) return rc;
         if ((rc = prof_mark(c))) return rc;
         if ((rc = prof_mark(c))) return rc;
-        if (mesp)
-            mes_epilogue_kernel<<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
-                a, *mesp, pmean, npb, sumsq, T, mc, mvalid, d_mean ? d_mean + c0 : nullptr, d_var ? d_var + c0 : nullptr,
-                d_score ? d_score + c0 : nullptr);
-        else
-            acq_epilogue_kernel<<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
-                a, pmean, npb, sumsq, T, mc, mvalid, d_mean ? d_mean + c0 : nullptr, d_var ? d_var + c0 : nullptr,
-                d_score ? d_score + c0 : nullptr);
+        const auto epilogue = [&](auto mes) {
+            acq_epilogue_kernel<std::is_same<decltype(mes), MesSpec>::value><<<(unsigned)((mvalid + 255) / 256), 256, 0, st>>>(
+                s.a, pmean, npb, sumsq, T, mc, mvalid, d_mean ? d_mean + c0 : nullptr, d_var ? d_var + c0 : nullptr,
+                d_score ? d_score + c0 : nullptr, mes);
+        };
+        if (s.a.acq == ACQ_MES) epilogue(s.mes); else epilogue(NoMes{});
         KL(c);
         if ((rc = prof_mark(c))) return rc;
         if (c->profile && c->prof_used >= 6 * 512) {       // bound the event pool
@@ -1124,8 +1133,8 @@ int sweep_device(abo_gp* g, const double* dXc, int64_t m, int bo, int acq, const
 
 // host candidates per piece of sweep_host_pieces
 constexpr int64_t HOST_PIECE = 262144;
-static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
-                             double* h_var, double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
+static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, const AcqSweep& s, double* h_mean, double* h_var,
+                             double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
 
 extern "C" int32_t abo_gp_posterior(abo_gp* g, const double* Xc, int64_t m, int32_t outputs, double* mean, double* var) {
     if (!g || !Xc) return abo_fail(ABO_ERR_INVALID, "null argument");
@@ -1135,7 +1144,7 @@ extern "C" int32_t abo_gp_posterior(abo_gp* g, const double* Xc, int64_t m, int3
     abo_ctx* c = g->ctx;
     CU(cudaSetDevice(c->device));
     if (outputs == 1 && m > HOST_PIECE && !c->profile)
-        return sweep_host_pieces(g, Xc, m, -1, nullptr, mean, var, nullptr, 0, nullptr, nullptr);
+        return sweep_host_pieces(g, Xc, m, AcqSweep{prior_spec(g, 0)}, mean, var, nullptr, 0, nullptr, nullptr);
     cudaStream_t st = c->stream;
     double *dXc, *dm, *dv;
     int rc;
@@ -1144,7 +1153,8 @@ extern "C" int32_t abo_gp_posterior(abo_gp* g, const double* Xc, int64_t m, int3
     if ((rc = ws_get(c, WS_OUT_B, sizeof(double) * (size_t)m * outputs, (void**)&dv))) return rc;
     CU(cudaMemcpyAsync(dXc, Xc, sizeof(double) * m * g->d, cudaMemcpyHostToDevice, st));
     for (int bo = 0; bo < outputs; ++bo)
-        if ((rc = sweep_device(g, dXc, m, bo, -1, nullptr, dm + (int64_t)bo * m, dv + (int64_t)bo * m, nullptr))) return rc;
+        if ((rc = sweep_device(g, dXc, m, bo, AcqSweep{prior_spec(g, bo)}, dm + (int64_t)bo * m, dv + (int64_t)bo * m, nullptr)))
+            return rc;
     if (mean) CU(cudaMemcpyAsync(mean, dm, sizeof(double) * m * outputs, cudaMemcpyDeviceToHost, st));
     if (var) CU(cudaMemcpyAsync(var, dv, sizeof(double) * m * outputs, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -1171,9 +1181,8 @@ extern "C" int32_t abo_acq_eval_grad(abo_gp* g, int32_t acq_id, const double* pa
                                      double* scores, double* grad, double* mean, double* var) {
     if (!g || !Xc || !params || !scores || !grad) return abo_fail(ABO_ERR_INVALID, "null argument");
     if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
-    if ((acq_id < 0 || acq_id > 2) && acq_id != ACQ_MES) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
-    MesSpec mes;
-    if (acq_id == ACQ_MES) { const int rc = mes_spec(params, &mes); if (rc) return rc; }
+    AcqSweep s;
+    if (const int rc = acq_parse(g, acq_id, params, 0, &s)) return rc;
     if (g->d > AG_MAXD) return abo_fail(ABO_ERR_INVALID, "abo_acq_eval_grad supports d <= %d", AG_MAXD);
     if (m <= 0) return ABO_OK;
     abo_ctx* c = g->ctx;
@@ -1197,12 +1206,6 @@ extern "C" int32_t abo_acq_eval_grad(abo_gp* g, int32_t acq_id, const double* pa
     if ((rc = ws_get(c, WS_GRAD_OUT, sizeof(double) * (size_t)(mc + 3 * m + m * d), (void**)&out))) return rc;
     double *colsq = out, *dS = out + mc, *dM = dS + m, *dV = dM + m, *dG = dV + m;
     CU(cudaMemcpyAsync(dXc, Xc, sizeof(double) * m * d, cudaMemcpyHostToDevice, st));
-    AcqSpec a;
-    a.acq = acq_id;
-    a.p0 = params[0];
-    a.p1 = (acq_id != ACQ_UCB) ? params[1] : 0.0;
-    a.mean_c = g->mean_c[0];
-    a.kss = g->scale;
     for (int64_t c0 = 0; c0 < m; c0 += mc) {
         const int64_t mvalid = std::min(mc, m - c0);
         const int64_t mpad = (mvalid + NB - 1) / NB * NB;
@@ -1219,13 +1222,11 @@ extern "C" int32_t abo_acq_eval_grad(abo_gp* g, int32_t acq_id, const double* pa
         acq_grad_partial_kernel<<<dim3(npbg, (unsigned)mpad), 128, 0, st>>>(gp_spec(g), g->dXsT, g->ldx, g->n, g->dAlpha, Z,
                                                                            mpad, dXc + c0 * d, mvalid, part);
         KL(c);
-        if (acq_id == ACQ_MES)
-            mes_grad_finish_kernel<<<(unsigned)((mvalid + 127) / 128), 128, 0, st>>>(a, mes, d, pmean, npb, colsq, part, npbg, mc,
-                                                                                     mpad, mvalid, dS + c0, dG + c0 * d, dM + c0,
-                                                                                     dV + c0);
-        else
-            acq_grad_finish_kernel<<<(unsigned)((mvalid + 127) / 128), 128, 0, st>>>(a, d, pmean, npb, colsq, part, npbg, mc, mpad,
-                                                                                     mvalid, dS + c0, dG + c0 * d, dM + c0, dV + c0);
+        const auto finish = [&](auto mes) {
+            acq_grad_finish_kernel<std::is_same<decltype(mes), MesSpec>::value><<<(unsigned)((mvalid + 127) / 128), 128, 0, st>>>(
+                s.a, d, pmean, npb, colsq, part, npbg, mc, mpad, mvalid, dS + c0, dG + c0 * d, dM + c0, dV + c0, mes);
+        };
+        if (s.a.acq == ACQ_MES) finish(s.mes); else finish(NoMes{});
         KL(c);
     }
     CU(cudaMemcpyAsync(scores, dS, sizeof(double) * m, cudaMemcpyDeviceToHost, st));
@@ -1347,9 +1348,9 @@ static int gp_posterior_sample_run(abo_gp* g, const double* Xc, int64_t m, int64
         if ((rc = launch_gemm_tma(c, tmW, tmW, q, st))) return rc;
     }
     {
-        AcqSpec a{};                                                                     // mu = m + sum of the partial means
-        a.acq = -1; a.mean_c = g->mean_c[0]; a.kss = g->scale;
-        acq_epilogue_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(a, pmean, npb, nullptr, 0, Mpad, m, mu, nullptr, nullptr);
+        // mu = m + sum of the partial means
+        acq_epilogue_kernel<false><<<(unsigned)((m + 255) / 256), 256, 0, st>>>(prior_spec(g, 0), pmean, npb, nullptr, 0, Mpad, m, mu,
+                                                                                nullptr, nullptr, NoMes{});
         KL(c);
     }
     philox_normal_kernel<<<(unsigned)((Spad * Mpad / 4 + 255) / 256), 256, 0, st>>>(seed, 0, 0, 1.0, S, m, Spad, Mpad, Mpad, Z);
@@ -1619,13 +1620,13 @@ static void topk_emit(std::vector<TopItem>& items, int64_t k, int64_t* top_idx, 
 }
 
 static int scores_select_readback(abo_ctx* c, const double* dS, int64_t m, double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
-static int acq_eval_common(abo_gp* g, int acq_id, const double* params, const double* dXc, int64_t m, double* d_scores,
-                           double* h_scores, int64_t k, int64_t* top_idx, double* top_val) {
+static int acq_eval_common(abo_gp* g, const AcqSweep& s, const double* dXc, int64_t m, double* d_scores, double* h_scores,
+                           int64_t k, int64_t* top_idx, double* top_val) {
     abo_ctx* c = g->ctx;
     int rc;
     double* dS = d_scores;
     if (!dS && (rc = ws_get(c, WS_OUT_A, sizeof(double) * (size_t)m, (void**)&dS))) return rc;
-    if ((rc = sweep_device(g, dXc, m, 0, acq_id, params, nullptr, nullptr, dS))) return rc;
+    if ((rc = sweep_device(g, dXc, m, 0, s, nullptr, nullptr, dS))) return rc;
     return scores_select_readback(c, dS, m, h_scores, k, top_idx, top_val);
 }
 // scores on the device -> (optionally) the host, and the stable top-k of them
@@ -1677,16 +1678,12 @@ static int scores_select_readback(abo_ctx* c, const double* dS, int64_t m, doubl
     return ABO_OK;
 }
 
-static int acq_check(abo_gp* g, int acq_id, const double* params, const void* Xc, int64_t m, int64_t k,
-                     int64_t* top_idx, double* top_val) {
+// the arguments every acquisition entry point takes; with `s`, (acq_id, params) parsed into it
+static int acq_check(abo_gp* g, const double* params, const void* Xc, int64_t m, int64_t k, int64_t* top_idx, double* top_val,
+                     int acq_id = -1, AcqSweep* s = nullptr) {
     if (!g || !Xc || !params) return abo_fail(ABO_ERR_INVALID, "null argument");
     if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
-    if ((acq_id < 0 || acq_id > 2) && acq_id != ACQ_MES) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_id);
-    if (acq_id == ACQ_MES) {
-        MesSpec mes;
-        const int rc = mes_spec(params, &mes);
-        if (rc) return rc;
-    }
+    if (s) { if (const int rc = acq_parse(g, acq_id, params, 0, s)) return rc; }
     if (m < 0 || k < 0) return abo_fail(ABO_ERR_INVALID, "negative size");
     if (k > 0 && (!top_idx || !top_val)) return abo_fail(ABO_ERR_INVALID, "top-k buffers are NULL");
     return ABO_OK;
@@ -1696,12 +1693,12 @@ static int acq_check(abo_gp* g, int acq_id, const double* params, const void* Xc
 // is being evaluated the host stages piece i+1 (H2D on the copy stream), then reads back the results of
 // piece i-1 (scores if asked for, and the K best of the piece, selected on the device).  Per-candidate results
 // do not depend on the piece size.
-// acq_id < 0: posterior mean / variance of output 0 (h_mean / h_var, each may be NULL).
-static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
-                                 double* h_var, double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
-static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
-                             double* h_var, double* h_scores, int64_t k, int64_t* top_idx, double* top_val) {
-    const int rc = sweep_host_pieces_run(g, Xc, m, acq_id, params, h_mean, h_var, h_scores, k, top_idx, top_val);
+// s.a.acq < 0: posterior mean / variance of output 0 (h_mean / h_var, each may be NULL).
+static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, const AcqSweep& s, double* h_mean, double* h_var,
+                                 double* h_scores, int64_t k, int64_t* top_idx, double* top_val);
+static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, const AcqSweep& s, double* h_mean, double* h_var,
+                             double* h_scores, int64_t k, int64_t* top_idx, double* top_val) {
+    const int rc = sweep_host_pieces_run(g, Xc, m, s, h_mean, h_var, h_scores, k, top_idx, top_val);
     if (rc) {
         // an error return must not leave copies or kernels in flight that target the caller's host buffers or the
         // workspace slots (the next call may re-allocate them): drain both streams, keep the first error message
@@ -1712,9 +1709,10 @@ static int sweep_host_pieces(abo_gp* g, const double* Xc, int64_t m, int acq_id,
     }
     return rc;
 }
-static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, int acq_id, const double* params, double* h_mean,
-                                 double* h_var, double* h_scores, int64_t k, int64_t* top_idx, double* top_val) {
+static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, const AcqSweep& s, double* h_mean, double* h_var,
+                                 double* h_scores, int64_t k, int64_t* top_idx, double* top_val) {
     abo_ctx* c = g->ctx;
+    const int acq_id = s.a.acq;
     cudaStream_t st = c->stream, sc = c->stream3;
     const int d = g->d;
     const int64_t piece = HOST_PIECE;
@@ -1747,8 +1745,8 @@ static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, int acq
     CU(cudaEventRecord(c->ev_h2d[0], sc));
     for (int64_t i = 0; i < np; ++i) {
         CU(cudaStreamWaitEvent(st, c->ev_h2d[i & 1], 0));
-        if (acq_id >= 0) rc = sweep_device(g, dXc + off(i) * d, cnt(i), 0, acq_id, params, nullptr, nullptr, dA + off(i));
-        else rc = sweep_device(g, dXc + off(i) * d, cnt(i), 0, -1, nullptr, dA + off(i), dB + off(i), nullptr);
+        if (acq_id >= 0) rc = sweep_device(g, dXc + off(i) * d, cnt(i), 0, s, nullptr, nullptr, dA + off(i));
+        else rc = sweep_device(g, dXc + off(i) * d, cnt(i), 0, s, dA + off(i), dB + off(i), nullptr);
         if (rc) return rc;
         if (Kp > 0 && (rc = device_topk_launch(c, slot[i & 1], dA + off(i), cnt(i), std::min(Kp, cnt(i)), st))) return rc;
         CU(cudaEventRecord(c->ev_pc[i & 1], st));
@@ -1766,25 +1764,27 @@ static int sweep_host_pieces_run(abo_gp* g, const double* Xc, int64_t m, int acq
 
 extern "C" int32_t abo_acq_eval(abo_gp* g, int32_t acq_id, const double* params, const double* Xc, int64_t m,
                                 double* scores, int64_t k, int64_t* top_idx, double* top_val) {
-    int rc = acq_check(g, acq_id, params, Xc, m, k, top_idx, top_val);
+    AcqSweep s;
+    int rc = acq_check(g, params, Xc, m, k, top_idx, top_val, acq_id, &s);
     if (rc) return rc;
     if (m == 0) return ABO_OK;
     abo_ctx* c = g->ctx;
     CU(cudaSetDevice(c->device));
-    if (m > HOST_PIECE && !c->profile) return sweep_host_pieces(g, Xc, m, acq_id, params, nullptr, nullptr, scores, k, top_idx, top_val);
+    if (m > HOST_PIECE && !c->profile) return sweep_host_pieces(g, Xc, m, s, nullptr, nullptr, scores, k, top_idx, top_val);
     double* dXc;
     if ((rc = ws_get(c, WS_CAND, sizeof(double) * (size_t)m * g->d, (void**)&dXc))) return rc;
     CU(cudaMemcpyAsync(dXc, Xc, sizeof(double) * m * g->d, cudaMemcpyHostToDevice, c->stream));
-    return acq_eval_common(g, acq_id, params, dXc, m, nullptr, scores, k, top_idx, top_val);
+    return acq_eval_common(g, s, dXc, m, nullptr, scores, k, top_idx, top_val);
 }
 
 extern "C" int32_t abo_acq_eval_dev(abo_gp* g, int32_t acq_id, const double* params, const double* d_Xc, int64_t m,
                                     double* d_scores, int64_t k, int64_t* top_idx, double* top_val) {
-    int rc = acq_check(g, acq_id, params, d_Xc, m, k, top_idx, top_val);
+    AcqSweep s;
+    int rc = acq_check(g, params, d_Xc, m, k, top_idx, top_val, acq_id, &s);
     if (rc) return rc;
     if (m == 0) return ABO_OK;
     CU(cudaSetDevice(g->ctx->device));
-    return acq_eval_common(g, acq_id, params, d_Xc, m, d_scores, nullptr, k, top_idx, top_val);
+    return acq_eval_common(g, s, d_Xc, m, d_scores, nullptr, k, top_idx, top_val);
 }
 
 extern "C" int32_t abo_fill_distance(abo_ctx* c, const double* X, int64_t n, int32_t d, const double* S, int64_t m,

@@ -4,18 +4,18 @@
 
 extern "C" int32_t abo_acq_eval_multi(abo_gp* g, int32_t nmem, const int32_t* acq_ids, const double* weights, const double* params,
                                       const double* Xc, int64_t m, double* scores, int64_t k, int64_t* top_idx, double* top_val) {
-    if (!g || !acq_ids || !weights || !params || !Xc) return abo_fail(ABO_ERR_INVALID, "null argument");
-    if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
+    if (!acq_ids || !weights) return abo_fail(ABO_ERR_INVALID, "null argument");
+    int rc = acq_check(g, params, Xc, m, k, top_idx, top_val);
+    if (rc) return rc;
     if (nmem < 1 || nmem > AM_MAXMEM) return abo_fail(ABO_ERR_INVALID, "1 <= members <= %d", AM_MAXMEM);
-    if (m < 0 || k < 0) return abo_fail(ABO_ERR_INVALID, "negative size");
-    if (k > 0 && (!top_idx || !top_val)) return abo_fail(ABO_ERR_INVALID, "top-k buffers are NULL");
     MultiSpec ms;
     ms.nmem = nmem;
     bool need_grad = false;
-    for (int q = 0; q < nmem; ++q) {
-        if (acq_ids[q] < 0 || acq_ids[q] > 3) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_ids[q]);
-        ms.acq[q] = acq_ids[q]; ms.w[q] = weights[q]; ms.p0[q] = params[2 * q]; ms.p1[q] = params[2 * q + 1];
-        need_grad |= acq_ids[q] == 3;
+    for (int q = 0; q < nmem; ++q) {            // ABO_ACQ_MES is not a member
+        if (acq_ids[q] < ACQ_EI || acq_ids[q] > ACQ_GRADNORM_UCB) return abo_fail(ABO_ERR_INVALID, "unknown acquisition id %d", acq_ids[q]);
+        ms.acq[q] = with_acq(AcqSpec{}, acq_ids[q], params + 2 * q);
+        ms.w[q] = weights[q];
+        need_grad |= acq_ids[q] == ACQ_GRADNORM_UCB;
     }
     if (need_grad && g->p < 2) return abo_fail(ABO_ERR_INVALID, "GradientNormUCB needs a GradientGP surrogate (p = d + 1)");
     if (g->p > AM_MAXP) return abo_fail(ABO_ERR_INVALID, "abo_acq_eval_multi supports p <= %d", AM_MAXP);
@@ -24,7 +24,6 @@ extern "C" int32_t abo_acq_eval_multi(abo_gp* g, int32_t nmem, const int32_t* ac
     CU(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     const int d = g->d;
-    int rc;
     double *dXc, *dS;
     if ((rc = ws_get(c, WS_CAND, sizeof(double) * (size_t)m * d, (void**)&dXc))) return rc;
     if ((rc = ws_get(c, WS_OUT_A, sizeof(double) * (size_t)m, (void**)&dS))) return rc;
@@ -34,7 +33,7 @@ extern "C" int32_t abo_acq_eval_multi(abo_gp* g, int32_t nmem, const int32_t* ac
         double *dM, *dV;
         if ((rc = ws_get(c, WS_OUT_B, sizeof(double) * (size_t)m * 2, (void**)&dM))) return rc;
         dV = dM + m;
-        if ((rc = sweep_device(g, dXc, m, 0, -1, nullptr, dM, dV, nullptr))) return rc;
+        if ((rc = sweep_device(g, dXc, m, 0, AcqSweep{prior_spec(g, 0)}, dM, dV, nullptr))) return rc;
         acq_multi_combine_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(ms, dM, dV, m, dS);
         KL(c);
         return scores_select_readback(c, dS, m, scores, k, top_idx, top_val);

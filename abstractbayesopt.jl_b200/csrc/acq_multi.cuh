@@ -18,8 +18,8 @@ constexpr int AM_MAXMEM = 8;      // ensemble members
 constexpr int AM_ROWS = 512;      // rows of W per partial block
 struct MultiSpec {
     int nmem;
-    int acq[AM_MAXMEM];           // 0 EI, 1 PI, 2 UCB, 3 GradientNormUCB
-    double w[AM_MAXMEM], p0[AM_MAXMEM], p1[AM_MAXMEM];
+    double w[AM_MAXMEM];
+    AcqSpec acq[AM_MAXMEM];       // EI, PI, UCB or GradientNormUCB (p0 = beta)
 };
 
 // part[chunk][pair][c] = sum_{i in chunk} W[i][b*mp + c] * W[i][b2*mp + c],  pair = b(b+1)/2 + b2, b2 <= b < nout
@@ -71,7 +71,7 @@ __global__ void __launch_bounds__(128) acq_multi_finish_kernel(KSpec spec, Multi
     };
     double total = 0.0;
     bool need_grad = false;
-    for (int q = 0; q < ms.nmem; ++q) need_grad |= ms.acq[q] == 3;
+    for (int q = 0; q < ms.nmem; ++q) need_grad |= ms.acq[q].acq == ACQ_GRADNORM_UCB;
     double gn_mu = 0.0, gn_var = 0.0;
     if (need_grad) {
         // mu_sq = m.m + tr S ;  var_sq = 4 m^T S m + 2 sum S_ij^2      (S symmetric: off-diagonals counted twice)
@@ -90,12 +90,8 @@ __global__ void __launch_bounds__(128) acq_multi_finish_kernel(KSpec spec, Multi
     const double var0 = sigma(0, 0);
     for (int q = 0; q < ms.nmem; ++q) {
         double v;
-        if (ms.acq[q] == 3) v = -gn_mu + ms.p0[q] * sqrt(fmax(gn_var, 1e-12));
-        else {
-            AcqSpec a;
-            a.acq = ms.acq[q]; a.p0 = ms.p0[q]; a.p1 = ms.p1[q]; a.mean_c = 0.0; a.kss = 0.0;
-            v = acq_value(a, mu[0], var0);
-        }
+        if (ms.acq[q].acq == ACQ_GRADNORM_UCB) v = -gn_mu + ms.acq[q].p0 * sqrt(fmax(gn_var, 1e-12));
+        else v = acq_value(ms.acq[q], mu[0], var0);
         total = fma(ms.w[q], v, total);
     }
     score[c] = total;
@@ -107,11 +103,7 @@ __global__ void acq_multi_combine_kernel(MultiSpec ms, const double* __restrict_
     const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (c >= m) return;
     double total = 0.0;
-    for (int q = 0; q < ms.nmem; ++q) {
-        AcqSpec a;
-        a.acq = ms.acq[q]; a.p0 = ms.p0[q]; a.p1 = ms.p1[q]; a.mean_c = 0.0; a.kss = 0.0;
-        total = fma(ms.w[q], acq_value(a, mean[c], var[c]), total);
-    }
+    for (int q = 0; q < ms.nmem; ++q) total = fma(ms.w[q], acq_value(ms.acq[q], mean[c], var[c]), total);
     score[c] = total;
 }
 

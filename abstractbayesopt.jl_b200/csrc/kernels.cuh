@@ -22,7 +22,7 @@ constexpr int NB = 128;                 // tile / panel width everywhere
 constexpr double JITTER = 1e-18;        // AbstractGPs default_σ² (StandardGP.jl:361-379 via FiniteGP)
 
 enum KernelId { K_SE = 0, K_M52 = 1, K_M72 = 2, K_AM52 = 3, K_AM72 = 4, K_ADM52 = 5, K_ADM72 = 6 };
-enum AcqId { ACQ_EI = 0, ACQ_PI = 1, ACQ_UCB = 2, ACQ_MES = 4 };
+enum AcqId { ACQ_EI = 0, ACQ_PI = 1, ACQ_UCB = 2, ACQ_GRADNORM_UCB = 3, ACQ_MES = 4 };
 
 constexpr int ARD_MAXD = 32;
 struct KSpec {
@@ -743,6 +743,24 @@ __device__ __forceinline__ double acq_value(const AcqSpec& a, double mu, double 
     return normcdf_ref(z);
 }
 
+// d acq_value / d mu, d acq_value / d var
+__device__ __forceinline__ void acq_value_grad(const AcqSpec& a, double mu, double var, double& dmu, double& dvar) {
+    if (a.acq == ACQ_UCB) {
+        dmu = -1.0;
+        dvar = (var > 0.0) ? a.p0 * 0.5 / sqrt(var) : 0.0;
+    } else {
+        const double delta = (a.p1 - a.p0) - mu;
+        if (var <= 1e-12) {
+            dmu = (delta > 0.0) ? -1.0 : 0.0;
+            dvar = 0.0;
+        } else {
+            const double sig = sqrt(var), z = delta / sig;
+            if (a.acq == ACQ_EI) { dmu = -normcdf_ref(z); dvar = normpdf_ref(z) * 0.5 / sig; }
+            else { dmu = -normpdf_ref(z) / sig; dvar = -normpdf_ref(z) * z * 0.5 / var; }
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // max-value entropy search (Wang & Jegelka, ICML 2017), minimising: for K sampled minimum values y*_k,
 //   MES = (1/K) sum_k h(gamma_k),  gamma_k = (mu - y*_k) / sigma,  h(g) = g r(g) / 2 - log Phi(g),  r = phi / Phi,
@@ -820,39 +838,56 @@ __device__ __forceinline__ double mes_value_grad(const MesSpec& s, double mu, do
     return acc / s.K;
 }
 
+// The acquisition of every sweep epilogue, chosen at compile time: MES = true scores max-value entropy search for the y*
+// in `mes`, MES = false the EI / PI / UCB of `a`, and no score at all when `a` is posterior only (acq < 0).
+template <bool MES>
+__device__ __forceinline__ void acq_score(const AcqSpec& a, const MesArg<MES>& mes, double mu, double var, double* score_out,
+                                          int64_t c) {
+    if constexpr (MES) {
+        if (score_out) score_out[c] = mes_value(mes, mu, var);
+    } else {
+        if (score_out && a.acq >= 0) score_out[c] = acq_value(a, mu, var);
+    }
+}
+
+// the same acquisition with its d / d mu and d / d var (a not posterior only)
+template <bool MES>
+__device__ __forceinline__ void acq_score_grad(const AcqSpec& a, const MesArg<MES>& mes, double mu, double var, double* score_out,
+                                               int64_t c, double& dmu, double& dvar) {
+    if constexpr (MES) {
+        score_out[c] = mes_value_grad(mes, mu, var, dmu, dvar);
+    } else {
+        score_out[c] = acq_value(a, mu, var);
+        acq_value_grad(a, mu, var, dmu, dvar);
+    }
+}
+
+// mean and variance of candidate c from the partial sums of the K* builder (pmean[b][c]) and of the contraction
+// (sumsq[t][c]), also stored to the nullable mean_out / var_out
+__device__ __forceinline__ void posterior_mean_var(const AcqSpec& a, const double* __restrict__ pmean, int npb,
+                                                   const double* __restrict__ sumsq, int ntile, int64_t mc, int64_t c,
+                                                   double* __restrict__ mean_out, double* __restrict__ var_out, double& mu,
+                                                   double& var) {
+    mu = 0.0;
+    for (int b = 0; b < npb; ++b) mu += pmean[(int64_t)b * mc + c];
+    mu += a.mean_c;
+    double q = 0.0;
+    for (int t = 0; t < ntile; ++t) q += sumsq[(int64_t)t * mc + c];
+    var = (a.kss - q) + JITTER;
+    if (mean_out) mean_out[c] = mu;
+    if (var_out) var_out[c] = var;
+}
+
+template <bool MES>
 __global__ void acq_epilogue_kernel(AcqSpec a, const double* __restrict__ pmean, int npb,
                                     const double* __restrict__ sumsq, int ntile, int64_t mc, int64_t mvalid,
                                     double* __restrict__ mean_out, double* __restrict__ var_out,
-                                    double* __restrict__ score_out) {
+                                    double* __restrict__ score_out, const __grid_constant__ MesArg<MES> mes) {
     const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (c >= mvalid) return;
-    double mu = 0.0;
-    for (int b = 0; b < npb; ++b) mu += pmean[(int64_t)b * mc + c];
-    mu += a.mean_c;
-    double q = 0.0;
-    for (int t = 0; t < ntile; ++t) q += sumsq[(int64_t)t * mc + c];
-    const double var = (a.kss - q) + JITTER;
-    if (mean_out) mean_out[c] = mu;
-    if (var_out) var_out[c] = var;
-    if (score_out && a.acq >= 0) score_out[c] = acq_value(a, mu, var);
-}
-
-// the same for MES: acq_epilogue_kernel's mean / variance, then mes_value
-__global__ void mes_epilogue_kernel(AcqSpec a, const __grid_constant__ MesSpec mes, const double* __restrict__ pmean, int npb,
-                                    const double* __restrict__ sumsq, int ntile, int64_t mc, int64_t mvalid,
-                                    double* __restrict__ mean_out, double* __restrict__ var_out,
-                                    double* __restrict__ score_out) {
-    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (c >= mvalid) return;
-    double mu = 0.0;
-    for (int b = 0; b < npb; ++b) mu += pmean[(int64_t)b * mc + c];
-    mu += a.mean_c;
-    double q = 0.0;
-    for (int t = 0; t < ntile; ++t) q += sumsq[(int64_t)t * mc + c];
-    const double var = (a.kss - q) + JITTER;
-    if (mean_out) mean_out[c] = mu;
-    if (var_out) var_out[c] = var;
-    if (score_out) score_out[c] = mes_value(mes, mu, var);
+    double mu, var;
+    posterior_mean_var(a, pmean, npb, sumsq, ntile, mc, c, mean_out, var_out, mu, var);
+    acq_score<MES>(a, mes, mu, var, score_out, c);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1633,63 +1668,18 @@ __global__ void __launch_bounds__(128) acq_grad_partial_kernel(KSpec spec, const
     }
 }
 
-// one thread per candidate: value and gradient of EI / PI / UCB from (mu, var, grad mu, grad var)
+// one thread per candidate: value and gradient of the acquisition from (mu, var, grad mu, grad var)
+template <bool MES>
 __global__ void acq_grad_finish_kernel(AcqSpec a, int d, const double* __restrict__ pmean, int npb_mean,
                                        const double* __restrict__ colsq, const double* __restrict__ part, int npb,
                                        int64_t mc, int64_t mpad, int64_t m, double* __restrict__ score,
                                        double* __restrict__ grad, double* __restrict__ mean_out,
-                                       double* __restrict__ var_out) {
+                                       double* __restrict__ var_out, const __grid_constant__ MesArg<MES> mes) {
     const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (c >= m) return;
-    double mu = 0.0;
-    for (int b = 0; b < npb_mean; ++b) mu += pmean[(int64_t)b * mc + c];
-    mu += a.mean_c;
-    const double var = (a.kss - colsq[c]) + JITTER;
-    if (mean_out) mean_out[c] = mu;
-    if (var_out) var_out[c] = var;
-    score[c] = acq_value(a, mu, var);
-    // d acq / d mu, d acq / d var
-    double dmu, dvar;
-    if (a.acq == ACQ_UCB) {
-        dmu = -1.0;
-        dvar = (var > 0.0) ? a.p0 * 0.5 / sqrt(var) : 0.0;
-    } else {
-        const double delta = (a.p1 - a.p0) - mu;
-        if (var <= 1e-12) {
-            dmu = (delta > 0.0) ? -1.0 : 0.0;
-            dvar = 0.0;
-        } else {
-            const double sig = sqrt(var), z = delta / sig;
-            if (a.acq == ACQ_EI) { dmu = -normcdf_ref(z); dvar = normpdf_ref(z) * 0.5 / sig; }
-            else { dmu = -normpdf_ref(z) / sig; dvar = -normpdf_ref(z) * z * 0.5 / var; }
-        }
-    }
-    for (int b = 0; b < d; ++b) {
-        double gm = 0.0, gv = 0.0;
-        for (int pb = 0; pb < npb; ++pb) {
-            gm += part[(((int64_t)pb * mpad + c) * 2 + 0) * AG_MAXD + b];
-            gv += part[(((int64_t)pb * mpad + c) * 2 + 1) * AG_MAXD + b];
-        }
-        grad[c * d + b] = dmu * gm + dvar * (-2.0 * gv);
-    }
-}
-
-// the same for MES (d MES / d mu, d MES / d var from mes_value_grad)
-__global__ void mes_grad_finish_kernel(AcqSpec a, const __grid_constant__ MesSpec mes, int d, const double* __restrict__ pmean,
-                                       int npb_mean, const double* __restrict__ colsq, const double* __restrict__ part, int npb,
-                                       int64_t mc, int64_t mpad, int64_t m, double* __restrict__ score,
-                                       double* __restrict__ grad, double* __restrict__ mean_out,
-                                       double* __restrict__ var_out) {
-    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (c >= m) return;
-    double mu = 0.0;
-    for (int b = 0; b < npb_mean; ++b) mu += pmean[(int64_t)b * mc + c];
-    mu += a.mean_c;
-    const double var = (a.kss - colsq[c]) + JITTER;
-    if (mean_out) mean_out[c] = mu;
-    if (var_out) var_out[c] = var;
-    double dmu, dvar;
-    score[c] = mes_value_grad(mes, mu, var, dmu, dvar);
+    double mu, var, dmu, dvar;
+    posterior_mean_var(a, pmean, npb_mean, colsq, 1, mc, c, mean_out, var_out, mu, var);
+    acq_score_grad<MES>(a, mes, mu, var, score, c, dmu, dvar);
     for (int b = 0; b < d; ++b) {
         double gm = 0.0, gv = 0.0;
         for (int pb = 0; pb < npb; ++pb) {

@@ -104,8 +104,8 @@ __device__ __forceinline__ double phi_value(int kind, double u) {
     return (kind == K_AM72 && u < 1e-10) ? 1.0 - (7.0 / 10.0) * u : v;
 }
 
-// MES = true: the candidate-tile epilogue evaluates max-value entropy search for the y* in `mes` (mes_value) instead of
-// acq_value; the EI / PI / UCB instantiations take an empty last parameter and are unchanged.
+// MES = true: the candidate-tile epilogue evaluates max-value entropy search for the y* in `mes` (acq_score); the EI / PI / UCB
+// instantiations take an empty last parameter.
 template <int DT, bool MES = false>
 __global__ void __launch_bounds__(FS_THREADS, 1)
 sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const FusedParams p,
@@ -314,11 +314,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 const double var = (p.acq.kss - qacc[tid]) + JITTER;
                 if (p.mean_out) p.mean_out[gc] = mu;
                 if (p.var_out) p.var_out[gc] = var;
-                if constexpr (MES) {
-                    if (p.score_out) p.score_out[gc] = mes_value(mes, mu, var);
-                } else {
-                    if (p.score_out && p.acq.acq >= 0) p.score_out[gc] = acq_value(p.acq, mu, var);
-                }
+                acq_score<MES>(p.acq, mes, mu, var, p.score_out, gc);
             }
             qacc[tid] = 0.0; macc[tid] = 0.0;
         }
