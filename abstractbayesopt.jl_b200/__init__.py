@@ -15,7 +15,7 @@ from .surrogates import (AbstractSurrogate, GradientGP, StandardGP, get_kernel_c
                          _update_model_parameters)
 from .acquisition import (AbstractAcquisition, EnsembleAcquisition, ExpectedImprovement, GradientNormUCB,
                           MaxValueEntropySearch, PathwiseThompsonSampling, ProbabilityImprovement, ThompsonSampling,
-                          UpperConfidenceBound)
+                          UpperConfidenceBound, qExpectedImprovement)
 from .domains import AbstractDomain, ContinuousDomain
 from .parallel import (init_nccl_context, merge_topk, shard_range, sharded_nlml_batch, sharded_restarts, sharded_topk,
                        sync_posterior)

@@ -21,7 +21,7 @@ SYMBOLS = [
     "abo_gp_clone", "abo_gp_n", "abo_gp_alpha", "abo_gp_factor", "abo_gp_posterior", "abo_gp_posterior_cov", "abo_acq_eval", "abo_acq_eval_dev", "abo_acq_eval_grad",
     "abo_nlml_batch", "abo_potrf_dev", "abo_fill_distance", "abo_nccl_unique_id", "abo_ctx_init_rank", "abo_gp_sync",
     "abo_topk_allgather", "abo_allgather_f64", "abo_ctx_ranks", "abo_ctx_trim", "abo_acq_eval_multi", "abo_standardize", "abo_gp_set_params_ard", "abo_nlml_batch_ard",
-    "abo_gp_posterior_sample", "abo_gp_pathwise_sample", "abo_gp_pathwise_sample_dev",
+    "abo_gp_posterior_sample", "abo_gp_pathwise_sample", "abo_gp_pathwise_sample_dev", "abo_acq_qei",
 ]
 
 
@@ -86,6 +86,7 @@ def lib():
             "abo_acq_eval_dev": [vp, i32, vp, vp, i64, vp, i64, vp, vp],
             "abo_acq_eval_multi": [vp, i32, vp, vp, vp, vp, i64, vp, i64, vp, vp],
             "abo_acq_eval_grad": [vp, i32, vp, vp, i64, vp, vp, vp, vp],
+            "abo_acq_qei": [vp, vp, i32, vp, i64, i64, u64, dbl, vp, vp, vp],
             "abo_nlml_batch": [vp, vp, vp, i64, vp, i64, vp, vp, vp],
             "abo_nlml_batch_ard": [vp, vp, vp, i64, vp, i64, vp, vp, vp],
             "abo_potrf_dev": [vp, vp, i64, i64, C.POINTER(i64)],
@@ -416,6 +417,22 @@ class GpHandle:
         scores = np.empty(m); grad = np.empty((m, self.d))
         check(lib().abo_acq_eval_grad(self._h, acq_id, ptr(params), ptr(Xc), m, ptr(scores), ptr(grad), None, None))
         return scores, grad
+
+    def acq_qei(self, params, q, Xb, S, seed, jitter=1e-10, want_grad=False):
+        """Monte-Carlo batch expected improvement of B batches of q points, Xb of shape (B, q, d), params = (xi, best_y):
+        (values (B,), d values / d Xb (B, q, d) or None, the jitter tau of each batch (B,))."""
+        q, S, seed = int(q), int(S), int(seed)
+        Xb = f64(Xb)
+        if Xb.ndim != 3 or Xb.shape[1] != q or Xb.shape[2] != self.d:
+            raise DimensionMismatch(f"batches must be B x {q} x {self.d}")
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2^64)")
+        B = Xb.shape[0]
+        params = f64(params)
+        values = np.empty(max(B, 1)); tau = np.empty(max(B, 1))
+        grad = np.empty((max(B, 1), q, self.d)) if want_grad else None
+        check(lib().abo_acq_qei(self._h, ptr(params), q, ptr(Xb), B, S, seed, float(jitter), ptr(values), ptr(grad), ptr(tau)))
+        return values[:B], (grad[:B] if want_grad else None), tau[:B]
 
     def acq_eval_dev(self, acq_id, params, d_xc: int, m: int, d_scores: int = 0, k=0):
         params = f64(params)

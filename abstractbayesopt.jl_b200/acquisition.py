@@ -191,6 +191,47 @@ class MaxValueEntropySearch(AbstractAcquisition):
         return MaxValueEntropySearch(self.seed + 1, _get_minimum(surrogate, ys), self.num_max_values, self.num_features)
 
 
+@dataclass(frozen=True)
+class qExpectedImprovement(AbstractAcquisition):
+    """Monte-Carlo batch expected improvement, qEI (Ginsbourger et al. 2010; BoTorch qExpectedImprovement), minimising:
+    the expected improvement of the best of q points evaluated together, (1/S) sum_s max((best_y - xi) - min_j f_{s,j}, 0)
+    over S joint posterior draws f_s of the batch (abo_acq_qei).  Batches of near-duplicates score no better than one of
+    their points, so a maximiser spreads its q points where each adds something.  The draws use the same num_samples base
+    normals for every batch (from `seed`), so the value is a smooth, deterministic function of the points with an exact
+    gradient.  optimize_acquisition proposes (q, d) batches for it and `optimize` evaluates q points per iteration;
+    `update` takes the new incumbent and advances the seed."""
+    xi: float
+    best_y: float
+    q: int
+    num_samples: int = 512
+    seed: int = 0
+
+    @staticmethod
+    def _batches(h, batches):
+        b = np.asarray(batches, dtype=np.float64)
+        return b[None] if b.ndim == 2 else b
+
+    def __call__(self, surrogate, batches):
+        """qEI of each batch of `batches`, shape (B, q, d) (or one (q, d) batch): B values."""
+        h = _need_posterior(surrogate)
+        return h.acq_qei([self.xi, self.best_y], self.q, self._batches(h, batches), self.num_samples, self.seed)[0]
+
+    def value_and_grad(self, surrogate, batches):
+        """qEI of each batch and its gradient with respect to every coordinate of its points: (B,), (B, q, d)."""
+        h = _need_posterior(surrogate)
+        v, g, _ = h.acq_qei([self.xi, self.best_y], self.q, self._batches(h, batches), self.num_samples, self.seed,
+                            want_grad=True)
+        return v, g
+
+    def topk(self, surrogate, x, k, want_scores=True):
+        raise TypeError("qExpectedImprovement scores batches of q points, not single points (see optimize_acquisition)")
+
+    def copy(self): return qExpectedImprovement(self.xi, self.best_y, self.q, self.num_samples, self.seed)
+
+    def update(self, ys, surrogate):
+        return qExpectedImprovement(self.xi, _get_minimum(surrogate, ys), self.q, self.num_samples, self.seed + 1)
+
+
 def nan_min_reduce(arrays):
     """Elementwise minimum of equally long arrays; a NaN in any of them gives NaN there (np.minimum)."""
     out = np.asarray(arrays[0], dtype=np.float64)

@@ -60,8 +60,11 @@ def optimize_acquisition(acqf, surrogate, domain, n_grid=10_000, n_local=100, rn
     them (refine=True): analytic for EI / PI / UCB (abo_acq_eval_grad), batched central differences —
     all starts x (2 d + 1) points in one device call — for GradientNormUCB and ensembles.  refine="scipy" keeps the reference's sequential,
     finite-difference scheme (SciPy L-BFGS-B); refine=False returns the best grid point, and so does an acquisition
-    without a gradient (ThompsonSampling), whatever `refine` says."""
+    without a gradient (ThompsonSampling), whatever `refine` says.
+    A batch acquisition (`acqf.q` > 1, qExpectedImprovement) gets a (q, d) batch instead: see _optimize_batch."""
     rng = np.random.default_rng() if rng is None else rng
+    if getattr(acqf, "q", 1) > 1:
+        return _optimize_batch(acqf, surrogate, domain, n_grid, n_local, rng, refine)
     grid = latin_hypercube(n_grid, domain.lower, domain.upper, rng)
     _, top_idx, top_val = acqf.topk(surrogate, grid, n_local, want_scores=False)
     starts = grid[top_idx]
@@ -84,6 +87,36 @@ def optimize_acquisition(acqf, surrogate, domain, n_grid=10_000, n_local=100, rn
     X, f, _, failed = lockstep_lbfgsb(fg, starts, domain.lower, domain.upper, g_tol=1e-5, f_abstol=2.2e-9, max_iter=50)
     f = np.where(failed | ~np.isfinite(f), np.inf, f)
     return np.array(X[int(np.argmin(f))])                 # first best on ties, like the `>` update of :67-70
+
+
+def _optimize_batch(acqf, surrogate, domain, n_grid, n_local, rng, refine):
+    """optimize_acquisition for an acquisition of q-point batches: the LHS grid, randomly permuted and cut into
+    n_grid // q raw batches, is scored in ONE value-only call; the n_local best finite batches start lock-step L-BFGS over
+    their q d coordinates inside the box, one value-and-gradient call per step; the best batch is returned as a (q, d)
+    array, the first on ties.  refine=False returns the best raw batch ("scipy" refines like True)."""
+    q, d = int(acqf.q), len(domain.lower)
+    nb = n_grid // q
+    if nb < 1:
+        raise ValueError(f"n_grid = {n_grid} holds no batch of q = {q} points")
+    grid = latin_hypercube(n_grid, domain.lower, domain.upper, rng)
+    raw = grid[rng.permutation(n_grid)[:nb * q]].reshape(nb, q, d)
+    vals = np.asarray(acqf(surrogate, raw), dtype=np.float64)
+    finite = np.flatnonzero(np.isfinite(vals))
+    if finite.size == 0:
+        return np.array(raw[0])
+    order = finite[np.argsort(-vals[finite], kind="stable")]
+    starts = raw[order[:n_local]]
+    if refine is False:
+        return np.array(starts[0])
+
+    def fg(X, idx):
+        val, grad = acqf.value_and_grad(surrogate, X[idx].reshape(len(idx), q, d))
+        return -val, -grad.reshape(len(idx), q * d)
+
+    X, f, _, failed = lockstep_lbfgsb(fg, starts.reshape(len(starts), q * d), np.tile(domain.lower, q),
+                                      np.tile(domain.upper, q), g_tol=1e-5, f_abstol=2.2e-9, max_iter=50)
+    f = np.where(failed | ~np.isfinite(f), np.inf, f)
+    return np.array(X[int(np.argmin(f))]).reshape(q, d)
 
 
 def lockstep_lbfgsb(fg, x0, lower, upper, g_tol=1e-6, f_abstol=2.2e-9, max_iter=100, history=6, max_ls=20):
@@ -309,9 +342,20 @@ def rescale_output(ys, params):
             for y in ys]
 
 
+def _observe(BO, x, mu, sd, rng):
+    """BO.func at x with the loop's observation noise, appended to ys_non_std; returns the standardised observation."""
+    y = np.asarray(BO.func(x), dtype=np.float64)
+    s0 = float(np.ravel(sd)[0])
+    y = y + math.sqrt(BO.noise) / s0 * rng.standard_normal(y.shape) if BO.noise > 0 else y
+    BO.ys_non_std.append(y)
+    return (y - mu) / s0 if isinstance(BO.model, GradientGP) else (y - mu) / sd
+
+
 def optimize(BO: BOStruct, standardize="mean_scale", hyper_params="all", num_restarts_HP=1, n_grid=10_000,
              n_local=100, rng=None, refine=True, ard=False):
-    """optimize(BO; standardize, hyper_params, num_restarts_HP) (bayesian_opt.jl:364-449)."""
+    """optimize(BO; standardize, hyper_params, num_restarts_HP) (bayesian_opt.jl:364-449).  With a batch acquisition
+    (`BO.acq.q` > 1, qExpectedImprovement) every iteration proposes q points, evaluates BO.func at each and appends them
+    one by one (update_bo, with its rollback); max_iter then counts batches and acq_list holds each batch's value."""
     if standardize not in ("mean_scale", "scale_only", "mean_only", None):
         raise ValueError("standardize must be one of mean_scale, scale_only, mean_only, None")
     if hyper_params not in ("all", "length_scale_only", None):
@@ -338,11 +382,15 @@ def optimize(BO: BOStruct, standardize="mean_scale", hyper_params="all", num_res
         x_cand = optimize_acquisition(BO.acq, BO.model, BO.domain, n_grid=n_grid, n_local=n_local, rng=rng,
                                       refine=refine)
         acq_list.append(float(BO.acq(BO.model, x_cand[None, :])[0]))
-        y = np.asarray(BO.func(x_cand), dtype=np.float64)
-        s0 = float(np.ravel(sd)[0])
-        y = y + math.sqrt(BO.noise) / s0 * rng.standard_normal(y.shape) if BO.noise > 0 else y
-        BO.ys_non_std.append(y)
-        y_std = (y - mu) / s0 if isinstance(BO.model, GradientGP) else (y - mu) / sd
+        if getattr(BO.acq, "q", 1) > 1:                  # a batch: its q points are evaluated and appended one by one
+            i += 1
+            for x in x_cand:
+                y_std = _observe(BO, x, mu, sd, rng)
+                BO = update_bo(BO, x, y_std, i)          # a failed append stops the loop, the points before it kept
+                if BO.flag:
+                    break
+            continue
+        y_std = _observe(BO, x_cand, mu, sd, rng)
         i += 1                                           # incremented BEFORE update(BO, ...) (bayesian_opt.jl:441-445):
         BO = update_bo(BO, x_cand, y_std, i)             # BO.iter = i + 1, so exactly max_iter passes run
     return BO, acq_list, (mu, sd)

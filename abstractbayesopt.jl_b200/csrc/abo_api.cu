@@ -20,6 +20,7 @@
 #include "sweep_fused.cuh"
 #include "gemm_tma.cuh"
 #include "sample.cuh"
+#include "qei.cuh"
 #include "abo_internal.h"
 
 using namespace abo;
@@ -1277,6 +1278,92 @@ extern "C" int32_t abo_gp_posterior_cov(abo_gp* g, const double* Xc, int64_t m, 
     cov_finish_kernel<<<(unsigned)((Mo * Mo + 255) / 256), 256, 0, st>>>(gp_spec(g), dXc, m, outputs, mp, G, Mpad, dcov, Mo, 0, 0.0);
     KL(c);
     CU(cudaMemcpyAsync(cov, dcov, sizeof(double) * Mo * Mo, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return ABO_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Monte-Carlo batch expected improvement over B batches of q points (qei.cuh).  Once per call: the S x q base normals
+// (key offset 2^62).  Per chunk of whole batches (about 2048 points):
+//   K* value rows -> W = L^-1 K*^T (TMA GEMM) -> q x q Gram blocks of W^T W and the means -> per-batch Cholesky, estimate
+//   and, with a gradient, C = d qEI / d Sigma -> Z = L^-T W (DMMA GEMM) -> R = (C + C^T) Z per batch (into the K* buffer)
+//   -> acq_grad_partial_kernel on R -> the per-point gradient.
+// ------------------------------------------------------------------------------------------
+constexpr int64_t QEI_MAX_S = 4096;
+constexpr uint64_t QEI_KEY_OFFSET = 1ull << 62;
+extern "C" int32_t abo_acq_qei(abo_gp* g, const double* params, int32_t q, const double* Xb, int64_t B, int64_t S,
+                               uint64_t seed, double jitter, double* values, double* grad, double* jitter_used) {
+    if (!g || !params || !Xb || !values) return abo_fail(ABO_ERR_INVALID, "null argument");
+    if (!g->fitted) return abo_fail(ABO_ERR_NOT_FITTED, "surrogate has no posterior (call update first)");
+    if (q < 1 || q > QEI_MAXQ) return abo_fail(ABO_ERR_INVALID, "qEI needs 1 <= q <= %d", QEI_MAXQ);
+    if (S < 1 || S > QEI_MAX_S) return abo_fail(ABO_ERR_INVALID, "qEI needs 1 <= S <= %lld", (long long)QEI_MAX_S);
+    if (g->d > AG_MAXD) return abo_fail(ABO_ERR_INVALID, "abo_acq_qei supports d <= %d", AG_MAXD);
+    if (!(jitter > 0) || !std::isfinite(jitter)) return abo_fail(ABO_ERR_INVALID, "jitter must be positive and finite");
+    if (B <= 0) return ABO_OK;
+    abo_ctx* c = g->ctx;
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const int64_t Npad = g->Npad, M = B * q;
+    const int d = g->d;
+    const int64_t nbc = std::max<int64_t>(1, 2048 / q);                 // batches per chunk
+    const int64_t mc = (nbc * q + NB - 1) / NB * NB;                    // columns per chunk, padded
+    const int64_t vpts = (Npad + g->p - 1) / g->p;
+    const int npb = (int)((vpts + 127) / 128);
+    const int npbg = (int)((g->n + 127) / 128);
+    const int ldz = (q + 3) / 4 * 4;
+    const bool want_grad = grad != nullptr;
+    double *dXb, *Ks, *pmean, *W, *Z = nullptr, *part = nullptr, *out, *zn, *bs;
+    int rc;
+    if ((rc = ws_get(c, WS_CAND, sizeof(double) * (size_t)M * d, (void**)&dXb)) ||
+        (rc = ws_get(c, WS_KS, sizeof(double) * (size_t)mc * Npad, (void**)&Ks)) ||
+        (rc = ws_get(c, WS_PMEAN, sizeof(double) * (size_t)npb * mc, (void**)&pmean)) ||
+        (rc = ws_get(c, WS_GRAD_W, sizeof(double) * (size_t)mc * Npad, (void**)&W)) ||
+        (rc = ws_get(c, WS_QEI_Z, sizeof(double) * (size_t)S * ldz, (void**)&zn)) ||
+        // per chunk: Gram [nbc q q] | mu [nbc q] | C [nbc q q] | d mu [nbc q]
+        (rc = ws_get(c, WS_QEI_BATCH, sizeof(double) * (size_t)nbc * q * (2 * q + 2), (void**)&bs)) ||
+        // values [B] | tau [B] | grad [B q d]
+        (rc = ws_get(c, WS_GRAD_OUT, sizeof(double) * (size_t)(2 * B + (want_grad ? M * d : 0)), (void**)&out)))
+        return rc;
+    if (want_grad &&
+        ((rc = ws_get(c, WS_GRAD_Z, sizeof(double) * (size_t)mc * Npad, (void**)&Z)) ||
+         (rc = ws_get(c, WS_GRAD_PART, sizeof(double) * (size_t)npbg * mc * 2 * AG_MAXD, (void**)&part))))
+        return rc;
+    double *Gm = bs, *mu = Gm + nbc * q * q, *Cb = mu + nbc * q, *dmu = Cb + nbc * q * q;
+    double *dV = out, *dT = out + B, *dG = out + 2 * B;
+    const double delta = params[1] - params[0];                        // (best_y - xi), EI's improvement convention
+    CU(cudaMemcpyAsync(dXb, Xb, sizeof(double) * M * d, cudaMemcpyHostToDevice, st));
+    philox_normal_kernel<<<(unsigned)((S * ldz / 4 + 255) / 256), 256, 0, st>>>(seed, QEI_KEY_OFFSET, 0, 1.0, S, q, S, ldz, ldz, zn);
+    KL(c);
+    const size_t smem = sizeof(double) * 4 * (size_t)q * (q + 1);
+    for (int64_t b0 = 0; b0 < B; b0 += nbc) {
+        const int64_t nb = std::min(nbc, B - b0), c0 = b0 * q, ncols = nb * q;
+        const int64_t mpad = (ncols + NB - 1) / NB * NB;
+        if ((rc = launch_ks_d(c, g, dXb, c0, M, 0, Ks, pmean, mpad, mc, npb, st))) return rc;
+        if ((rc = linv_times_ks(c, g, Ks, mpad, W, st))) return rc;                  // W = L^-1 K*^T   [Npad][mpad]
+        qei_gram_kernel<<<(unsigned)nb, 128, 0, st>>>(W, Npad, mpad, q, pmean, npb, mc, g->mean_c[0], Gm, mu);
+        KL(c);
+        qei_batch_kernel<<<(unsigned)nb, 32, smem, st>>>(gp_spec(g), dXb + c0 * d, q, Gm, mu, zn, S, ldz, delta, jitter,
+                                                         want_grad ? 1 : 0, dV + b0, dT + b0, dmu, Cb);
+        KL(c);
+        if (!want_grad) continue;
+        GemmParams z{};                                                                // Z = L^-T W      (k >= row)
+        z.A = g->dLinv; z.lda = g->ld; z.B = W; z.ldb = mpad; z.C = Z; z.ldc = mpad;
+        z.M = (int)Npad; z.N = (int)mpad; z.K = (int)Npad; z.alpha = 1.0; z.beta = 0.0; z.flags = KLO_M;
+        CU((launch_gemm(z, 1, st)));
+        KL(c);
+        double* R = Ks;                                                                // K* is consumed: R takes its place
+        qei_combine_kernel<<<dim3((unsigned)((ncols + 127) / 128), (unsigned)Npad), 128, 0, st>>>(Z, mpad, q, ncols, Cb, R);
+        KL(c);
+        acq_grad_partial_kernel<<<dim3(npbg, (unsigned)mpad), 128, 0, st>>>(gp_spec(g), g->dXsT, g->ldx, g->n, g->dAlpha, R,
+                                                                           mpad, dXb + c0 * d, ncols, part);
+        KL(c);
+        qei_grad_finish_kernel<<<(unsigned)((ncols + 127) / 128), 128, 0, st>>>(gp_spec(g), dXb + c0 * d, q, ncols, part, npbg,
+                                                                                mpad, dmu, Cb, dT + b0, dG + c0 * d);
+        KL(c);
+    }
+    CU(cudaMemcpyAsync(values, dV, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+    if (jitter_used) CU(cudaMemcpyAsync(jitter_used, dT, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+    if (want_grad) CU(cudaMemcpyAsync(grad, dG, sizeof(double) * M * d, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return ABO_OK;
 }

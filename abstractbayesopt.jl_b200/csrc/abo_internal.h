@@ -34,6 +34,7 @@ enum WsSlot {
     WS_TOPK, WS_SELECT, WS_GRAD_W, WS_GRAD_Z, WS_GRAD_PART, WS_GRAD_OUT, WS_TRTRI_U, WS_NLML_U,
     WS_SAMPLE_G, WS_SAMPLE_SIGMA, WS_SAMPLE_Z, WS_SAMPLE_F,       // joint posterior sampler: W^T W, Sigma + tau I -> its factor, Z^T, draws
     WS_PATH_FEAT, WS_PATH_PHI, WS_PATH_COEF, WS_PATH_R, WS_PATH_Y, WS_PATH_F,  // pathwise sampler: features, Phi, [alpha - V | Theta'], R -> V, Y, draws
+    WS_QEI_Z, WS_QEI_BATCH,                                        // batch expected improvement: base normals, per-batch Gram / mu / C / d mu
     WS_COUNT
 };
 

@@ -234,6 +234,35 @@ int32_t abo_acq_eval_multi(abo_gp* gp, int32_t nmem, const int32_t* acq_ids, con
 int32_t abo_acq_eval_grad(abo_gp* gp, int32_t acq_id, const double* params, const double* Xc, int64_t m,
                           double* scores, double* grad, double* mean, double* var);
 
+/* Monte-Carlo batch expected improvement, qEI (Ginsbourger et al. 2010; BoTorch qExpectedImprovement), for a minimiser:
+ * B batches of q points each scored jointly, so that a batch of near-duplicates scores no better than one of them.
+ * params = {xi, best_y}.  Xb: B x q x d, batch-major, then point-major (point j of batch b at Xb[(b q + j) d]).
+ * For batch b with points x_1 .. x_q, value output (also for a GradientGP), in the model's units:
+ *     mu (q)         the posterior mean, as abo_gp_posterior;
+ *     Sigma (q x q)  the posterior covariance, as abo_gp_posterior_cov(outputs = 1), its 1e-18 I included;
+ *     L = chol(Sigma + tau I), tau the first tau_k = jitter * sigma^2 * 10^k, k = 0 .. 6, whose Cholesky succeeds (the
+ *                    ladder of abo_gp_posterior_sample, walked per batch);
+ *     z_s            normals [0, q) of the Philox stream with key (seed, 2^62 + s), s = 0 .. S-1, in the layout of
+ *                    abo_gp_posterior_sample; this key range is disjoint from that sampler's (seed, s) and from the pathwise
+ *                    sampler's (seed, 2^63 + s) and (seed, 2^64 - 1 - l).  Every batch uses the same z_s (common random
+ *                    numbers), so the estimate is a smooth, deterministic function of the points;
+ *     f_s = mu + L z_s,   I_s = max((best_y - xi) - min_j f_{s,j}, 0)   (EI's convention: delta = (best_y - xi) - mu);
+ *     values[b] = (1/S) sum_s I_s, summed in ascending s.
+ * grad (nullable, B x q x d): the exact derivative of that expression with respect to every coordinate of the q points,
+ * tau held fixed, the min taken at its first minimising j; a sample with I_s = 0 contributes nothing.
+ * jitter_used (nullable, B): the tau of each batch.  A batch whose Cholesky fails at k = 6 gets a NaN value, NaN gradient
+ * and NaN jitter_used, and the call still returns ABO_OK.
+ * 1 <= q <= 32, 1 <= S <= 4096, d <= 32, jitter positive and finite, otherwise ABO_ERR_INVALID; B <= 0 is a no-op and there
+ * is no cap on B (batches go through in chunks of whole batches, about 2048 points each).  StandardGP (isotropic or ARD)
+ * and the value output of a GradientGP.  The posterior held by gp is only read.
+ * Guarantees: a batch's value, gradient and tau are bit-identical whatever other batches are in the call and wherever
+ * chunk boundaries fall; the value does not depend on whether grad is NULL; the same arguments give the same bits.
+ * Device workspace: about 8 (2 c N + B q d + 2 B + S q) bytes with c = 2048 points per chunk and N = n p rounded up to 128,
+ * plus 8 (c N + B q d + c n / 2) with a gradient: 134 MB + 8 (B q d + 2 B) at n p = 8192 without a gradient (abo_ctx_trim
+ * releases it). */
+int32_t abo_acq_qei(abo_gp* gp, const double* params, int32_t q, const double* Xb, int64_t B, int64_t S, uint64_t seed,
+                    double jitter, double* values, double* grad, double* jitter_used);
+
 /* nlml(model, [log l, log sig2], xs, ys) and its gradient for R parameter vectors at once
  * (StandardGP.jl:99-149, GradientGP.jl:684-738, driven by bayesian_opt.jl:259-300).
  * logparams: R x 2 (row r = {log l, log sig2}); nlml: R; grad: R x 2 (may be NULL);

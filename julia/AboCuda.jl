@@ -441,6 +441,25 @@ acq_id(::MaxValueEntropy) = Int32(4); acq_params(a::MaxValueEntropy) = Float64[l
 (a::MaxValueEntropy)(m::CuStandardGP, x::AbstractVector) = acq_eval(a, m, x)[1]
 (a::MaxValueEntropy)(m::CuGradientGP, x::AbstractVector) = acq_eval(a, m, x)[1]
 
+# Monte-Carlo batch expected improvement (abo_acq_qei, include/abo.h) of every batch in `batches`, a vector of B batches
+# of q points each: (values, jitter_used), both of length B.  Every batch uses the same num_samples base normals, drawn
+# from seed, so the values are a deterministic function of the points; a batch whose covariance does not factor gets NaN.
+function qei(m::Union{CuStandardGP,CuGradientGP}, batches::AbstractVector; xi::Real, best_y::Real, num_samples::Integer=512,
+             seed::Integer=0, jitter::Real=1e-10)
+    m.gpx === nothing && error("surrogate has no posterior: call update(model, xs, ys) first")
+    B = length(batches)
+    B == 0 && return Float64[], Float64[]
+    q = length(first(batches))
+    all(length(b) == q for b in batches) || throw(DimensionMismatch("every batch must hold the same number of points"))
+    Xb = Matrix{Float64}(points(collect(Iterators.flatten(batches))))   # d x (B q): batch-major, then point-major
+    params = Float64[xi, best_y]
+    vals = Vector{Float64}(undef, B); τ = Vector{Float64}(undef, B)
+    check(GC.@preserve params Xb vals τ ccall((:abo_acq_qei, LIB), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int32, Ptr{Float64}, Int64, Int64, UInt64, Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        m.gpx.h, params, Int32(q), Xb, B, num_samples, UInt64(seed), Float64(jitter), vals, C_NULL, τ))
+    vals, τ
+end
+
 # monte_carlo_fill_distance (src/BO_utils.jl:140-159) on the device; the caller draws the uniform samples
 function fill_distance(X::Matrix{Float64}, S::Matrix{Float64})         # both d x count, column-major = point-major
     out = Ref{Float64}(0.0)
